@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- throughput of the VFGS hardware-layer hot path on B200.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--workload NAME]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--workload NAME] [--dump-outputs DIR]
 
 One "step" is one batch of synthetic frames of the workload's size through the hot path (default: the
 BASELINE.json headline, 3840x2160 10-bit 4:2:0): PASSES calls of the C-ABI device entry point, each over
@@ -309,6 +309,30 @@ def parity_gate(hw, G, case, fmt, depth, od, rank, world):
     return done, None
 
 
+DUMP_SAMPLES = 1 << 22  # output samples written by --dump-outputs over all ranks: 16 MB of values + 32 MB of indices
+
+
+def dump_outputs(out_dir, dst, hw, rank=0, world=1):
+    """What the last timed step left in the output pool, for comparing two builds on the same inputs: a fixed,
+    seeded sample of the output samples (all of them if the pool is smaller) as float32, their flat indices into the
+    pool as float64, and the four LFSR registers the next call would start from. With several ranks each writes its
+    share of the sample, so the files stay within the same total size."""
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    suffix = "" if world == 1 else f"_rank{rank}"
+    n, k = dst.numel(), DUMP_SAMPLES // world
+    if n <= k:
+        idx = np.arange(n, dtype=np.int64)
+    else:
+        idx = np.unique(np.random.default_rng(2024 + rank).integers(0, n, size=k, dtype=np.int64))
+    vals = dst.index_select(0, torch.from_numpy(idx).to(dst.device)).cpu().numpy()
+    if vals.dtype == np.int16:
+        vals = vals.view(np.uint16)  # 10-bit codes travel as int16 tensors
+    np.save(os.path.join(out_dir, f"output_sample{suffix}.npy"), vals.astype(np.float32))
+    np.save(os.path.join(out_dir, f"output_sample_index{suffix}.npy"), idx.astype(np.float64))
+    np.save(os.path.join(out_dir, f"lfsr_after{suffix}.npy"), np.array(hw.get_lfsr(), dtype=np.float64))
+
+
 def run_b200_arm(args):
     import torch
     import torch.distributed as dist
@@ -431,6 +455,9 @@ def run_b200_arm(args):
     e1.record(stream)
     barrier()
     clocks = sampler.result()
+    if args.dump_outputs:
+        # before the copy below overwrites the output pool
+        dump_outputs(args.dump_outputs, dst, hw, rank, world)
     ms = e0.elapsed_time(e1)
     k_ms, k_n = hw.kernel_time()
     hw.kernel_timing(False)
@@ -612,7 +639,12 @@ def main():
     ap.add_argument("--in-place", action="store_true", help="diagnostic: output written over the input (same depth only)")
     ap.add_argument("--data", default="uniform", choices=["uniform", "natural"],
                     help="sample distribution of the synthetic frames (uniform random codes = worst case for the LUT/pattern gathers)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="after the timed steps, write a seeded sample of the last step's output frames and the LFSR "
+                         "registers as DIR/*.npy (CUDA path only)")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs needs --impl b200")
     if args.warmup < 3 and args.impl == "b200":
         args.warmup = 3  # timing rule: at least 3 warm-up steps
     sys.exit(run_reference_arm(args) if args.impl == "reference" else run_b200_arm(args))

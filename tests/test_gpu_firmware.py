@@ -41,23 +41,26 @@ def test_device_firmware_programs_the_reference_state(hw, case):
     assert states_equal(hw.state(), G.state(case), G.cases[case]["nslot"]) == [], case
 
 
-@pytest.mark.parametrize("case", ["fgs_sei.cfg|d10|420|g100", "fgs_sei_ar_test1.cfg|d10|420|g100", "fgs_afgs1_test1.cfg|d10|420|g100",
-                                  "fgs_sei_ff_test7.cfg|d8|420|g100"])
+@pytest.mark.parametrize("case", CASES)
 def test_device_firmware_then_frames(hw, case):
+    """Frames through the tables the device firmware built, for every golden configuration; 10-bit input also to
+    8-bit output (the CLI's --outdepth 8)."""
     import torch
     meta = G.cases[case]
-    init_from_golden(hw, case)
     w, h, n = 512, 152, 3
     frames = synth_frames(n, w, h, meta["fmt"], meta["depth"], seed=31)
-    o = Oracle(); program_case(o, G, case)
-    want = o.add_grain_frames(frames, n, w, h, 0)
     src = torch.from_numpy(frames.view(np.int16) if frames.dtype == np.uint16 else frames).cuda()
-    dst = torch.empty_like(src)
-    hw.add_grain_frames_device(src, dst, n, w, h, 0)
-    torch.cuda.synchronize()
-    got = dst.cpu().numpy()
-    got = got.view(np.uint16) if frames.dtype == np.uint16 else got
-    assert np.array_equal(got, want), first_mismatch(got, want, w, h, meta["fmt"], n)
+    for od in ((0, 8) if meta["depth"] == 10 else (0,)):
+        init_from_golden(hw, case)
+        o = Oracle(); program_case(o, G, case)
+        want = o.add_grain_frames(frames, n, w, h, od)
+        dst = torch.empty(frames.size, dtype=torch.uint8 if (od == 8 or meta["depth"] == 8) else torch.int16, device="cuda")
+        hw.add_grain_frames_device(src, dst, n, w, h, od)
+        torch.cuda.synchronize()
+        got = dst.cpu().numpy()
+        got = got.view(np.uint16) if got.dtype == np.int16 else got
+        assert np.array_equal(got, want), (od, first_mismatch(got, want, w, h, meta["fmt"], n))
+        assert hw.get_lfsr() == o.get_lfsr(), od
 
 
 def test_configuration_switch_with_frames_in_flight(hw):
