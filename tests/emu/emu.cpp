@@ -184,7 +184,9 @@ extern "C" int emu_add_grain_frames(const void* state, const void* in, void* out
 
 // Launch planning of a whole-frame call, without running anything (host logic only): which kernel serves each
 // component, the fast kernel's shared-memory layout and lane-unit width. out (ints): kind[3], fsmem, fpad,
-// fimg_off[3], fimg_bytes[3], fwide[3], funits_per_row[3], gather_smem, fallwide.
+// fimg_off[3], fimg_bytes[3], fwide[3], funits_per_row[3], gather_smem, fallwide, warp-tasks per frame of the fast,
+// EDGE, gather and general launches, gather_fold, gather_shift, EDGE funits_per_row[3], gather gunits_per_row[3]
+// (31 ints).
 extern "C" void emu_plan(const void* state, int width, int height, int out_depth, int in_place, int mode, int* out)
 {
 	const StateDump& d = *(const StateDump*)state;
@@ -235,6 +237,12 @@ extern "C" void emu_plan(const void* state, int width, int height, int out_depth
 	for (int c = 0; c < 3; c++) out[k++] = lp.fast.funits_per_row[c];
 	out[k++] = lp.gather_smem;
 	out[k++] = lp.fast.fallwide;
+	// warp-tasks of one frame per launch: fast, EDGE, gather, general
+	out[k++] = lp.fast.ftasks_per_frame; out[k++] = lp.edge.ftasks_per_frame; out[k++] = lp.gather.gtasks_per_frame;
+	out[k++] = lp.general.rows * lp.general.tasks_per_stripe;
+	out[k++] = lp.gather_fold; out[k++] = lp.gather_shift;
+	for (int c = 0; c < 3; c++) out[k++] = lp.edge.funits_per_row[c];
+	for (int c = 0; c < 3; c++) out[k++] = lp.gather.gunits_per_row[c];
 }
 
 // ---- firmware layer (fw_host.h + fw_device.h run with one host thread) ---------------------------

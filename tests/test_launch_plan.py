@@ -22,7 +22,7 @@ def emu():
 
 def plan(emu, o, w, h, od=0, in_place=0, mode=0):
     st = RefState(); o.L.oracle_get_state(o.h, C.byref(st))
-    out = np.zeros(20, dtype=np.int32)
+    out = np.zeros(32, dtype=np.int32)
     emu.emu_plan(C.byref(st), w, h, od, in_place, mode, out.ctypes.data_as(C.c_void_p))
     return {"kind": list(out[0:3]), "fsmem": int(out[3]), "fpad": int(out[4]), "fimg_off": list(out[5:8]),
             "fimg_bytes": list(out[8:11]), "fwide": list(out[11:14]), "units": list(out[14:17]), "gather_smem": int(out[17]),

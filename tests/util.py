@@ -101,6 +101,27 @@ RANDOM_STATES = [
 ]
 
 
+# bench.py's default run (--steps 20 --warmup 5) on the largest box the project reports on (--gpus 8)
+BENCH_STEPS, BENCH_WARMUP, BENCH_GPUS = 20, 5, 8
+
+
+def bench_call(workload: str, gpus: int = BENCH_GPUS):
+    """(frames per call, calls per step, first frame of the last call) of a default weak-scaling bench.py run of
+    `workload`, computed the way bench.py computes them: the last call is the last pass of the last step on the
+    highest rank, which starts furthest into the sequence."""
+    import bench
+    _, w, h, fmt, depth, od = bench.WORKLOADS[workload]
+    _, in_bytes, out_bytes = bench.frame_geometry(w, h, fmt, depth, od)
+    frames = int(max(8, min(4096, bench.POOL_INPUT_BYTES // in_bytes)))
+    passes = max(1, int(round(4.0e11 / (frames * (in_bytes + out_bytes)))))
+    s, p, rank = BENCH_WARMUP + BENCH_STEPS - 1, passes - 1, gpus - 1
+    return frames, passes, ((s * passes + p) * gpus + rank) * frames
+
+
+def bench_last_call_first_frame(workload: str) -> int:
+    return bench_call(workload)[2]
+
+
 def aligned_empty(n, dtype, offset=0):
     """n zeroed elements whose first byte sits `offset` bytes after a 64-byte boundary (numpy itself only promises 16):
     the 16-samples-per-lane paths of the fast kernel need 16 / 32-byte aligned rows."""
