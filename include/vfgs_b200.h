@@ -43,6 +43,20 @@ typedef struct vfgs_b200_planes {
 	int64_t frame_stride;  /* between consecutive frames, same for the three planes */
 } vfgs_b200_planes;
 
+/* Semi-planar frames, the layout of hardware video decoders and encoders: per frame a Y plane, then one plane in which
+ * U and V alternate on every chroma line. All strides are in BYTES. */
+#define VFGS_B200_NV12 1  /* 8-bit samples: Y plane, then one plane of interleaved U,V pairs (NV12 / NV16) */
+#define VFGS_B200_P010 2  /* 10-bit samples in bits 15..6 of little-endian uint16 (P010 / P210) */
+
+typedef struct vfgs_b200_semiplanar {
+	void*   y;
+	void*   uv;            /* U0 V0 U1 V1 ... on every chroma line */
+	int64_t stride_y;      /* bytes between luma lines */
+	int64_t stride_uv;     /* bytes between chroma lines */
+	int64_t frame_stride;  /* bytes between consecutive frames, same for both planes */
+	int     format;        /* VFGS_B200_NV12 | VFGS_B200_P010 */
+} vfgs_b200_semiplanar;
+
 /* Bind the library to a CUDA device (default: the current device at first use). */
 int vfgs_b200_init(int device);
 /* Hardware state back to the power-on values of src/vfgs_hw.c:49-63. */
@@ -68,6 +82,25 @@ int vfgs_b200_add_grain_frames_device(const void* in, void* out, int nframes, in
  * 8-samples-per-lane form; anything else the EDGE variant (DESIGN.md section 4). */
 int vfgs_b200_add_grain_planes_device(const vfgs_b200_planes* in, const vfgs_b200_planes* out,
                                       int nframes, int width, int height, int out_depth, void* stream);
+
+/* nframes semi-planar frames in DEVICE memory; asynchronous on `stream`. The chroma geometry is that of the planar
+ * calls: a UV line holds cw = width / subx pairs, the plane has ch = height / suby lines.
+ *   Output: the input deinterleaved, P010 samples taken as word >> 6, run through the planar path, and the result
+ *   reinterleaved with P010 samples written as value << 6, bit for bit; the LFSR registers advance exactly as for a
+ *   planar call of the same size, so semi-planar, planar and line calls and vfgs_b200_skip_frames interleave
+ *   bit-exactly. The low 6 bits of P010 input are ignored and written as zero.
+ *   Formats: in->format must match the configured depth (NV12 <-> 8, P010 <-> 10); out->format is in->format, or
+ *   NV12 from P010 (the fused (v + 2) >> 2 conversion of out_depth = 8). Only 4:2:0 and 4:2:2 are accepted (4:4:4
+ *   frames are planar: vfgs_b200_add_grain_planes_device).
+ *   in == out (same pointers, strides and format) is allowed; any other overlap, null pointers, line strides shorter
+ *   than a row and P010 planes or strides that are not 2-byte aligned are refused with VFGS_B200_ERR_ARG before any
+ *   device work.
+ *   Speed: with single-pattern chroma, widths that are multiples of 16 and planes, line strides and frame stride that
+ *   are multiples of 32 bytes (P010; 16 for NV12), U and V run on the fast kernel's interleaved lane; P010 luma takes
+ *   the 16-samples-per-lane fast path under the same conditions, or the gather kernel for sample-adaptive patterns.
+ *   Everything else takes the general kernel, which is correct everywhere and not fast (DESIGN.md section 13). */
+int vfgs_b200_add_grain_semiplanar_device(const vfgs_b200_semiplanar* in, const vfgs_b200_semiplanar* out,
+                                          int nframes, int width, int height, void* stream);
 
 /* nframes packed planar frames in HOST memory; returns when `out` is complete. Frames are cut into
  * chunks that flow through a ring of device buffers on three streams (H2D / kernels / D2H) so the
@@ -116,7 +149,8 @@ void vfgs_b200_pipeline_stats(unsigned long long out[2]);
 
 /* Geometry of the last grain kernel launch: out[0]=grid, out[1]=block, out[2]=dynamic smem bytes,
  * out[3]=SM count of the bound device, out[4]=which grain kernels the last frame call launched
- * (bit 0 fast, bit 1 general, bit 2 gather, bit 3 the fast kernel's EDGE variant). */
+ * (bit 0 fast, bit 1 general, bit 2 gather, bit 3 the fast kernel's EDGE variant, bit 4 the fast kernel's interleaved
+ * U/V lane of semi-planar frames). */
 void vfgs_b200_last_launch(int out[5]);
 
 #ifdef __cplusplus

@@ -4,7 +4,10 @@ through the setters (depth, format, 1-8 pattern slots per bank, legal range, sca
 random picture sizes, in-range and garbage samples, frame offsets into a running sequence, in-place operation, every
 kernel-selection mode. Test tool, no GPU.
 
-    python scripts/fuzz_emulation.py [seed] [seconds]
+    python scripts/fuzz_emulation.py [seed] [seconds] [--semiplanar]
+
+--semiplanar: semi-planar frames (vfgs_b200_add_grain_semiplanar_device, tests/emu/emu_semiplanar.cpp) instead, 4:2:0 / 4:2:2,
+NV12 / P010 / P010 -> NV12, random widths, base alignments, padded pitches and in place.
 
 (Found in round 1: a Cr component with its own fast-kernel image next to a sample-adaptive Cb got an empty image.)"""
 import ctypes as C
@@ -60,13 +63,49 @@ def one_case(emu, rng):
     return None
 
 
-def run(seed: int, seconds: float, max_cases: int = 0):
-    emu = C.CDLL(build_emu())
-    emu.emu_add_grain_frames.argtypes = [C.c_void_p] * 3 + [C.c_int] * 6
+def one_semiplanar_case(emu, rng):
+    from tests.semiplanar import Surface, planar_to_semi, run_emu_semi, semi_to_planar
+    depth = int(rng.choice([8, 10])); fmt = str(rng.choice(["420", "422"]))
+    one = rng.integers(0, 2) == 0  # half of the cases with one pattern per bank (the interleaved fast lane)
+    spec = (int(rng.integers(1, 1 << 30)), depth, fmt, 1 if one else int(rng.integers(1, 9)), 1 if one else int(rng.integers(1, 9)),
+            int(rng.integers(0, 2)), int(rng.integers(2, 8)), bool(rng.integers(0, 4) == 0))
+    w = int(rng.choice(WIDTHS)) & ~1; h = max(2, int(rng.integers(1, 70))) & ~1; n = int(rng.integers(1, 4))
+    ch = h // (2 if fmt == "420" else 1)
+    p010 = depth == 10
+    frames = synth_frames(n, w, h, fmt, depth, seed=spec[0] % 1000)
+    first = int(rng.integers(0, 5000)) if rng.integers(0, 3) == 0 else 0
+    for p010_out in ((True, False) if p010 else (False,)):
+        for in_place in ((False, True) if p010_out == p010 else (False,)):
+            mode = int(rng.choice([0, 0, 1, 2]))
+            o = Oracle(); program_random_state(o, *spec)
+            isz, osz = (2 if p010 else 1), (2 if p010_out else 1)
+            offset = int(rng.choice([0, 0, 32, 16, 8, 4, 2])) & ~(isz - 1)
+            pads = [int(rng.choice([0, 0, 16, 32, 64, 2])) & ~(max(isz, osz) - 1) for _ in range(2)]
+            src = Surface(n, w, h, ch, isz, w * isz + pads[0], w * isz + pads[1], offset)
+            Y, UV = planar_to_semi(frames, n, w, h, fmt, p010, rng=rng)
+            src.fill(Y, UV)
+            dst = src if in_place else Surface(n, w, h, ch, osz, w * osz + pads[0], w * osz + pads[1], int(rng.choice([offset, 0])) & ~(osz - 1))
+            mask = run_emu_semi(emu, o, src, dst, n, w, h, p010_out, first=first, mode=mode)
+            o.skip_frames(first, w, h)
+            want = o.add_grain_frames(frames, n, w, h, 0 if p010_out == p010 else 8)
+            got = semi_to_planar(*dst.planes(), p010_out)
+            if not np.array_equal(got, want):
+                return (f"MISMATCH semiplanar spec={spec} w={w} h={h} n={n} p010_out={p010_out} in_place={in_place} mode={mode} "
+                        f"offset={offset} pads={pads} mask={mask}: {first_mismatch(got, want, w, h, fmt, n)}")
+    return None
+
+
+def run(seed: int, seconds: float, max_cases: int = 0, semiplanar: bool = False):
+    if semiplanar:
+        from tests.semiplanar import load_emu
+        emu = load_emu()
+    else:
+        emu = C.CDLL(build_emu())
+        emu.emu_add_grain_frames.argtypes = [C.c_void_p] * 3 + [C.c_int] * 6
     rng = np.random.default_rng(seed)
     t0, n = time.time(), 0
     while time.time() - t0 < seconds and (max_cases == 0 or n < max_cases):
-        bad = one_case(emu, rng)
+        bad = one_semiplanar_case(emu, rng) if semiplanar else one_case(emu, rng)
         if bad:
             return n, bad
         n += 1
@@ -74,6 +113,8 @@ def run(seed: int, seconds: float, max_cases: int = 0):
 
 
 if __name__ == "__main__":
-    n, bad = run(int(sys.argv[1]) if len(sys.argv) > 1 else 0, float(sys.argv[2]) if len(sys.argv) > 2 else 60)
+    semi = "--semiplanar" in sys.argv
+    argv = [a for a in sys.argv[1:] if a != "--semiplanar"]
+    n, bad = run(int(argv[0]) if argv else 0, float(argv[1]) if len(argv) > 1 else 60, semiplanar=semi)
     print(bad or f"fuzz ok: {n} cases")
     sys.exit(1 if bad else 0)

@@ -28,7 +28,9 @@ B200_SYMBOLS = (
     "vfgs_b200_set_lfsr", "vfgs_b200_host_alloc", "vfgs_b200_host_free", "vfgs_b200_launch_count",
     "vfgs_b200_last_launch", "vfgs_b200_get_state", "vfgs_b200_kernel_timing", "vfgs_b200_kernel_time",
     "vfgs_b200_force_general_kernel", "vfgs_b200_pipeline_stats", "vfgs_b200_init_sei", "vfgs_b200_init_afgs1",
+    "vfgs_b200_add_grain_semiplanar_device",
 )
+NV12, P010 = 1, 2  # VFGS_B200_NV12 / VFGS_B200_P010
 
 
 class VfgsError(RuntimeError):
@@ -39,6 +41,24 @@ class Planes(C.Structure):
     """vfgs_b200_planes (include/vfgs_b200.h)."""
     _fields_ = [("y", C.c_void_p), ("u", C.c_void_p), ("v", C.c_void_p),
                 ("stride_y", C.c_int64), ("stride_c", C.c_int64), ("frame_stride", C.c_int64)]
+
+
+class SemiPlanes(C.Structure):
+    """vfgs_b200_semiplanar (include/vfgs_b200.h): a Y plane and one plane of interleaved U,V pairs."""
+    _fields_ = [("y", C.c_void_p), ("uv", C.c_void_p), ("stride_y", C.c_int64), ("stride_uv", C.c_int64),
+                ("frame_stride", C.c_int64), ("format", C.c_int)]
+
+
+def surface_planes(t, height: int, fmt: int) -> SemiPlanes:
+    """The usual decoder surface: a CUDA tensor of shape (n, height + ch, pitch) (uint8 for NV12, 16-bit for P010;
+    pitch in samples) holding per frame `height` Y rows and then the `ch` UV rows, all at the same pitch."""
+    if t.dim() != 3 or not t.is_contiguous():
+        raise VfgsError("surface must be a contiguous (n, height + ch, pitch) tensor")
+    if t.element_size() != (2 if fmt == P010 else 1):
+        raise VfgsError("NV12 surfaces hold 8-bit samples, P010 surfaces 16-bit ones")
+    pitch = t.shape[2] * t.element_size()
+    base = t.data_ptr()
+    return SemiPlanes(base, base + height * pitch, pitch, pitch, t.shape[1] * pitch, fmt)
 
 
 _lib = None
@@ -74,6 +94,7 @@ def load_library(global_symbols: bool = False) -> C.CDLL:
     L.vfgs_b200_frame_bytes.restype = C.c_size_t
     L.vfgs_b200_add_grain_frames_device.argtypes = [vp, vp, ci, ci, ci, ci, vp]
     L.vfgs_b200_add_grain_planes_device.argtypes = [C.POINTER(Planes), C.POINTER(Planes), ci, ci, ci, ci, vp]
+    L.vfgs_b200_add_grain_semiplanar_device.argtypes = [C.POINTER(SemiPlanes), C.POINTER(SemiPlanes), ci, ci, ci, vp]
     L.vfgs_b200_add_grain_frames_host.argtypes = [vp, vp, ci, ci, ci, ci]
     L.vfgs_b200_skip_frames.argtypes = [C.c_int64, ci, ci]
     L.vfgs_b200_get_lfsr.argtypes = [vp]
@@ -162,7 +183,8 @@ class VfgsHw:
     def last_launch(self) -> dict:
         a = (C.c_int * 5)()
         self.L.vfgs_b200_last_launch(a)
-        kernels = [n for bit, n in ((1, "fgs_apply_fast_kernel"), (8, "fgs_apply_fast_kernel<EDGE>"), (4, "fgs_apply_gather_kernel"), (2, "fgs_apply_kernel")) if a[4] & bit]
+        kernels = [n for bit, n in ((1, "fgs_apply_fast_kernel"), (8, "fgs_apply_fast_kernel<EDGE>"), (4, "fgs_apply_gather_kernel"), (2, "fgs_apply_kernel"),
+                                           (16, "fgs_apply_fast_kernel<interleaved UV>")) if a[4] & bit]
         return {"grid": a[0], "block": a[1], "smem": a[2], "sms": a[3], "kernels": kernels}
 
     def state(self) -> dict:
@@ -206,6 +228,22 @@ class VfgsHw:
     def add_grain_planes_device(self, pin: Planes, pout: Planes, nframes, width, height, out_depth=0, stream_ptr=0):
         self._chk(self.L.vfgs_b200_add_grain_planes_device(
             C.byref(pin), C.byref(pout), nframes, width, height, out_depth, C.c_void_p(stream_ptr)))
+
+    def add_grain_semiplanar_device(self, pin: SemiPlanes, pout: SemiPlanes, nframes, width, height, stream_ptr=0):
+        """Semi-planar (NV12 / P010) frames in device memory, see vfgs_b200_add_grain_semiplanar_device."""
+        self._chk(self.L.vfgs_b200_add_grain_semiplanar_device(
+            C.byref(pin), C.byref(pout), nframes, width, height, C.c_void_p(stream_ptr)))
+
+    def add_grain_surfaces(self, src, dst, nframes, width, height, out_format=None, stream=None):
+        """src/dst: decoder-style surfaces, CUDA tensors of shape (n, height + ch, pitch) (surface_planes). The input
+        format follows the configured depth (NV12 for 8, P010 for 10); out_format defaults to the input format
+        (NV12 from P010 is the fused 10 -> 8 conversion). src is dst for in place."""
+        import torch
+        if stream is None:
+            stream = torch.cuda.current_stream(src.device)
+        in_fmt = P010 if src.element_size() == 2 else NV12
+        self.add_grain_semiplanar_device(surface_planes(src, height, in_fmt), surface_planes(dst, height, out_format or in_fmt),
+                                         nframes, width, height, stream.cuda_stream)
 
     def add_grain_frames_host(self, src, dst, nframes, width, height, out_depth=0):
         """src/dst: host buffers (numpy arrays or pinned torch CPU tensors)."""

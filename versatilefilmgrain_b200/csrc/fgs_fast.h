@@ -752,6 +752,21 @@ VFGS_HD void fast_task_body(const FgsParams& p, smem_addr_t lut, const TaskGeom&
 // 256-bit access (LDG.256 / STG.256, sm_100), 128-bit for the 8-bit output of the fused 10 -> 8 conversion. Taken when
 // the component's width is a multiple of 16 and its rows are aligned to the access size (plan_launches, FgsParams::fwide).
 // (Round 2, measured under the sustained protocol: profiles/r02_wide16_ab.md.)
+// P010 samples (value in bits 15..6 of a uint16) to and from the LSB-aligned form of the arithmetic, two per word. The low
+// six bits of the input are ignored; after the clip a value is at most 1020, so the shift back up cannot carry across the halves.
+template <int N>
+VFGS_HD void msb_to_lsb(const uint32_t* raw, uint32_t* out)
+{
+#pragma unroll
+	for (int k = 0; k < N; k++) out[k] = (raw[k] >> 6) & 0x03ff03ffu;
+}
+template <int N>
+VFGS_HD void lsb_to_msb(uint32_t* w)
+{
+#pragma unroll
+	for (int k = 0; k < N; k++) w[k] <<= 6;
+}
+
 struct WideLane {
 	smem_addr_t own0, own1;  // pattern rows of line j = 0: samples 0..7 and 8..15 (two blocks when the block size is 8)
 	smem_addr_t lh, rh;      // halo bytes: last column of the block to the left / first column of the block to the right
@@ -778,7 +793,8 @@ VFGS_HD void blend_octet(int g[8], uint32_t u0, uint32_t u1, int w_cur, int w_up
 }
 // One line of one wide lane: 16 samples in raw (8-bit: four words of four bytes, 16-bit: eight words of two samples),
 // result in outw (four words of 8-bit samples or eight of 16-bit samples).
-template <bool IN16, bool OUT8, int NSH>
+// MSB: 16-bit samples hold the value in bits 15..6 (P010 luma): shifted down here, the caller shifts the result back up.
+template <bool IN16, bool OUT8, int NSH, bool MSB = false>
 VFGS_HD void wide_line(const WideLane& L, int rc, int w_cur, int w_up, const WideUp& U, int ru,
                        const uint32_t* raw, uint32_t* outw)
 {
@@ -810,8 +826,11 @@ VFGS_HD void wide_line(const WideLane& L, int rc, int w_cur, int w_up, const Wid
 	ga[0] = L.has_left ? f0 : ga[0];
 	gb[7] = L.has_right ? f15 : gb[7];
 	if (IN16) {
-		scale_add_clip_16bit<OUT8>(L.lut, L.lo2, L.hi2, ga, raw, outw);
-		scale_add_clip_16bit<OUT8>(L.lut, L.lo2, L.hi2, gb, raw + 4, outw + (OUT8 ? 2 : 4));
+		uint32_t cv[8];
+		if (MSB) msb_to_lsb<8>(raw, cv);
+		const uint32_t* r = MSB ? cv : raw;
+		scale_add_clip_16bit<OUT8>(L.lut, L.lo2, L.hi2, ga, r, outw);
+		scale_add_clip_16bit<OUT8>(L.lut, L.lo2, L.hi2, gb, r + 4, outw + (OUT8 ? 2 : 4));
 	} else {
 		scale_add_clip_8bit(L.lut, L.lo2, L.hi2, ga, raw[0], raw[1], outw[0], outw[1]);
 		scale_add_clip_8bit(L.lut, L.lo2, L.hi2, gb, raw[2], raw[3], outw[2], outw[3]);
@@ -829,7 +848,7 @@ VFGS_HD void wide_line(const WideLane& L, int rc, int w_cur, int w_up, const Wid
 #ifndef VFGS_WIDE16_LB8
 #define VFGS_WIDE16_LB8 2  // 8-bit output (768 threads)
 #endif
-template <bool IN16, bool OUT8, int NSH, bool ALLWIDE = false>
+template <bool IN16, bool OUT8, int NSH, bool ALLWIDE = false, bool MSB = false>
 VFGS_HD void wide_task_body(const FgsParams& p, smem_addr_t lut, const TaskGeom& t, int k0, int lane)
 {
 	const int c = t.c;
@@ -895,7 +914,191 @@ VFGS_HD void wide_task_body(const FgsParams& p, smem_addr_t lut, const TaskGeom&
 			int wc = 0, wu = 0, ru = 0;
 			if (q == 0 && ovl) { wc = ysh ? 20 : 12; wu = ysh ? 20 : 24; ru = (16 >> ysh) * L.stride; }
 			if (q == 1 && ovl && !ysh) { wc = 24; wu = 12; ru = 17 * L.stride; }
-			wide_line<IN16, OUT8, NSH>(L, rc, wc, wu, U, ru, raw[q], w);
+			wide_line<IN16, OUT8, NSH, MSB>(L, rc, wc, wu, U, ru, raw[q], w);
+			if (MSB && OB == 2) lsb_to_msb<OW>(w);
+			if (IN16) ld_global_32_if(nxt, raw[q], line + LB < nl);
+			else ld_global_16_if(nxt, raw[q], line + LB < nl);
+			if (line < nl) {
+				if (OB == 2) st_global_32(dst, w);
+				else st_global_16(dst, w);
+			}
+			rc += L.stride; nxt += in_pitch; dst += out_pitch;
+		}
+		ovl = false;
+	}
+}
+
+// ---- interleaved chroma (semi-planar frames) -------------------------------------------------------
+// A UV line holds U0 V0 U1 V1 ...; with 4:2:0 / 4:2:2 a chroma block is 8 samples, so 16 consecutive samples of the line
+// are one block of U and the same block of V. A lane unit is that pair: one 256-bit access per line for 16-bit samples
+// (128-bit for 8-bit samples and for the 8-bit output of the fused 10 -> 8 conversion), two pattern octets (U's window
+// from component 1's entry of the block, V's from component 2's), four halo bytes, and no lane-internal edge. Every packed
+// 16-bit pair of the arithmetic is (U_k, V_k): U's LUT serves the low half, V's the high half, and the S16x2 add and clip
+// run unchanged because U and V share the clip range.
+template <bool OUT8>
+VFGS_HD void scale_add_clip_uv_16bit(smem_addr_t lut_u, smem_addr_t lut_v, uint32_t lo2, uint32_t hi2, const int* gu, const int* gv,
+                                     const uint32_t raw[4], uint32_t* outw)
+{
+	constexpr int kRound = OUT8 ? 0x28000 : 0x8000; // see scale_add_clip_16bit
+	uint32_t r[4];
+#pragma unroll
+	for (int k = 0; k < 4; k++) {
+		const int s_lo = (int)lds32(lut_u | (smem_addr_t)((raw[k] << 5) & 0x7f80u));
+		const int s_hi = (int)lds32(lut_v | (smem_addr_t)(shr_fma<11>(raw[k]) & 0x7f80u));
+		const int a_lo = s_lo * gu[k] + kRound;
+		const int a_hi = s_hi * gv[k] + kRound;
+		const uint32_t d2 = prmt((uint32_t)a_lo, (uint32_t)a_hi, 0x7632);
+		const uint32_t v2 = min_u16x2(raw[k], 0x3fff3fffu);
+		r[k] = min_s16x2(add_max_s16x2(v2, d2, lo2), hi2);
+	}
+	if (OUT8) {
+#pragma unroll
+		for (int k = 0; k < 4; k++) r[k] *= 64u;
+		outw[0] = prmt(r[0], r[1], 0x7531);
+		outw[1] = prmt(r[2], r[3], 0x7531);
+	} else {
+		outw[0] = r[0]; outw[1] = r[1]; outw[2] = r[2]; outw[3] = r[3];
+	}
+}
+VFGS_HD void scale_add_clip_uv_8bit(smem_addr_t lut_u, smem_addr_t lut_v, uint32_t lo2, uint32_t hi2, const int* gu, const int* gv,
+                                    uint32_t raw0, uint32_t raw1, uint32_t& out0, uint32_t& out1)
+{
+	uint32_t r[4];
+#pragma unroll
+	for (int k = 0; k < 4; k++) {
+		const uint32_t v2 = prmt(k < 2 ? raw0 : raw1, 0u, (k & 1) ? 0x4342 : 0x4140);
+		const int s_lo = (int)lds32(lut_u | (smem_addr_t)((v2 << 7) & 0x7f80u));
+		const int s_hi = (int)lds32(lut_v | (smem_addr_t)(shr_fma<9>(v2) & 0x7f80u));
+		const int a_lo = s_lo * gu[k] + 0x8000;
+		const int a_hi = s_hi * gv[k] + 0x8000;
+		const uint32_t d2 = prmt((uint32_t)a_lo, (uint32_t)a_hi, 0x7632);
+		r[k] = min_s16x2(add_max_s16x2(v2, d2, lo2), hi2);
+	}
+	out0 = prmt(r[0], r[1], 0x6420);
+	out1 = prmt(r[2], r[3], 0x6420);
+}
+
+struct UvLane {
+	smem_addr_t own_u, own_v;              // pattern rows of line j = 0 of the block's U and V windows
+	smem_addr_t lh_u, rh_u, lh_v, rh_v;    // halo bytes: last column of the block to the left / first of the block to the right
+	smem_addr_t lut_u, lut_v;
+	int stride;
+	bool has_left, has_right;
+	uint32_t lo2, hi2;
+};
+struct UvUp {
+	smem_addr_t own_u, own_v, lh_u, rh_u, lh_v, rh_v;
+};
+
+// One grain octet of an 8-sample block: vertical overlap and both block-edge filters (vfgs_hw.c:223-229, 250-259).
+VFGS_HD void block_octet(smem_addr_t own, smem_addr_t lh, smem_addr_t rh, smem_addr_t up_own, smem_addr_t up_lh, smem_addr_t up_rh,
+                         bool has_left, bool has_right, int rc, int w_cur, int w_up, int ru, int g[8])
+{
+	uint32_t a0, a1;
+	octet(own + rc, a0, a1);
+	octet_to_ints(a0, a1, g);
+	int hl = has_left ? lds_s8(lh + rc) : 0;
+	int hr = has_right ? lds_s8(rh + rc) : 0;
+	if (w_cur) {
+		uint32_t u0, u1;
+		octet(up_own + ru, u0, u1);
+		blend_octet(g, u0, u1, w_cur, w_up);
+		if (has_left) hl = (hl * w_cur + lds_s8(up_lh + ru) * w_up + 16) >> 5;
+		if (has_right) hr = (hr * w_cur + lds_s8(up_rh + ru) * w_up + 16) >> 5;
+	}
+	const int f0 = (hl + 3 * g[0] + g[1] + 2) >> 2;
+	const int f7 = (g[6] + 3 * g[7] + hr + 2) >> 2;
+	g[0] = has_left ? f0 : g[0];
+	g[7] = has_right ? f7 : g[7];
+}
+
+// One line of one interleaved-chroma lane. raw: 16 samples U0 V0 .. U7 V7 as loaded (16-bit: eight words, P010 when IN16;
+// 8-bit: four words); outw: the same layout at the output depth.
+template <bool IN16, bool OUT8>
+VFGS_HD void uv_line(const UvLane& L, int rc, int w_cur, int w_up, const UvUp& U, int ru, const uint32_t* raw, uint32_t* outw)
+{
+	int gu[8], gv[8];
+	block_octet(L.own_u, L.lh_u, L.rh_u, U.own_u, U.lh_u, U.rh_u, L.has_left, L.has_right, rc, w_cur, w_up, ru, gu);
+	block_octet(L.own_v, L.lh_v, L.rh_v, U.own_v, U.lh_v, U.rh_v, L.has_left, L.has_right, rc, w_cur, w_up, ru, gv);
+	if (IN16) {
+		uint32_t cv[8];
+		msb_to_lsb<8>(raw, cv);
+		scale_add_clip_uv_16bit<OUT8>(L.lut_u, L.lut_v, L.lo2, L.hi2, gu, gv, cv, outw);
+		scale_add_clip_uv_16bit<OUT8>(L.lut_u, L.lut_v, L.lo2, L.hi2, gu + 4, gv + 4, cv + 4, outw + (OUT8 ? 2 : 4));
+	} else {
+		scale_add_clip_uv_8bit(L.lut_u, L.lut_v, L.lo2, L.hi2, gu, gv, raw[0], raw[1], outw[0], outw[1]);
+		scale_add_clip_uv_8bit(L.lut_u, L.lut_v, L.lo2, L.hi2, gu + 4, gv + 4, raw[2], raw[3], outw[2], outw[3]);
+	}
+}
+
+// k0: first chroma sample (of U and of V) of the lane; the block is k0 / 8. Same line pipeline as wide_task_body.
+template <bool IN16, bool OUT8, bool ALLWIDE = false>
+VFGS_HD void uv_task_body(const FgsParams& p, smem_addr_t lut, const TaskGeom& t, int k0, int lane)
+{
+	const Plane& pl = p.comp[1];
+	const int ysh = p.suby > 1 ? 1 : 0;
+	constexpr int LB = !IN16 ? VFGS_FAST_LB16 : OUT8 ? VFGS_WIDE16_LB8 : ALLWIDE ? VFGS_WIDE16_LBW : VFGS_WIDE16_LB;
+	static_assert(LB >= 2, "both vertical-overlap lines of a block-row must fall into the first group of lines");
+	constexpr int IB = IN16 ? 2 : 1, OB = (IN16 && !OUT8) ? 2 : 1;
+	constexpr int RW = IN16 ? 8 : 4, OW = OB == 2 ? 8 : 4;
+
+	const int cl0 = (t.r * 16) >> ysh;
+	int cl1 = cl0 + (16 >> ysh);
+	if (cl1 > pl.lines) cl1 = pl.lines;
+	const int nl = cl1 - cl0;
+	if (nl <= 0) return;
+
+	const long long in_pitch = pl.in_row_bytes, out_pitch = pl.out_row_bytes;
+	const uint8_t* src = pl.in + (long long)t.f * p.in_frame_bytes + (long long)cl0 * in_pitch + (long long)k0 * 2 * IB;
+	uint8_t* dst = pl.out + (long long)t.f * p.out_frame_bytes + (long long)cl0 * out_pitch + (long long)k0 * 2 * OB;
+
+	uint32_t raw[LB][RW];
+#pragma unroll
+	for (int q = 0; q < LB; q++) {
+		if (IN16) ld_global_32(src + (q < nl ? q : nl - 1) * in_pitch, raw[q]);
+		else ld_global_16(src + (q < nl ? q : nl - 1) * in_pitch, raw[q]);
+	}
+
+	const int b = k0 >> 3;
+	UvLane L;
+	L.has_left = b > 0;
+	L.has_right = b + 1 < p.nb;
+	L.stride = p.fpat_stride[1]; // U's and V's images have the same geometry
+	L.lut_u = lut + (smem_addr_t)(kLutBytes + lane * 4);
+	L.lut_v = lut + (smem_addr_t)(2 * kLutBytes + lane * 4);
+	constexpr int kOutBias = (IN16 && OUT8) ? 2 : 0;
+	L.lo2 = (uint32_t)(p.lo[1] + kOutBias) * 0x00010001u; L.hi2 = (uint32_t)(p.hi[1] + kOutBias) * 0x00010001u;
+
+	const smem_addr_t img_u = lut + (smem_addr_t)(ptrdiff_t)p.fimg_off[1], img_v = lut + (smem_addr_t)(ptrdiff_t)p.fimg_off[2];
+	const int srow = t.r - p.stream_row0;
+	const uint16_t* w_u = p.woffs + (((long long)t.f * p.stream_rows + srow) * p.spitch + 1 + b) * 4 + 1; // V: w_u + 1
+	auto windows = [&](const uint16_t* w, UvUp& o) {
+		o.own_u = img_u + (smem_addr_t)w[0];
+		o.own_v = img_v + (smem_addr_t)w[1];
+		o.lh_u = o.rh_u = o.own_u; o.lh_v = o.rh_v = o.own_v;
+		if (L.has_left) { o.lh_u = img_u + (smem_addr_t)(w[-4] + 7); o.lh_v = img_v + (smem_addr_t)(w[-3] + 7); }
+		if (L.has_right) { o.rh_u = img_u + (smem_addr_t)w[4]; o.rh_v = img_v + (smem_addr_t)w[5]; }
+	};
+	UvUp C;
+	windows(w_u, C);
+	L.own_u = C.own_u; L.own_v = C.own_v; L.lh_u = C.lh_u; L.rh_u = C.rh_u; L.lh_v = C.lh_v; L.rh_v = C.rh_v;
+	UvUp U = C;
+	bool ovl = t.r > 0;
+	if (ovl) windows(w_u - p.spitch * 4, U);
+
+	int rc = 0;
+	const uint8_t* nxt = src + LB * in_pitch;
+#pragma unroll 1
+	for (int base = 0; base < nl; base += LB) {
+#pragma unroll
+		for (int q = 0; q < LB; q++) {
+			const int line = base + q;
+			uint32_t w[OW];
+			int wc = 0, wu = 0, ru = 0;
+			if (q == 0 && ovl) { wc = ysh ? 20 : 12; wu = ysh ? 20 : 24; ru = (16 >> ysh) * L.stride; }
+			if (q == 1 && ovl && !ysh) { wc = 24; wu = 12; ru = 17 * L.stride; }
+			uv_line<IN16, OUT8>(L, rc, wc, wu, U, ru, raw[q], w);
+			if (OB == 2) lsb_to_msb<OW>(w);
 			if (IN16) ld_global_32_if(nxt, raw[q], line + LB < nl);
 			else ld_global_16_if(nxt, raw[q], line + LB < nl);
 			if (line < nl) {
@@ -916,7 +1119,9 @@ VFGS_HD void wide_task_body(const FgsParams& p, smem_addr_t lut, const TaskGeom&
 // not be a multiple of 256 samples).
 // ALLWIDE: every component of the launch takes the 16-samples-per-lane path (FgsParams::fallwide); the kernel variant then
 // has its own CTA size and more lines in flight per lane.
-template <bool IN16, bool OUT8, bool EDGE = false, bool ALLWIDE = false>
+// SEMI: semi-planar frames (NV12 / P010): component 1 is the interleaved UV plane (uv_task_body), component 2 has no
+// tasks, luma is served here only on the wide path (16-bit luma MSB-aligned).
+template <bool IN16, bool OUT8, bool EDGE = false, bool ALLWIDE = false, bool SEMI = false>
 VFGS_HD void process_task_fast(const FgsParams& p, smem_addr_t lut, uint32_t task, int lane)
 {
 	TaskGeom t;
@@ -932,6 +1137,13 @@ VFGS_HD void process_task_fast(const FgsParams& p, smem_addr_t lut, uint32_t tas
 	t.r = p.row_begin + (int)row;
 	t.seg = 0;
 	static_assert(!(ALLWIDE && EDGE), "the EDGE variant has no wide path");
+	static_assert(!(SEMI && EDGE), "the EDGE variant has no semi-planar form");
+	if constexpr (SEMI) {
+		const int u = (int)(unit - row * upr);
+		if (t.c) uv_task_body<IN16, OUT8, ALLWIDE>(p, lut, t, u * 8, lane);
+		else wide_task_body<IN16, OUT8, 4, ALLWIDE, IN16>(p, lut, t, u * 16, lane); // the host sends wide luma only
+		return;
+	}
 	if (ALLWIDE || (!EDGE && p.fwide[t.c])) { // 16 samples per lane
 		const int k0 = (int)(unit - row * upr) * 16;
 		if (t.c && p.subx > 1) wide_task_body<IN16, OUT8, 3, ALLWIDE>(p, lut, t, k0, lane);

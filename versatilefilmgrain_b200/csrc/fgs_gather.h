@@ -307,7 +307,8 @@ VFGS_HD void gather_ld_if(const uint8_t* p, uint32_t r[4], bool pred)
 // SHIFT (NSH = 4 only): the warp holds units 32 q - 1 .. 32 q + 30 instead, see the head of this file.
 // Every lane walks the full line count of a stripe (the exchange is a warp-wide shuffle); lanes outside the picture
 // or past the end of a short last stripe neither load nor store.
-template <bool IN16, bool OUT8, int NSH, bool FOLD, bool SHIFT>
+// MSB: 16-bit samples hold the value in bits 15..6 (P010 luma of semi-planar frames), converted where a line is used.
+template <bool IN16, bool OUT8, int NSH, bool FOLD, bool SHIFT, bool MSB = false>
 VFGS_HD void gather_task_body(const FgsParams& p, smem_addr_t luts, smem_addr_t img, int f, int c, uint32_t q, int lane)
 {
 	constexpr bool PAIR = NSH == 4;
@@ -400,6 +401,10 @@ VFGS_HD void gather_task_body(const FgsParams& p, smem_addr_t luts, smem_addr_t 
 			const int line = base + qq;
 			int g[8], sc[8], gh = 0;
 			bool done = false;
+			if constexpr (MSB) { // in place: the slot is refilled after this line
+				msb_to_lsb<4>(raw[qq], raw[qq]);
+				vh[qq] >>= 6;
+			}
 			if (FIRST && qq < 2 && !(qq == 1 && ysh)) { // vfgs_hw.c:173-188: lines 0 and 1 (line 0 only for vertically subsampled chroma)
 				if (ovl) { // per lane: a warp may hold the end of the first stripe and the start of the second
 					const int w_c = qq == 0 ? (ysh ? 20 : 12) : 24, w_u = qq == 0 ? (ysh ? 20 : 24) : 12;
@@ -432,6 +437,7 @@ VFGS_HD void gather_task_body(const FgsParams& p, smem_addr_t luts, smem_addr_t 
 			}
 			uint32_t w[4];
 			gather_finish<IN16, OUT8>(L, raw[qq], g, sc, w);
+			if constexpr (MSB && OB == 2) lsb_to_msb<4>(w);
 			const bool more = line + LB < nl;
 			gather_ld_if<IN16>(nxt, raw[qq], more);
 			if (!SHIFT) vh[qq] = ld_sample_if<IB>(nxt + halo_off, mem_halo && more);
@@ -450,7 +456,7 @@ VFGS_HD void gather_task_body(const FgsParams& p, smem_addr_t luts, smem_addr_t 
 
 // Gather-kernel task numbering: per frame the gather components one after the other, each cut into warp-tasks of
 // 32 consecutive flat units.
-template <bool IN16, bool OUT8, bool FOLD, bool SHIFT>
+template <bool IN16, bool OUT8, bool FOLD, bool SHIFT, bool MSB = false>
 VFGS_HD void process_task_gather(const FgsParams& p, smem_addr_t luts, smem_addr_t img, uint32_t task, int lane)
 {
 	const int f = (int)fastdiv(task, p.div_gtasks);
@@ -461,6 +467,11 @@ VFGS_HD void process_task_gather(const FgsParams& p, smem_addr_t luts, smem_addr
 #if !defined(__CUDA_ARCH__)
 	emu_warp().lane = lane; emu_warp().point = 0;
 #endif
+	if constexpr (MSB) { // luma only
+		if (SHIFT) gather_task_body<IN16, OUT8, 4, FOLD, true, true>(p, luts, img, f, c, q, lane);
+		else gather_task_body<IN16, OUT8, 4, FOLD, false, true>(p, luts, img, f, c, q, lane);
+		return;
+	}
 	if (SHIFT) gather_task_body<IN16, OUT8, 4, FOLD, true>(p, luts, img, f, c, q, lane); // the host never sends 8-sample blocks here
 	else if (c && p.subx > 1) gather_task_body<IN16, OUT8, 3, FOLD, false>(p, luts, img, f, c, q, lane);
 	else gather_task_body<IN16, OUT8, 4, FOLD, false>(p, luts, img, f, c, q, lane);

@@ -257,7 +257,8 @@ VFGS_HD void process_task(const FgsParams& p, const uint8_t* tab, uint32_t task,
 
 	const uint8_t* fin = pl.in + (long long)t.f * p.in_frame_bytes;
 	uint8_t* fout = pl.out + (long long)t.f * p.out_frame_bytes;
-	const bool full = pl.vec && (k0 + kSamplesPerLane <= pl.width);
+	const int ilv = p.ilv[c], msb_in = p.msb_in, msb_out = p.msb_out; // semi-planar: sample index k is at k << ilv
+	const bool full = pl.vec && !ilv && (k0 + kSamplesPerLane <= pl.width);
 	const bool need_nb = L.uniform_slot < 0;
 	const bool to8 = p.in_bytes == 2 && p.out_bytes == 1;
 
@@ -278,7 +279,7 @@ VFGS_HD void process_task(const FgsParams& p, const uint8_t* tab, uint32_t task,
 					// picture tail or unaligned rows: sample by sample, zero right of the picture
 					int s[8];
 #pragma unroll
-					for (int e = 0; e < 8; e++) s[e] = (k0 + e < pl.width) ? ld_sample(row, k0 + e, p.in_bytes) : 0;
+					for (int e = 0; e < 8; e++) s[e] = (k0 + e < pl.width) ? ld_sample(row, (k0 + e) << ilv, p.in_bytes) : 0;
 					if (p.in_bytes == 2) {
 #pragma unroll
 						for (int e = 0; e < 4; e++) raw[q][e] = (uint32_t)s[2 * e] | ((uint32_t)s[2 * e + 1] << 16);
@@ -288,8 +289,8 @@ VFGS_HD void process_task(const FgsParams& p, const uint8_t* tab, uint32_t task,
 							raw[q][e] = (uint32_t)s[4 * e] | ((uint32_t)s[4 * e + 1] << 8) | ((uint32_t)s[4 * e + 2] << 16) | ((uint32_t)s[4 * e + 3] << 24);
 					}
 				}
-				vl[q] = (need_nb && L.has_left) ? ld_sample(row, k0 - 1, p.in_bytes) : 0;
-				vr[q] = (need_nb && L.has_right && k0 + 8 < pl.width) ? ld_sample(row, k0 + 8, p.in_bytes) : 0;
+				vl[q] = (need_nb && L.has_left) ? ld_sample(row, (k0 - 1) << ilv, p.in_bytes) >> msb_in : 0;
+				vr[q] = (need_nb && L.has_right && k0 + 8 < pl.width) ? ld_sample(row, (k0 + 8) << ilv, p.in_bytes) >> msb_in : 0;
 			}
 		}
 #pragma unroll
@@ -300,7 +301,7 @@ VFGS_HD void process_task(const FgsParams& p, const uint8_t* tab, uint32_t task,
 				int v[8], o[8];
 				if (p.in_bytes == 2) {
 #pragma unroll
-					for (int e = 0; e < 4; e++) { v[2 * e] = raw[q][e] & 0xffff; v[2 * e + 1] = raw[q][e] >> 16; }
+					for (int e = 0; e < 4; e++) { v[2 * e] = (raw[q][e] & 0xffff) >> msb_in; v[2 * e + 1] = raw[q][e] >> (16 + msb_in); }
 				} else {
 #pragma unroll
 					for (int e = 0; e < 8; e++) v[e] = (raw[q][e >> 2] >> ((e & 3) * 8)) & 0xff;
@@ -315,7 +316,7 @@ VFGS_HD void process_task(const FgsParams& p, const uint8_t* tab, uint32_t task,
 					if (p.out_bytes == 2) {
 						uint32_t w[4];
 #pragma unroll
-						for (int e = 0; e < 4; e++) w[e] = (uint32_t)o[2 * e] | ((uint32_t)o[2 * e + 1] << 16);
+						for (int e = 0; e < 4; e++) w[e] = ((uint32_t)o[2 * e] << msb_out) | ((uint32_t)o[2 * e + 1] << (16 + msb_out));
 						st_global_16(orow + k0 * 2, w);
 					} else {
 						uint32_t w[2];
@@ -328,8 +329,8 @@ VFGS_HD void process_task(const FgsParams& p, const uint8_t* tab, uint32_t task,
 #pragma unroll
 					for (int e = 0; e < 8; e++)
 						if (k0 + e < pl.width) {
-							if (p.out_bytes == 2) ((uint16_t*)orow)[k0 + e] = (uint16_t)o[e];
-							else orow[k0 + e] = (uint8_t)o[e];
+							if (p.out_bytes == 2) ((uint16_t*)orow)[(k0 + e) << ilv] = (uint16_t)(o[e] << msb_out);
+							else orow[(k0 + e) << ilv] = (uint8_t)o[e];
 						}
 				}
 			}

@@ -172,10 +172,19 @@ int ensure_ctx(int device)
 		fgs_apply_fast_kernel<false, false><<<1, 32, 1024>>>(pp);
 		pp.probe = d_probe + 3;
 		fgs_apply_fast_kernel<true, false, false, true><<<1, 32, 1024>>>(pp);
-		uint32_t pads[4] = {0, 0, 0, 0};
+		pp.probe = d_probe + 4;
+		fgs_apply_fast_kernel<false, false, false, false, true><<<1, 32, 1024>>>(pp);
+		pp.probe = d_probe + 5;
+		fgs_apply_fast_kernel<true, true, false, false, true><<<1, 32, 1024>>>(pp);
+		pp.probe = d_probe + 6;
+		fgs_apply_fast_kernel<true, false, false, false, true><<<1, 32, 1024>>>(pp);
+		pp.probe = d_probe + 7;
+		fgs_apply_fast_kernel<true, false, false, true, true><<<1, 32, 1024>>>(pp);
+		uint32_t pads[8] = {0, 0, 0, 0, 0, 0, 0, 0};
 		CUDA_TRY(cudaMemcpy(pads, d_probe, sizeof(pads), cudaMemcpyDeviceToHost));
-		if (pads[0] != pads[1] || pads[0] != pads[2] || pads[0] != pads[3])
-			return set_err(VFGS_B200_ERR_CUDA, "fast kernel variants place dynamic shared memory differently (%u, %u, %u, %u)", pads[0], pads[1], pads[2], pads[3]);
+		for (int i = 1; i < 8; i++)
+			if (pads[i] != pads[0])
+				return set_err(VFGS_B200_ERR_CUDA, "fast kernel variants place dynamic shared memory differently (%u, %u)", pads[0], pads[i]);
 		c.fast_pad = (int)pads[0];
 	}
 	CUDA_TRY(cudaMemcpy(c.d_pow2, jump_table().pow2, sizeof(uint32_t) * kJumpBits * 32, cudaMemcpyHostToDevice));
@@ -317,6 +326,8 @@ enum KernelKind { kGeneral = 0, kFast = 1, kGather = 2, kFastEdge = 3 };
 template <bool FOLD, bool SHIFT>
 GrainKernel gather_kernel(const FgsParams& p)
 {
+	if (p.msb_in) // P010 luma of semi-planar frames
+		return p.out_bytes == 1 ? fgs_apply_gather_kernel<true, true, FOLD, SHIFT, true> : fgs_apply_gather_kernel<true, false, FOLD, SHIFT, true>;
 	return p.in_bytes == 1 ? fgs_apply_gather_kernel<false, false, FOLD, SHIFT>
 	     : p.out_bytes == 1 ? fgs_apply_gather_kernel<true, true, FOLD, SHIFT> : fgs_apply_gather_kernel<true, false, FOLD, SHIFT>;
 }
@@ -336,7 +347,11 @@ int launch_apply(const FgsParams& p, cudaStream_t stream, KernelKind kind = kGen
 	int threads = kCtaThreads, smem = p.blob_bytes;
 	if (kind == kFast || kind == kFastEdge) {
 		const bool allwide = kind == kFast && p.in_bytes == 2 && p.out_bytes == 2 && p.fallwide;
-		if (allwide)
+		if (kind == kFast && p.ilv[1]) // semi-planar frames
+			kern = allwide ? fgs_apply_fast_kernel<true, false, false, true, true>
+			     : p.in_bytes == 1 ? fgs_apply_fast_kernel<false, false, false, false, true>
+			     : p.out_bytes == 1 ? fgs_apply_fast_kernel<true, true, false, false, true> : fgs_apply_fast_kernel<true, false, false, false, true>;
+		else if (allwide)
 			kern = fgs_apply_fast_kernel<true, false, false, true>;
 		else if (kind == kFast)
 			kern = p.in_bytes == 1 ? fgs_apply_fast_kernel<false, false>
@@ -353,6 +368,10 @@ int launch_apply(const FgsParams& p, cudaStream_t stream, KernelKind kind = kGen
 			CUDA_TRY(cudaFuncSetAttribute(fgs_apply_fast_kernel<true, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
 			CUDA_TRY(cudaFuncSetAttribute(fgs_apply_fast_kernel<false, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
 			CUDA_TRY(cudaFuncSetAttribute(fgs_apply_fast_kernel<true, false, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+			CUDA_TRY(cudaFuncSetAttribute(fgs_apply_fast_kernel<false, false, false, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+			CUDA_TRY(cudaFuncSetAttribute(fgs_apply_fast_kernel<true, true, false, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+			CUDA_TRY(cudaFuncSetAttribute(fgs_apply_fast_kernel<true, false, false, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+			CUDA_TRY(cudaFuncSetAttribute(fgs_apply_fast_kernel<true, false, false, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
 			c.fast_smem_attr = smem;
 		}
 	} else if (kind == kGather) {
@@ -360,8 +379,9 @@ int launch_apply(const FgsParams& p, cudaStream_t stream, KernelKind kind = kGen
 		threads = kGatherThreads; smem = gather_smem;
 		if (smem > c.gather_smem_attr) {
 			FgsParams v = p; // every variant of the gather kernel
-			for (int io = 0; io < 3; io++) {
-				v.in_bytes = io == 0 ? 1 : 2; v.out_bytes = io == 2 ? 2 : 1;
+			for (int io = 0; io < 5; io++) {
+				v.in_bytes = io == 0 ? 1 : 2; v.out_bytes = io == 2 || io == 4 ? 2 : 1;
+				v.msb_in = io >= 3 ? 6 : 0;
 				for (int fs = 0; fs < 4; fs++)
 					CUDA_TRY(cudaFuncSetAttribute(gather_kernel(v, (fs & 1) != 0, (fs & 2) != 0), cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
 			}
@@ -422,8 +442,41 @@ void advance_registers(const Geometry& g, uint64_t nframes)
 	h.rnd_up = jt.jump(h.line_rnd_up, (uint64_t)g.nb);
 }
 
+// One side of a frame call: three planes (planar), or a Y plane and one plane of interleaved U,V pairs (semi-planar:
+// plane[1] holds both, plane[2] is unused).
+struct FramePlanes {
+	uint8_t* plane[3];
+	int64_t stride[3];
+	int64_t frame_stride;
+	bool semi, msb; // msb: P010 samples (value in bits 15..6)
+};
+FramePlanes frame_planes(const vfgs_b200_planes& pl)
+{
+	FramePlanes f;
+	f.plane[0] = (uint8_t*)pl.y; f.plane[1] = (uint8_t*)pl.u; f.plane[2] = (uint8_t*)pl.v;
+	f.stride[0] = pl.stride_y; f.stride[1] = f.stride[2] = pl.stride_c;
+	f.frame_stride = pl.frame_stride;
+	f.semi = f.msb = false;
+	return f;
+}
+FramePlanes frame_planes(const vfgs_b200_semiplanar& pl)
+{
+	FramePlanes f;
+	f.plane[0] = (uint8_t*)pl.y; f.plane[1] = (uint8_t*)pl.uv; f.plane[2] = nullptr;
+	f.stride[0] = pl.stride_y; f.stride[1] = pl.stride_uv; f.stride[2] = 0;
+	f.frame_stride = pl.frame_stride;
+	f.semi = true; f.msb = pl.format == VFGS_B200_P010;
+	return f;
+}
+// Bytes of one frame's row of plane c and its line count (0 for the unused plane of a semi-planar side).
+int64_t plane_row_bytes(const FramePlanes& f, int c, const Geometry& g, size_t sample)
+{
+	return (int64_t)(c ? (f.semi ? (c == 1 ? 2 * g.cw : 0) : g.cw) : g.width) * (int64_t)sample;
+}
+int64_t plane_lines(const FramePlanes& f, int c, const Geometry& g) { return (f.semi && c == 2) ? 0 : c ? g.ch : g.height; }
+
 // Launch parameters and kernel assignment of a whole-frame call.
-void plan_frames(const vfgs_b200_planes& in, const vfgs_b200_planes& out, int n, const Geometry& g, bool in_place,
+void plan_frames(const FramePlanes& in, const FramePlanes& out, int n, const Geometry& g, bool in_place,
                  uint32_t* d_streams, FgsParams& p, LaunchPlan& lp, uint16_t*& d_woffs)
 {
 	fill_common(p, g);
@@ -431,14 +484,17 @@ void plan_frames(const vfgs_b200_planes& in, const vfgs_b200_planes& out, int n,
 	p.y_begin = 0; p.y_end = g.height;
 	p.row_begin = 0; p.rows = g.R;
 	p.in_frame_bytes = in.frame_stride; p.out_frame_bytes = out.frame_stride;
-	const void* ip[3] = {in.y, in.u, in.v};
-	void* op[3] = {out.y, out.u, out.v};
-	for (int c = 0; c < 3; c++) {
-		p.comp[c].in = (const uint8_t*)ip[c]; p.comp[c].out = (uint8_t*)op[c];
-		p.comp[c].in_row_bytes = c ? in.stride_c : in.stride_y;
-		p.comp[c].out_row_bytes = c ? out.stride_c : out.stride_y;
-		p.comp[c].width = c ? g.cw : g.width;
-		p.comp[c].lines = c ? g.ch : g.height;
+	if (in.semi) {
+		set_semiplanar_planes(p, in.plane[0], in.plane[1], in.stride[0], in.stride[1], out.plane[0], out.plane[1], out.stride[0],
+		                      out.stride[1], g.width, g.height, g.cw, g.ch, in.msb, out.msb);
+	} else {
+		for (int c = 0; c < 3; c++) {
+			p.comp[c].in = in.plane[c]; p.comp[c].out = out.plane[c];
+			p.comp[c].in_row_bytes = in.stride[c];
+			p.comp[c].out_row_bytes = out.stride[c];
+			p.comp[c].width = c ? g.cw : g.width;
+			p.comp[c].lines = c ? g.ch : g.height;
+		}
 	}
 	// one allocation holds both per-block tables: uint32 registers, then 4 x uint16 window offsets
 	d_woffs = (uint16_t*)(d_streams + (((size_t)n * g.R * g.spitch + 3) & ~(size_t)3)); // 16-byte aligned
@@ -448,19 +504,8 @@ void plan_frames(const vfgs_b200_planes& in, const vfgs_b200_planes& out, int n,
 	plan_launches(p, g_bi, g_kernel_mode, in_place, g_ctx.max_smem_optin - 1024, g_ctx.fast_pad, lp);
 }
 
-// In place, a kernel must not read what another warp may already have overwritten. The fast kernel and the gather
-// kernel's 16-sample-block lanes read nothing but their own samples; the general kernel (and the gather kernel's
-// 8-sample-block halo lanes, which plan_launches therefore never uses in place) read a neighbouring block's INPUT
-// sample when the pattern slot depends on the sample: those calls go through a scratch output buffer.
-bool in_place_needs_scratch(const LaunchPlan& lp)
-{
-	for (int c = 0; c < 3; c++)
-		if (lp.kind[c] == 2 && g_bi.uniform_pi[c] < 0) return true;
-	return false;
-}
-
 // Streams + grain kernels for `n` frames whose epoch-relative index starts at frame0.
-int run_frames_device(const vfgs_b200_planes& in, const vfgs_b200_planes& out, int n, const Geometry& g, bool in_place,
+int run_frames_device(const FramePlanes& in, const FramePlanes& out, int n, const Geometry& g, bool in_place,
                       uint32_t epoch, uint64_t frame0, uint32_t* d_streams, cudaStream_t stream,
                       cudaStream_t table_stream = nullptr, cudaEvent_t table_ready = nullptr)
 {
@@ -485,35 +530,34 @@ int run_frames_device(const vfgs_b200_planes& in, const vfgs_b200_planes& out, i
 		if (int rc = launch_apply(lp.gather, stream, kGather, lp.gather_smem, lp.gather_fold, lp.gather_shift)) return rc;
 	if (lp.any_general)
 		if (int rc = launch_apply(lp.general, stream, kGeneral)) return rc;
+	if (lp.any_fast && in.semi && lp.fast.fwide[1]) g_ctx.last_launch[4] |= 16; // the interleaved U/V lane ran
 	return images_after(stream);
 }
 
 // How the output planes lie relative to the input planes: 0 disjoint, 1 in place (every overlapping plane pair is
-// the same plane with the same strides and sample size), -1 anything else (partial overlap: not supported).
+// the same plane with the same strides and row bytes), -1 anything else (partial overlap: not supported).
 // Planes of consecutive frames interleave in memory (Y0 U0 V0 Y1 ...), so plane pairs are compared frame by frame in
 // closed form: with a common frame stride S, frame f1 of one plane meets frame f2 of the other iff their byte
-// extents overlap for some k = f1 - f2 within the batch.
-int aliasing(const vfgs_b200_planes& in, const vfgs_b200_planes& out, int n, const Geometry& g)
+// extents overlap for some k = f1 - f2 within the batch. A semi-planar side has two planes (Y, interleaved UV).
+int aliasing(const FramePlanes& in, const FramePlanes& out, int n, const Geometry& g)
 {
-	const uint8_t* ip[3] = {(const uint8_t*)in.y, (const uint8_t*)in.u, (const uint8_t*)in.v};
-	const uint8_t* op[3] = {(const uint8_t*)out.y, (const uint8_t*)out.u, (const uint8_t*)out.v};
-	auto extent = [&](const vfgs_b200_planes& pl, int c, size_t sample) { // bytes one frame's plane spans
-		const int64_t lines = c ? g.ch : g.height, width = c ? g.cw : g.width;
-		if (lines < 1 || width < 1) return (int64_t)0;
-		return (lines - 1) * (c ? pl.stride_c : pl.stride_y) + width * (int64_t)sample;
+	auto extent = [&](const FramePlanes& pl, int c, size_t sample) { // bytes one frame's plane spans
+		const int64_t lines = plane_lines(pl, c, g), row = plane_row_bytes(pl, c, g, sample);
+		if (lines < 1 || row < 1) return (int64_t)0;
+		return (lines - 1) * pl.stride[c] + row;
 	};
 	// bounding ranges of the two calls' buffers
 	const uint8_t *ilo = nullptr, *ihi = nullptr, *olo = nullptr, *ohi = nullptr;
 	for (int c = 0; c < 3; c++) {
 		const int64_t ei = extent(in, c, g.in_sample), eo = extent(out, c, g.out_sample);
 		if (ei > 0) {
-			const uint8_t* e = ip[c] + (int64_t)(n - 1) * in.frame_stride + ei;
-			if (!ilo || ip[c] < ilo) ilo = ip[c];
+			const uint8_t* e = in.plane[c] + (int64_t)(n - 1) * in.frame_stride + ei;
+			if (!ilo || in.plane[c] < ilo) ilo = in.plane[c];
 			if (!ihi || e > ihi) ihi = e;
 		}
 		if (eo > 0) {
-			const uint8_t* e = op[c] + (int64_t)(n - 1) * out.frame_stride + eo;
-			if (!olo || op[c] < olo) olo = op[c];
+			const uint8_t* e = out.plane[c] + (int64_t)(n - 1) * out.frame_stride + eo;
+			if (!olo || out.plane[c] < olo) olo = out.plane[c];
 			if (!ohi || e > ohi) ohi = e;
 		}
 	}
@@ -525,20 +569,20 @@ int aliasing(const vfgs_b200_planes& in, const vfgs_b200_planes& out, int n, con
 		for (int j = 0; j < 3; j++) {
 			const int64_t ei = extent(in, i, g.in_sample), ej = extent(out, j, g.out_sample);
 			if (ei <= 0 || ej <= 0) continue;
-			const bool same = i == j && ip[i] == op[j] && g.in_sample == g.out_sample &&
-			                  (i ? in.stride_c == out.stride_c : in.stride_y == out.stride_y);
+			const bool same = i == j && in.plane[i] == out.plane[j] && in.stride[i] == out.stride[j] &&
+			                  plane_row_bytes(in, i, g, g.in_sample) == plane_row_bytes(out, j, g, g.out_sample) && in.msb == out.msb;
 			bool hit;
 			if (n > 1 && S > 0) {
 				// frame f1 of the input plane against frame f2 of the output plane: [f1 S, f1 S + ei) meets [D + f2 S, D + f2 S + ej)
 				// iff D - ei < k S < D + ej for k = f1 - f2, |k| <= n - 1
-				const int64_t D = (int64_t)(op[j] - ip[i]);
+				const int64_t D = (int64_t)(out.plane[j] - in.plane[i]);
 				auto floor_div = [](int64_t a, int64_t b) { int64_t q = a / b; return (a % b != 0 && ((a < 0) != (b < 0))) ? q - 1 : q; };
 				int64_t k_lo = floor_div(D - ei, S) + 1, k_hi = -floor_div(-(D + ej), S) - 1;
 				if (k_lo < -(int64_t)(n - 1)) k_lo = -(int64_t)(n - 1);
 				if (k_hi > (int64_t)(n - 1)) k_hi = (int64_t)(n - 1);
 				hit = k_lo <= k_hi;
 			} else {
-				hit = !(ip[i] + ei <= op[j] || op[j] + ej <= ip[i]);
+				hit = !(in.plane[i] + ei <= out.plane[j] || out.plane[j] + ej <= in.plane[i]);
 			}
 			if (!hit) continue;
 			if (!same) return -1;
@@ -559,6 +603,76 @@ int prepare(int device)
 {
 	if (int rc = ensure_ctx(device)) return rc;
 	return upload_blob();
+}
+
+// Body of the device frame entry points, after their own argument checks: overlap check (before any device work),
+// then the grain launches, through a scratch output buffer where in place would not be safe.
+int run_call(const FramePlanes& in, const FramePlanes& out, int nframes, const Geometry& g, cudaStream_t st)
+{
+	const int alias = nframes ? aliasing(in, out, nframes, g) : 0; // argument check first: needs no device
+	if (alias < 0)
+		return set_err(VFGS_B200_ERR_ARG, g.in_depth != g.out_depth ? "in-place needs equal depths"
+		               : "input and output planes overlap without being identical (same planes, strides and depth)");
+	if (int rc = prepare(-1)) return rc;
+	if (nframes == 0) return VFGS_B200_OK;
+	const bool in_place = alias == 1;
+	Context& c = g_ctx;
+	if (c.used_stream && c.last_stream != st) CUDA_TRY(cudaStreamSynchronize(c.last_stream)); // d_streams is shared
+	c.last_stream = st; c.used_stream = true;
+	bool scratch = false;
+	if (in_place) { // cheap host-side planning pass: which kernels would serve the components
+		FgsParams pp; LaunchPlan lpp; uint16_t* w = nullptr;
+		plan_frames(in, out, nframes, g, true, nullptr, pp, lpp, w);
+		scratch = in_place_needs_scratch(lpp, g_bi);
+	}
+	if (scratch) {
+		// In place with sample-adaptive pattern selection on a kernel that reads the neighbouring block's INPUT
+		// sample (see in_place_needs_scratch), which another warp may already have overwritten. The frames go
+		// through a scratch output buffer (packed, in the caller's layout) in sub-batches and are copied back (two
+		// extra passes over the data; the reference's own in-place order, block after block along a line, has no
+		// such hazard).
+		const size_t fb = g.out_frame_bytes;
+		int per = (int)((256u << 20) / fb);
+		if (per < 1) per = 1;
+		if (per > nframes) per = nframes;
+		if (int rc = grow(c.d_scratch, c.scratch_cap, (size_t)per * fb)) return rc;
+		if (int rc = grow(c.d_streams, c.streams_cap, (size_t)per * g.R * g.spitch * kBlockTableBytes + 16)) return rc;
+		const uint32_t epoch = hw().line_rnd;
+		const int nplanes = in.semi ? 2 : 3;
+		FramePlanes po = out;
+		size_t soff[3] = {0, 0, 0};
+		for (int k = 0; k < nplanes; k++) { // packed scratch frames: the planes back to back, rows tightly packed
+			po.stride[k] = plane_row_bytes(out, k, g, g.out_sample);
+			if (k + 1 < 3) soff[k + 1] = soff[k] + (size_t)po.stride[k] * (size_t)plane_lines(out, k, g);
+		}
+		po.frame_stride = (int64_t)fb;
+		for (int f0 = 0; f0 < nframes; f0 += per) {
+			const int n = nframes - f0 < per ? nframes - f0 : per;
+			FramePlanes pi = in;
+			for (int k = 0; k < nplanes; k++) {
+				pi.plane[k] = in.plane[k] + (size_t)f0 * in.frame_stride;
+				po.plane[k] = c.d_scratch + soff[k];
+			}
+			if (int rc = run_frames_device(pi, po, n, g, false, epoch, (uint64_t)f0, c.d_streams, st)) return rc;
+			for (int f = 0; f < n; f++) // rows of the caller's planes may be padded: 2-D copies, plane by plane
+				for (int k = 0; k < nplanes; k++) {
+					const size_t row = (size_t)po.stride[k];
+					CUDA_TRY(cudaMemcpy2DAsync(out.plane[k] + (size_t)(f0 + f) * out.frame_stride, (size_t)out.stride[k],
+					                           c.d_scratch + (size_t)f * fb + soff[k], row, row, (size_t)plane_lines(out, k, g),
+					                           cudaMemcpyDeviceToDevice, st));
+				}
+		}
+		advance_registers(g, (uint64_t)nframes);
+		return VFGS_B200_OK;
+	}
+	const int t = (int)(c.tab_next++ & 1u);
+	if (int rc = grow(c.d_tab[t], c.tab_cap[t], (size_t)nframes * g.R * g.spitch * kBlockTableBytes + 16)) return rc;
+	if (c.tab_used[t]) CUDA_TRY(cudaStreamWaitEvent(c.s_tab, c.tab_free[t], 0)); // the grain kernels of two calls ago read this buffer
+	if (int rc = run_frames_device(in, out, nframes, g, in_place, hw().line_rnd, 0, c.d_tab[t], st, c.s_tab, c.tab_ready[t])) return rc;
+	CUDA_TRY(cudaEventRecord(c.tab_free[t], st));
+	c.tab_used[t] = true;
+	advance_registers(g, (uint64_t)nframes);
+	return VFGS_B200_OK;
 }
 
 } // namespace
@@ -741,66 +855,33 @@ int vfgs_b200_add_grain_planes_device(const vfgs_b200_planes* in, const vfgs_b20
 	if (!in || !out || nframes < 0) return set_err(VFGS_B200_ERR_ARG, "null planes or negative frame count");
 	Geometry g;
 	if (int rc = make_geometry(g, width, height, out_depth)) return rc;
-	const int alias = nframes ? aliasing(*in, *out, nframes, g) : 0; // argument check first: needs no device
-	if (alias < 0)
-		return set_err(VFGS_B200_ERR_ARG, g.in_depth != g.out_depth ? "in-place needs equal depths"
-		               : "input and output planes overlap without being identical (same planes, strides and depth)");
-	if (int rc = prepare(-1)) return rc;
-	if (nframes == 0) return VFGS_B200_OK;
-	const bool in_place = alias == 1;
-	Context& c = g_ctx;
-	cudaStream_t st = (cudaStream_t)stream;
-	if (c.used_stream && c.last_stream != st) CUDA_TRY(cudaStreamSynchronize(c.last_stream)); // d_streams is shared
-	c.last_stream = st; c.used_stream = true;
-	bool scratch = false;
-	if (in_place) { // cheap host-side planning pass: which kernels would serve the components
-		FgsParams pp; LaunchPlan lpp; uint16_t* w = nullptr;
-		plan_frames(*in, *out, nframes, g, true, nullptr, pp, lpp, w);
-		scratch = in_place_needs_scratch(lpp);
+	return run_call(frame_planes(*in), frame_planes(*out), nframes, g, (cudaStream_t)stream);
+}
+
+int vfgs_b200_add_grain_semiplanar_device(const vfgs_b200_semiplanar* in, const vfgs_b200_semiplanar* out, int nframes,
+                                          int width, int height, void* stream)
+{
+	if (!in || !out || nframes < 0) return set_err(VFGS_B200_ERR_ARG, "null planes or negative frame count");
+	if (!in->y || !in->uv || !out->y || !out->uv) return set_err(VFGS_B200_ERR_ARG, "null plane pointer");
+	const HwState& h = hw();
+	const int depth = 8 + h.bs;
+	if (in->format != (depth == 10 ? VFGS_B200_P010 : VFGS_B200_NV12))
+		return set_err(VFGS_B200_ERR_ARG, "input format %d does not match the configured depth %d (NV12 = 8, P010 = 10)", in->format, depth);
+	if (out->format != in->format && !(out->format == VFGS_B200_NV12 && in->format == VFGS_B200_P010))
+		return set_err(VFGS_B200_ERR_ARG, "output format %d from input format %d (same format, or NV12 from P010)", out->format, in->format);
+	if (h.csubx != 2)
+		return set_err(VFGS_B200_ERR_ARG, "semi-planar frames are 4:2:0 or 4:2:2 (4:4:4 frames are planar)");
+	Geometry g;
+	if (int rc = make_geometry(g, width, height, out->format == in->format ? 0 : 8)) return rc;
+	for (int side = 0; side < 2; side++) {
+		const vfgs_b200_semiplanar& f = side ? *out : *in;
+		const int64_t sample = (int64_t)(side ? g.out_sample : g.in_sample);
+		if (f.stride_y < (int64_t)g.width * sample || f.stride_uv < 2 * (int64_t)g.cw * sample)
+			return set_err(VFGS_B200_ERR_ARG, "%s line stride shorter than a row", side ? "output" : "input");
+		if (sample == 2 && (((uintptr_t)f.y | (uintptr_t)f.uv | (uint64_t)f.stride_y | (uint64_t)f.stride_uv | (uint64_t)f.frame_stride) & 1))
+			return set_err(VFGS_B200_ERR_ARG, "%s P010 planes and strides must be 2-byte aligned", side ? "output" : "input");
 	}
-	if (scratch) {
-		// In place with sample-adaptive pattern selection on a kernel that reads the neighbouring block's INPUT
-		// sample (see in_place_needs_scratch), which another warp may already have overwritten. The frames go
-		// through a scratch output buffer in sub-batches and are copied back (two extra passes over the data; the
-		// reference's own in-place order, block after block along a line, has no such hazard).
-		const size_t fb = g.out_frame_bytes;
-		int per = (int)((256u << 20) / fb);
-		if (per < 1) per = 1;
-		if (per > nframes) per = nframes;
-		if (int rc = grow(c.d_scratch, c.scratch_cap, (size_t)per * fb)) return rc;
-		if (int rc = grow(c.d_streams, c.streams_cap, (size_t)per * g.R * g.spitch * kBlockTableBytes + 16)) return rc;
-		const uint32_t epoch = hw().line_rnd;
-		const size_t ysz = g.ysam * g.out_sample, csz = g.csam * g.out_sample;
-		for (int f0 = 0; f0 < nframes; f0 += per) {
-			const int n = nframes - f0 < per ? nframes - f0 : per;
-			vfgs_b200_planes pi = *in, po;
-			pi.y = (uint8_t*)in->y + (size_t)f0 * in->frame_stride;
-			pi.u = (uint8_t*)in->u + (size_t)f0 * in->frame_stride;
-			pi.v = (uint8_t*)in->v + (size_t)f0 * in->frame_stride;
-			packed_planes(po, c.d_scratch, g, g.out_sample, g.out_frame_bytes);
-			if (int rc = run_frames_device(pi, po, n, g, false, epoch, (uint64_t)f0, c.d_streams, st)) return rc;
-			for (int f = 0; f < n; f++) { // rows of the caller's planes may be padded: 2-D copies, plane by plane
-				const uint8_t* s = c.d_scratch + (size_t)f * fb;
-				uint8_t* dy = (uint8_t*)out->y + (size_t)(f0 + f) * out->frame_stride;
-				uint8_t* du = (uint8_t*)out->u + (size_t)(f0 + f) * out->frame_stride;
-				uint8_t* dv = (uint8_t*)out->v + (size_t)(f0 + f) * out->frame_stride;
-				const size_t yrow = (size_t)g.width * g.out_sample, crow = (size_t)g.cw * g.out_sample;
-				CUDA_TRY(cudaMemcpy2DAsync(dy, (size_t)out->stride_y, s, yrow, yrow, (size_t)g.height, cudaMemcpyDeviceToDevice, st));
-				CUDA_TRY(cudaMemcpy2DAsync(du, (size_t)out->stride_c, s + ysz, crow, crow, (size_t)g.ch, cudaMemcpyDeviceToDevice, st));
-				CUDA_TRY(cudaMemcpy2DAsync(dv, (size_t)out->stride_c, s + ysz + csz, crow, crow, (size_t)g.ch, cudaMemcpyDeviceToDevice, st));
-			}
-		}
-		advance_registers(g, (uint64_t)nframes);
-		return VFGS_B200_OK;
-	}
-	const int t = (int)(c.tab_next++ & 1u);
-	if (int rc = grow(c.d_tab[t], c.tab_cap[t], (size_t)nframes * g.R * g.spitch * kBlockTableBytes + 16)) return rc;
-	if (c.tab_used[t]) CUDA_TRY(cudaStreamWaitEvent(c.s_tab, c.tab_free[t], 0)); // the grain kernels of two calls ago read this buffer
-	if (int rc = run_frames_device(*in, *out, nframes, g, in_place, hw().line_rnd, 0, c.d_tab[t], st, c.s_tab, c.tab_ready[t])) return rc;
-	CUDA_TRY(cudaEventRecord(c.tab_free[t], st));
-	c.tab_used[t] = true;
-	advance_registers(g, (uint64_t)nframes);
-	return VFGS_B200_OK;
+	return run_call(frame_planes(*in), frame_planes(*out), nframes, g, (cudaStream_t)stream);
 }
 
 int vfgs_b200_add_grain_frames_device(const void* in, void* out, int nframes, int width, int height,
@@ -855,7 +936,7 @@ int vfgs_b200_add_grain_frames_host(const void* in, void* out, int nframes, int 
 		vfgs_b200_planes pi, po;
 		packed_planes(pi, s.d_in, g, g.in_sample, g.in_frame_bytes);
 		packed_planes(po, s.d_out, g, g.out_sample, g.out_frame_bytes);
-		if (int rc = run_frames_device(pi, po, n, g, false, epoch, (uint64_t)f0, s.d_streams, c.s_k)) return rc;
+		if (int rc = run_frames_device(frame_planes(pi), frame_planes(po), n, g, false, epoch, (uint64_t)f0, s.d_streams, c.s_k)) return rc;
 		CUDA_TRY(cudaEventRecord(s.k_done, c.s_k));
 		CUDA_TRY(cudaStreamWaitEvent(c.s_d2h, s.k_done, 0));
 		CUDA_TRY(cudaMemcpyAsync(hout + (size_t)f0 * g.out_frame_bytes, s.d_out, (size_t)n * g.out_frame_bytes, cudaMemcpyDeviceToHost, c.s_d2h));

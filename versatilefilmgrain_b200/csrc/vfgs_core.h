@@ -210,6 +210,12 @@ struct FgsParams {
 	// same indexing, four uint16 per block: byte offset (inside the fast image, block sign folded in) of the
 	// block's pattern window for Y, U, V (fast path only; written by lfsr_states_kernel)
 	const uint16_t* woffs;
+	// semi-planar frames (NV12 / P010, vfgs_b200_add_grain_semiplanar_device): U and V alternate on one plane.
+	// General kernel: comp[1] / comp[2] are views of that plane starting at U0 / V0 whose samples are every second
+	// one (ilv). Fast kernel (SEMI variants): comp[1] is the whole interleaved plane, comp[2] carries no tasks.
+	// msb_in / msb_out: 16-bit samples hold the value in bits 15..6 (P010): shift on load / store.
+	int ilv[3];
+	int msb_in, msb_out;
 };
 
 } // namespace vfgs

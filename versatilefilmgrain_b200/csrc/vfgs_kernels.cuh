@@ -166,7 +166,8 @@ inline int fast_threads(bool in16, bool out8, bool edge = false, bool allwide = 
 	return allwide ? VFGS_FAST_THREADS16W : edge ? VFGS_FAST_THREADS_EDGE : !in16 ? VFGS_FAST_THREADS_IN8 : out8 ? VFGS_FAST_THREADS8 : VFGS_FAST_THREADS16;
 }
 
-template <bool IN16, bool OUT8, bool EDGE = false, bool ALLWIDE = false>
+// SEMI: semi-planar frames (process_task_fast), same CTA sizes as the planar variants.
+template <bool IN16, bool OUT8, bool EDGE = false, bool ALLWIDE = false, bool SEMI = false>
 __global__ void __launch_bounds__(FastCta<IN16, OUT8, EDGE, ALLWIDE>::threads, 1)
 fgs_apply_fast_kernel(const __grid_constant__ FgsParams p)
 {
@@ -200,7 +201,7 @@ fgs_apply_fast_kernel(const __grid_constant__ FgsParams p)
 	const smem_addr_t lut = smem_addr(lut_ptr);
 	const long long stride = (long long)gridDim.x * kFastWarps;
 	for (long long task = (long long)blockIdx.x * kFastWarps + (threadIdx.x >> 5); task < p.total_tasks; task += stride)
-		process_task_fast<IN16, OUT8, EDGE, ALLWIDE>(p, lut, (uint32_t)task, lane);
+		process_task_fast<IN16, OUT8, EDGE, ALLWIDE, SEMI>(p, lut, (uint32_t)task, lane);
 }
 
 // Gather path: components with sample-adaptive pattern selection (fgs_gather.h). Shared memory: one
@@ -215,7 +216,8 @@ constexpr int kGatherThreads = VFGS_GATHER_THREADS; // one CTA per SM at up to 7
                                                     // measured ahead of 2 x 384 (one table image per SM) and of 640-832 and 960-1024 threads
 constexpr int kGatherWarps = kGatherThreads / 32;
 
-template <bool IN16, bool OUT8, bool FOLD, bool SHIFT>
+// MSB: P010 luma of semi-planar frames (16-bit input only).
+template <bool IN16, bool OUT8, bool FOLD, bool SHIFT, bool MSB = false>
 __global__ void __launch_bounds__(kGatherThreads, VFGS_GATHER_CTAS)
 fgs_apply_gather_kernel(const __grid_constant__ FgsParams p)
 {
@@ -247,7 +249,7 @@ fgs_apply_gather_kernel(const __grid_constant__ FgsParams p)
 	const smem_addr_t luts = smem_addr(lut_ptr), img = smem_addr(img_ptr);
 	const long long stride = (long long)gridDim.x * kGatherWarps;
 	for (long long task = (long long)blockIdx.x * kGatherWarps + (threadIdx.x >> 5); task < p.total_tasks; task += stride)
-		process_task_gather<IN16, OUT8, FOLD, SHIFT>(p, luts, img, (uint32_t)task, lane);
+		process_task_gather<IN16, OUT8, FOLD, SHIFT, MSB>(p, luts, img, (uint32_t)task, lane);
 }
 
 // ---- firmware layer: one pattern job (fw_device.h) -----------------------------------------------

@@ -195,6 +195,26 @@ inline bool aligned_for(const void* base, long long row, long long frame, size_t
 	return ((uintptr_t)base % unit) == 0 && (row % (long long)unit) == 0 && (frame % (long long)unit) == 0;
 }
 
+// Planes of a semi-planar call (NV12 / P010): comp[0] is the luma plane, comp[1] / comp[2] are views of the interleaved
+// UV plane that start at U0 / V0 and step over the other component's samples (FgsParams::ilv). msb_*: 16-bit samples
+// in bits 15..6. Set before finish_tasks.
+inline void set_semiplanar_planes(FgsParams& p, const uint8_t* y_in, const uint8_t* uv_in, long long sy_in, long long suv_in,
+                                  uint8_t* y_out, uint8_t* uv_out, long long sy_out, long long suv_out, int width, int height,
+                                  int cw, int ch, bool msb_in, bool msb_out)
+{
+	for (int c = 0; c < 3; c++) {
+		p.comp[c].in = c ? uv_in + (c - 1) * p.in_bytes : y_in;
+		p.comp[c].out = c ? uv_out + (c - 1) * p.out_bytes : y_out;
+		p.comp[c].in_row_bytes = c ? suv_in : sy_in;
+		p.comp[c].out_row_bytes = c ? suv_out : sy_out;
+		p.comp[c].width = c ? cw : width;
+		p.comp[c].lines = c ? ch : height;
+		p.ilv[c] = c ? 1 : 0;
+	}
+	p.msb_in = msb_in ? 6 : 0;
+	p.msb_out = msb_out ? 6 : 0;
+}
+
 // Segments per line, vector-access eligibility and the task count, once planes and sizes are set.
 inline void finish_tasks(FgsParams& p)
 {
@@ -257,9 +277,32 @@ inline void plan_launches(const FgsParams& p, const TableInfo& bi, int mode, boo
 	lp.any_fast = lp.any_gather = lp.any_general = lp.any_edge = false;
 	int* kind = lp.kind;
 	int ngather = 0;
+	// semi-planar frames (FgsParams::ilv): U and V alternate on one plane, so they take ONE kind of kernel (two launches
+	// must not write alternate samples of the same words): the fast kernel's interleaved lane when both are single-slot
+	// and the plane allows one access per line and lane, else the general kernel. 16-bit (P010) luma takes the wide fast
+	// path or the gather kernel, both with the MSB conversion, else the general kernel; 8-bit (NV12) luma is a planar plane,
+	// except that the SEMI fast kernel serves it on the wide path only: where planar rows would take 8 samples per lane,
+	// it takes the (planar) EDGE variant.
+	const bool semi = p.ilv[1] != 0;
 	for (int c = 0; c < 3; c++) {
 		const bool aligned = p.comp[c].vec && (p.comp[c].width % kSamplesPerLane) == 0;
 		kind[c] = 2;
+		if (semi && c) {
+			if (mode == 0 && bi.fast_ok[1] && bi.fast_ok[2] && p.comp[0].width % 16 == 0 &&
+			    aligned_for(p.comp[1].in, p.comp[1].in_row_bytes, p.in_frame_bytes, (size_t)(16 * p.in_bytes)) &&
+			    aligned_for(p.comp[1].out, p.comp[1].out_row_bytes, p.out_frame_bytes, (size_t)(16 * p.out_bytes)))
+				kind[c] = 0;
+			continue;
+		}
+		if (semi && p.msb_in) {
+			const bool wide = VFGS_FAST_WIDE16 != 0 && p.comp[0].width % 16 == 0 &&
+			                  aligned_for(p.comp[0].in, p.comp[0].in_row_bytes, p.in_frame_bytes, (size_t)(16 * p.in_bytes)) &&
+			                  aligned_for(p.comp[0].out, p.comp[0].out_row_bytes, p.out_frame_bytes, (size_t)(16 * p.out_bytes));
+			if (mode == 0 && bi.fast_ok[0] && wide) kind[c] = 0;
+			else if (mode != 1 && aligned && (!bi.fast_ok[0] || mode == 2)) kind[c] = 1;
+			if (kind[c] == 1) ngather++;
+			continue;
+		}
 		if (aligned && mode != 1) {
 			// in place: the gather kernel's shifted numbering (SHIFT) reads nothing but a lane's own samples, but exists for
 			// 16-sample blocks only; the aligned numbering recomputes the warps' outer neighbours from INPUT samples
@@ -276,6 +319,10 @@ inline void plan_launches(const FgsParams& p, const TableInfo& bi, int mode, boo
 		    aligned_for(p.comp[c].out, p.comp[c].out_row_bytes, p.out_frame_bytes, (size_t)p.out_bytes))
 			kind[c] = 3;
 #endif
+		if (semi && kind[c] == 0 &&
+		    !(VFGS_FAST_WIDE8 != 0 && p.comp[0].width % 16 == 0 && aligned_for(p.comp[0].in, p.comp[0].in_row_bytes, p.in_frame_bytes, 16) &&
+		      aligned_for(p.comp[0].out, p.comp[0].out_row_bytes, p.out_frame_bytes, 16)))
+			kind[c] = 3;
 		if (kind[c] == 1) ngather++;
 	}
 	for (int which = 0; which < 2; which++) { // the fast kernel's tables must fit as well (plain launch, EDGE launch)
@@ -323,13 +370,17 @@ inline void plan_launches(const FgsParams& p, const TableInfo& bi, int mode, boo
 			             aligned_for(f.comp[c].in, f.comp[c].in_row_bytes, f.in_frame_bytes, (size_t)(16 * f.in_bytes)) &&
 			             aligned_for(f.comp[c].out, f.comp[c].out_row_bytes, f.out_frame_bytes, (size_t)(16 * f.out_bytes));
 			f.funits_per_row[c] = kind[c] == k ? (f.comp[c].width + (f.fwide[c] ? 16 : kSamplesPerLane) - 1) / (f.fwide[c] ? 16 : kSamplesPerLane) : 0;
+			if (semi && c) { // the interleaved lane: one unit per chroma block of U and V (8 samples each), on component 1 only
+				f.fwide[c] = c == 1 && kind[1] == k;
+				f.funits_per_row[c] = f.fwide[c] ? f.comp[1].width / 8 : 0;
+			}
 			f.ftasks[c] = (f.funits_per_row[c] * f.rows + 31) / 32;
 			f.ftasks_per_frame += f.ftasks[c];
 			f.div_funits[c] = make_fastdiv((uint32_t)(f.funits_per_row[c] > 0 ? f.funits_per_row[c] : 1));
 		}
 		f.div_ftasks = make_fastdiv((uint32_t)(f.ftasks_per_frame > 0 ? f.ftasks_per_frame : 1));
 		int served = 0, wide = 0;
-		for (int c = 0; c < 3; c++) if (kind[c] == k) { served++; wide += f.fwide[c] ? 1 : 0; }
+		for (int c = 0; c < (semi ? 2 : 3); c++) if (kind[c] == k) { served++; wide += f.fwide[c] ? 1 : 0; }
 		f.fallwide = served > 0 && wide == served;
 	}
 	lp.gather_shift = in_place && ngather > 0;
@@ -361,6 +412,17 @@ inline void plan_launches(const FgsParams& p, const TableInfo& bi, int mode, boo
 	lp.fast.total_tasks = (long long)lp.fast.nframes * lp.fast.ftasks_per_frame;
 	lp.edge.total_tasks = (long long)lp.edge.nframes * lp.edge.ftasks_per_frame;
 	lp.gather.total_tasks = (long long)lp.gather.nframes * lp.gather.gtasks_per_frame;
+}
+
+// In place, a kernel must not read what another warp may already have overwritten. The fast kernel and the gather
+// kernel's 16-sample-block lanes read nothing but their own samples; the general kernel (and the gather kernel's
+// 8-sample-block halo lanes, which plan_launches therefore never uses in place) read a neighbouring block's INPUT
+// sample when the pattern slot depends on the sample: those calls go through a scratch output buffer.
+inline bool in_place_needs_scratch(const LaunchPlan& lp, const TableInfo& bi)
+{
+	for (int c = 0; c < 3; c++)
+		if (lp.kind[c] == 2 && bi.uniform_pi[c] < 0) return true;
+	return false;
 }
 
 // What lfsr_states_kernel needs to turn a block register into a pattern-window offset (FgsParams::woffs).
