@@ -153,6 +153,52 @@ void vfgs_b200_pipeline_stats(unsigned long long out[2]);
  * U/V lane of semi-planar frames). */
 void vfgs_b200_last_launch(int out[5]);
 
+/* ---- Grain sessions: many video streams, each with its own grain state, served by one batched call ----------------
+ *
+ * A session owns a copy of one complete hardware state (patterns, LUTs, scalars, the four LFSR registers) and that
+ * state's table images in device memory, built once. Calls on sessions neither read nor change the global state of the
+ * setters, vfgs_b200_init_sei / _afgs1 and the frame entry points above; setters do not affect existing sessions, and
+ * vfgs_b200_reset leaves them alive. A session belongs to the device the library is bound to. Like the rest of the
+ * library, sessions and job calls are used from one thread at a time. */
+typedef struct vfgs_b200_session vfgs_b200_session;
+
+/* Snapshot of the current hardware state (whatever the setters / vfgs_b200_init_sei / _afgs1 programmed, LFSR registers
+ * included), with its table images uploaded asynchronously to session-owned device memory. VFGS_B200_ERR_STATE when
+ * the state could never add grain (a pattern LUT entry above slot 8, scale_shift + bs outside 8..13). */
+int  vfgs_b200_session_create(vfgs_b200_session** out);
+/* Waits for the kernels that read this session (its last use only), then frees it. NULL is a no-op. */
+void vfgs_b200_session_destroy(vfgs_b200_session* s);
+/* The session's LFSR registers, order as vfgs_b200_get_lfsr. */
+void vfgs_b200_session_get_lfsr(const vfgs_b200_session* s, uint32_t regs[4]);
+void vfgs_b200_session_set_lfsr(vfgs_b200_session* s, const uint32_t regs[4]);
+/* vfgs_b200_skip_frames on the session's registers. */
+int  vfgs_b200_session_skip_frames(vfgs_b200_session* s, int64_t nframes, int width, int height);
+/* The session's state in the layout of vfgs_b200_get_state. */
+size_t vfgs_b200_session_get_state(const vfgs_b200_session* s, void* dst, size_t cap);
+
+/* One job: nframes frames of one session, in device memory. */
+typedef struct vfgs_b200_job {
+	vfgs_b200_session* session;
+	const vfgs_b200_planes* in;         /* planar frames ... */
+	const vfgs_b200_planes* out;
+	const vfgs_b200_semiplanar* sp_in;  /* ... or semi-planar ones: exactly one of the two pairs is set */
+	const vfgs_b200_semiplanar* sp_out;
+	int nframes, width, height;
+	int out_depth;                      /* planar jobs, as in vfgs_b200_add_grain_planes_device; 0 for semi-planar */
+} vfgs_b200_job;
+
+/* njobs jobs in DEVICE memory, asynchronous on `stream`. Output and the registers of every session afterwards are
+ * exactly what one vfgs_b200_add_grain_planes_device / _semiplanar_device call per job, in list order, would give, each
+ * made on its session's state and registers. A session may appear in several jobs; each then starts where the previous
+ * one left its registers (which advance on the host at enqueue).
+ *   Launches: one LFSR stream-kernel launch for all jobs, then one grain launch per kernel instantiation the jobs need
+ *   (the fast kernel's variants, its EDGE variant, the gather kernel's variants). A job whose plan needs the general
+ *   kernel, or in place the scratch detour, runs on its own through the single-job route.
+ *   Refused with VFGS_B200_ERR_ARG / _ERR_STATE before any device work: everything the single-job entry points refuse,
+ *   a null session, both or neither plane pairs set, njobs < 0, and buffers of two jobs that overlap (in place within
+ *   one job is allowed as in the single-job calls). */
+int vfgs_b200_add_grain_jobs_device(const vfgs_b200_job* jobs, int njobs, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -4,5 +4,5 @@ The product is the C-ABI shared library ``libvfgs_b200.so`` (sources in ``csrc/`
 ``include/vfgs_hw.h`` + ``include/vfgs_b200.h``). This package only builds it and mirrors its
 interface for Python callers (tests, bench); there is no Python or CPU compute path.
 """
-from .api import VfgsHw, VfgsError, load_library, LIB_PATH  # noqa: F401
+from .api import Job, Session, VfgsHw, VfgsError, load_library, LIB_PATH  # noqa: F401
 from .build import build  # noqa: F401

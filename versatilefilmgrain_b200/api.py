@@ -3,8 +3,9 @@
 ``VfgsHw`` exposes the ten functions of the reference's ``src/vfgs_hw.h:51-62`` (bound to the CUDA
 shim) plus the additive frame entry points of ``include/vfgs_b200.h``. Like the reference there is
 ONE hardware state per process (``src/vfgs_hw.c:49-63`` are file-scope statics), so every instance
-talks to the same state. Nothing here computes grain: without the compiled CUDA library the import
-of the library fails loudly.
+talks to the same state. ``Session`` objects (``VfgsHw.create_session``) hold independent copies of
+it, one per video stream, which ``VfgsHw.add_grain_jobs_device`` serves in one batched call. Nothing
+here computes grain: without the compiled CUDA library the import of the library fails loudly.
 """
 from __future__ import annotations
 
@@ -28,7 +29,9 @@ B200_SYMBOLS = (
     "vfgs_b200_set_lfsr", "vfgs_b200_host_alloc", "vfgs_b200_host_free", "vfgs_b200_launch_count",
     "vfgs_b200_last_launch", "vfgs_b200_get_state", "vfgs_b200_kernel_timing", "vfgs_b200_kernel_time",
     "vfgs_b200_force_general_kernel", "vfgs_b200_pipeline_stats", "vfgs_b200_init_sei", "vfgs_b200_init_afgs1",
-    "vfgs_b200_add_grain_semiplanar_device",
+    "vfgs_b200_add_grain_semiplanar_device", "vfgs_b200_session_create", "vfgs_b200_session_destroy",
+    "vfgs_b200_session_get_lfsr", "vfgs_b200_session_set_lfsr", "vfgs_b200_session_skip_frames",
+    "vfgs_b200_session_get_state", "vfgs_b200_add_grain_jobs_device",
 )
 NV12, P010 = 1, 2  # VFGS_B200_NV12 / VFGS_B200_P010
 
@@ -59,6 +62,24 @@ def surface_planes(t, height: int, fmt: int) -> SemiPlanes:
     pitch = t.shape[2] * t.element_size()
     base = t.data_ptr()
     return SemiPlanes(base, base + height * pitch, pitch, pitch, t.shape[1] * pitch, fmt)
+
+
+class _CJob(C.Structure):
+    """vfgs_b200_job (include/vfgs_b200.h)."""
+    _fields_ = [("session", C.c_void_p), ("in_", C.POINTER(Planes)), ("out", C.POINTER(Planes)),
+                ("sp_in", C.POINTER(SemiPlanes)), ("sp_out", C.POINTER(SemiPlanes)),
+                ("nframes", C.c_int), ("width", C.c_int), ("height", C.c_int), ("out_depth", C.c_int)]
+
+
+def _state_dict(raw: np.ndarray) -> dict:
+    o = 2 * 9 * 64 * 64
+    return {
+        "pattern": raw[:o].view(np.int8).reshape(2, 9, 64, 64).copy(),
+        "slut": raw[o:o + 768].reshape(3, 256).copy(),
+        "plut": raw[o + 768:o + 1536].reshape(3, 256).copy(),
+        "lfsr": raw[o + 1536:o + 1552].view(np.uint32).copy(),
+        "scalars": raw[o + 1552:o + 1584].view(np.int32).copy(),
+    }
 
 
 _lib = None
@@ -116,6 +137,17 @@ def load_library(global_symbols: bool = False) -> C.CDLL:
     L.vfgs_b200_init_afgs1.argtypes = [vp]
     L.vfgs_b200_get_state.argtypes = [vp, C.c_size_t]
     L.vfgs_b200_get_state.restype = C.c_size_t
+    L.vfgs_b200_session_create.argtypes = [C.POINTER(vp)]
+    L.vfgs_b200_session_destroy.argtypes = [vp]
+    L.vfgs_b200_session_destroy.restype = None
+    L.vfgs_b200_session_get_lfsr.argtypes = [vp, vp]
+    L.vfgs_b200_session_get_lfsr.restype = None
+    L.vfgs_b200_session_set_lfsr.argtypes = [vp, vp]
+    L.vfgs_b200_session_set_lfsr.restype = None
+    L.vfgs_b200_session_skip_frames.argtypes = [vp, C.c_int64, ci, ci]
+    L.vfgs_b200_session_get_state.argtypes = [vp, vp, C.c_size_t]
+    L.vfgs_b200_session_get_state.restype = C.c_size_t
+    L.vfgs_b200_add_grain_jobs_device.argtypes = [C.POINTER(_CJob), ci, vp]
     _lib = L
     return L
 
@@ -192,15 +224,7 @@ class VfgsHw:
         n = self.L.vfgs_b200_get_state(None, 0)
         buf = (C.c_uint8 * n)()
         self.L.vfgs_b200_get_state(buf, n)
-        raw = np.frombuffer(bytes(buf), dtype=np.uint8)
-        o = 2 * 9 * 64 * 64
-        return {
-            "pattern": raw[:o].view(np.int8).reshape(2, 9, 64, 64).copy(),
-            "slut": raw[o:o + 768].reshape(3, 256).copy(),
-            "plut": raw[o + 768:o + 1536].reshape(3, 256).copy(),
-            "lfsr": raw[o + 1536:o + 1552].view(np.uint32).copy(),
-            "scalars": raw[o + 1552:o + 1584].view(np.int32).copy(),
-        }
+        return _state_dict(np.frombuffer(bytes(buf), dtype=np.uint8))
 
     def get_lfsr(self):
         r = (C.c_uint32 * 4)()
@@ -250,3 +274,107 @@ class VfgsHw:
         def ptr(x):
             return _np_ptr(x) if isinstance(x, np.ndarray) else C.c_void_p(x.data_ptr())
         self._chk(self.L.vfgs_b200_add_grain_frames_host(ptr(src), ptr(dst), nframes, width, height, out_depth))
+
+    # ---- sessions: one grain state per video stream, many streams per call -------------------------
+    def create_session(self) -> "Session":
+        """Snapshot of the current hardware state (registers included) as an independent session."""
+        h = C.c_void_p()
+        self._chk(self.L.vfgs_b200_session_create(C.byref(h)))
+        return Session(self, h.value)
+
+    def add_grain_jobs_device(self, jobs, stream=None):
+        """jobs: a list of ``Job``s (device memory). One batched call, asynchronous on ``stream`` (a torch.cuda.Stream;
+        default: torch's current stream), equal to one single-job call per job in list order."""
+        import torch
+        if stream is None:
+            stream = torch.cuda.current_stream()
+        arr = (_CJob * max(len(jobs), 1))()
+        for k, j in enumerate(jobs):
+            c = arr[k]
+            c.session = j.session.handle if j.session is not None else None
+            if isinstance(j.src, SemiPlanes) or isinstance(j.dst, SemiPlanes):
+                c.sp_in, c.sp_out = (C.pointer(j.src) if j.src is not None else None), (C.pointer(j.dst) if j.dst is not None else None)
+            else:
+                c.in_, c.out = (C.pointer(j.src) if j.src is not None else None), (C.pointer(j.dst) if j.dst is not None else None)
+            c.nframes, c.width, c.height, c.out_depth = j.nframes, j.width, j.height, j.out_depth
+        self._chk(self.L.vfgs_b200_add_grain_jobs_device(arr, len(jobs), C.c_void_p(stream.cuda_stream)))
+
+
+class Session:
+    """One video stream's grain state (vfgs_b200_session): patterns, LUTs, scalars and LFSR registers, independent of
+    the global state and of other sessions. ``close()`` (or leaving a ``with`` block) frees it once the kernels that
+    read it are done."""
+
+    def __init__(self, hw: VfgsHw, handle: int):
+        self.hw, self.L, self.handle = hw, hw.L, handle
+        sc = self.get_state()["scalars"]
+        self.depth, self.csubx, self.csuby = 8 + int(sc[1]), int(sc[6]), int(sc[7])
+
+    def close(self):
+        if self.handle:
+            self.L.vfgs_b200_session_destroy(C.c_void_p(self.handle))
+            self.handle = None
+
+    def __enter__(self):
+        return self
+
+    def __exit__(self, *exc):
+        self.close()
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+    def get_lfsr(self):
+        r = (C.c_uint32 * 4)()
+        self.L.vfgs_b200_session_get_lfsr(C.c_void_p(self.handle), r)
+        return [int(v) for v in r]
+
+    def set_lfsr(self, regs):
+        r = (C.c_uint32 * 4)(*[int(v) & 0xFFFFFFFF for v in regs])
+        self.L.vfgs_b200_session_set_lfsr(C.c_void_p(self.handle), r)
+
+    def skip_frames(self, n, width, height):
+        self.hw._chk(self.L.vfgs_b200_session_skip_frames(C.c_void_p(self.handle), n, width, height))
+
+    def get_state(self) -> dict:
+        n = self.L.vfgs_b200_session_get_state(C.c_void_p(self.handle), None, 0)
+        buf = (C.c_uint8 * n)()
+        self.L.vfgs_b200_session_get_state(C.c_void_p(self.handle), buf, n)
+        return _state_dict(np.frombuffer(bytes(buf), dtype=np.uint8))
+
+    def frame_bytes(self, width, height, depth):
+        """Bytes of one packed planar frame with this session's chroma subsampling."""
+        s = 2 if depth > 8 else 1
+        return (width * height + 2 * (width // self.csubx) * (height // self.csuby)) * s
+
+
+class Job:
+    """One job of VfgsHw.add_grain_jobs_device: ``nframes`` frames of ``session`` from ``src`` to ``dst`` (a ``Planes``
+    or a ``SemiPlanes`` pair). ``tensors`` keeps the buffers the planes point into alive."""
+
+    def __init__(self, session, src, dst, nframes, width, height, out_depth=0, tensors=()):
+        self.session, self.src, self.dst = session, src, dst
+        self.nframes, self.width, self.height, self.out_depth = nframes, width, height, out_depth
+        self.tensors = tensors
+
+    @classmethod
+    def packed(cls, session: Session, src, dst, nframes, width, height, out_depth=0) -> "Job":
+        """Packed planar frames (the layout of add_grain_frames_device) in CUDA tensors, with the session's subsampling."""
+        def planes(t, depth):
+            s = 2 if depth > 8 else 1
+            cw, ch = width // session.csubx, height // session.csuby
+            b = t.data_ptr()
+            return Planes(b, b + width * height * s, b + (width * height + cw * ch) * s, width * s, cw * s,
+                          session.frame_bytes(width, height, depth))
+        od = out_depth or session.depth
+        return cls(session, planes(src, session.depth), planes(dst, od), nframes, width, height, out_depth, (src, dst))
+
+    @classmethod
+    def surfaces(cls, session: Session, src, dst, nframes, width, height, out_format=None) -> "Job":
+        """Decoder-style surfaces (surface_planes): CUDA tensors of shape (n, height + ch, pitch)."""
+        in_fmt = P010 if src.element_size() == 2 else NV12
+        return cls(session, surface_planes(src, height, in_fmt), surface_planes(dst, height, out_format or in_fmt), nframes,
+                   width, height, 0, (src, dst))

@@ -9,6 +9,8 @@
 #include <stdlib.h>
 #include <string.h>
 #include <time.h>
+#include <algorithm>
+#include <memory>
 #include <mutex>
 #include <thread>
 #include <vector>
@@ -75,6 +77,17 @@ struct Context {
 	cudaEvent_t tab_ready[2] = {nullptr, nullptr}, tab_free[2] = {nullptr, nullptr};
 	bool tab_used[2] = {false, false};
 	unsigned tab_next = 0;
+	// descriptors of a batched call (vfgs_b200_add_grain_jobs_device): stream-kernel job table, per-job launch
+	// parameters and task prefixes, staged in page-locked memory and copied on the table stream; they alternate with
+	// d_tab (same tab_free events); desc_copied: the staging buffer may be rewritten
+	uint8_t* h_desc[2] = {nullptr, nullptr};
+	uint8_t* d_desc[2] = {nullptr, nullptr};
+	size_t desc_cap[2] = {0, 0}, hdesc_cap[2] = {0, 0};
+	cudaEvent_t desc_copied[2] = {nullptr, nullptr};
+	bool desc_used[2] = {false, false};
+	int multi_smem_attr[512] = {}; // per group key (group_key): the MULTI kernel's dynamic shared memory attribute
+	int multi_occ_smem[512] = {}, multi_per_sm[512] = {}; // per group key: occupancy asked for that shared-memory size
+	std::vector<std::shared_ptr<CUevent_st>> call_events; // end-of-call events of batched calls, reused once no session holds one
 	Slot slot[kPipeSlots];
 	uint8_t* d_line = nullptr; // compat line path staging
 	size_t line_cap = 0;
@@ -180,9 +193,27 @@ int ensure_ctx(int device)
 		fgs_apply_fast_kernel<true, false, false, false, true><<<1, 32, 1024>>>(pp);
 		pp.probe = d_probe + 7;
 		fgs_apply_fast_kernel<true, false, false, true, true><<<1, 32, 1024>>>(pp);
-		uint32_t pads[8] = {0, 0, 0, 0, 0, 0, 0, 0};
+		MultiParams mp; // the MULTI forms of the same variants (batched calls)
+		memset(&mp, 0, sizeof(mp));
+		mp.probe = d_probe + 8;
+		fgs_apply_fast_multi_kernel<true, false><<<1, 32, 1024>>>(mp);
+		mp.probe = d_probe + 9;
+		fgs_apply_fast_multi_kernel<true, true><<<1, 32, 1024>>>(mp);
+		mp.probe = d_probe + 10;
+		fgs_apply_fast_multi_kernel<false, false><<<1, 32, 1024>>>(mp);
+		mp.probe = d_probe + 11;
+		fgs_apply_fast_multi_kernel<true, false, false, true><<<1, 32, 1024>>>(mp);
+		mp.probe = d_probe + 12;
+		fgs_apply_fast_multi_kernel<false, false, false, false, true><<<1, 32, 1024>>>(mp);
+		mp.probe = d_probe + 13;
+		fgs_apply_fast_multi_kernel<true, true, false, false, true><<<1, 32, 1024>>>(mp);
+		mp.probe = d_probe + 14;
+		fgs_apply_fast_multi_kernel<true, false, false, false, true><<<1, 32, 1024>>>(mp);
+		mp.probe = d_probe + 15;
+		fgs_apply_fast_multi_kernel<true, false, false, true, true><<<1, 32, 1024>>>(mp);
+		uint32_t pads[16] = {};
 		CUDA_TRY(cudaMemcpy(pads, d_probe, sizeof(pads), cudaMemcpyDeviceToHost));
-		for (int i = 1; i < 8; i++)
+		for (int i = 1; i < 16; i++)
 			if (pads[i] != pads[0])
 				return set_err(VFGS_B200_ERR_CUDA, "fast kernel variants place dynamic shared memory differently (%u, %u)", pads[0], pads[i]);
 		c.fast_pad = (int)pads[0];
@@ -195,6 +226,7 @@ int ensure_ctx(int device)
 	for (int t = 0; t < 2; t++) {
 		CUDA_TRY(cudaEventCreateWithFlags(&c.tab_ready[t], cudaEventDisableTiming));
 		CUDA_TRY(cudaEventCreateWithFlags(&c.tab_free[t], cudaEventDisableTiming));
+		CUDA_TRY(cudaEventCreateWithFlags(&c.desc_copied[t], cudaEventDisableTiming));
 	}
 	for (ImageSet& m : c.img) { // fixed-size allocations: nothing is (re)allocated, hence nothing synchronises, on a configuration change
 		CUDA_TRY(cudaMalloc((void**)&m.d_blob, kImageBlobCap));
@@ -257,19 +289,25 @@ int upload_blob()
 	return VFGS_B200_OK;
 }
 
-// Grain kernels about to be launched on `stream` read the current image set: they wait for its upload, and the set
+// The state a grain launch works on: the global one (g_hw, g_bi, the current image set) or a session's copy.
+struct StateRef {
+	HwState* h;
+	const TableInfo* bi;
+	ImageSet* img;
+};
+StateRef global_state() { return {&hw(), &g_bi, g_ctx.img_cur >= 0 ? &g_ctx.img[g_ctx.img_cur] : nullptr}; }
+
+// Grain kernels about to be launched on `stream` read the state's image set: they wait for its upload, and the set
 // remembers the last stream position that reads it.
-int images_before(cudaStream_t stream)
+int images_before(const StateRef& s, cudaStream_t stream)
 {
-	ImageSet& m = g_ctx.img[g_ctx.img_cur];
-	CUDA_TRY(cudaStreamWaitEvent(stream, m.uploaded, 0));
+	CUDA_TRY(cudaStreamWaitEvent(stream, s.img->uploaded, 0));
 	return VFGS_B200_OK;
 }
-int images_after(cudaStream_t stream)
+int images_after(const StateRef& s, cudaStream_t stream)
 {
-	ImageSet& m = g_ctx.img[g_ctx.img_cur];
-	CUDA_TRY(cudaEventRecord(m.last_use, stream));
-	m.in_use = true;
+	CUDA_TRY(cudaEventRecord(s.img->last_use, stream));
+	s.img->in_use = true;
 	return VFGS_B200_OK;
 }
 
@@ -282,9 +320,8 @@ struct Geometry {
 	size_t in_frame_bytes, out_frame_bytes;
 };
 
-int make_geometry(Geometry& g, int width, int height, int out_depth)
+int make_geometry(Geometry& g, const HwState& h, int width, int height, int out_depth)
 {
-	const HwState& h = hw();
 	// what add_grain_block asserts (vfgs_hw.c:168-170)
 	if (width <= 128) return set_err(VFGS_B200_ERR_STATE, "width must exceed 128 (vfgs_hw.c:168)");
 	if (h.scale_shift + h.bs < 8 || h.scale_shift + h.bs > 13)
@@ -308,15 +345,16 @@ int make_geometry(Geometry& g, int width, int height, int out_depth)
 	g.out_frame_bytes = (g.ysam + 2 * g.csam) * g.out_sample;
 	return VFGS_B200_OK;
 }
+int make_geometry(Geometry& g, int width, int height, int out_depth) { return make_geometry(g, hw(), width, height, out_depth); }
 
-void fill_common(FgsParams& p, const Geometry& g)
+void fill_common(FgsParams& p, const Geometry& g, const StateRef& s)
 {
 	memset(&p, 0, sizeof(p));
-	fill_state_params(p, hw(), g_bi);
+	fill_state_params(p, *s.h, *s.bi);
 	p.nb = g.nb; p.R = g.R;
 	p.in_bytes = (int)g.in_sample; p.out_bytes = (int)g.out_sample;
-	p.blob = g_ctx.img_cur >= 0 ? g_ctx.img[g_ctx.img_cur].d_blob : nullptr;
-	p.fblob = g_ctx.img_cur >= 0 ? g_ctx.img[g_ctx.img_cur].d_fblob : nullptr;
+	p.blob = s.img ? s.img->d_blob : nullptr;
+	p.fblob = s.img ? s.img->d_fblob : nullptr;
 	p.spitch = g.spitch;
 }
 
@@ -427,20 +465,7 @@ int launch_streams(uint32_t epoch, uint32_t* d_streams, uint16_t* d_woffs, const
 }
 
 // Register state after nframes whole frames (vfgs_hw.c:291-298,309-310 in closed form).
-void advance_registers(const Geometry& g, uint64_t nframes)
-{
-	if (!nframes) return;
-	HwState& h = hw();
-	const JumpTable& jt = jump_table();
-	const uint32_t s0 = h.line_rnd;
-	const uint64_t adv = nframes * (uint64_t)(g.R - 1) * (uint64_t)g.nb;
-	if (g.R >= 2) {
-		h.line_rnd_up = jt.jump(s0, adv - (uint64_t)g.nb);
-		h.line_rnd = jt.jump(s0, adv);
-	}
-	h.rnd = jt.jump(h.line_rnd, (uint64_t)g.nb);
-	h.rnd_up = jt.jump(h.line_rnd_up, (uint64_t)g.nb);
-}
+void advance_registers(HwState& h, const Geometry& g, uint64_t nframes) { advance_frames(h, g.R, g.nb, nframes, jump_table()); }
 
 // One side of a frame call: three planes (planar), or a Y plane and one plane of interleaved U,V pairs (semi-planar:
 // plane[1] holds both, plane[2] is unused).
@@ -476,10 +501,10 @@ int64_t plane_row_bytes(const FramePlanes& f, int c, const Geometry& g, size_t s
 int64_t plane_lines(const FramePlanes& f, int c, const Geometry& g) { return (f.semi && c == 2) ? 0 : c ? g.ch : g.height; }
 
 // Launch parameters and kernel assignment of a whole-frame call.
-void plan_frames(const FramePlanes& in, const FramePlanes& out, int n, const Geometry& g, bool in_place,
+void plan_frames(const StateRef& s, const FramePlanes& in, const FramePlanes& out, int n, const Geometry& g, bool in_place,
                  uint32_t* d_streams, FgsParams& p, LaunchPlan& lp, uint16_t*& d_woffs)
 {
-	fill_common(p, g);
+	fill_common(p, g, s);
 	p.nframes = n;
 	p.y_begin = 0; p.y_end = g.height;
 	p.row_begin = 0; p.rows = g.R;
@@ -501,18 +526,18 @@ void plan_frames(const FramePlanes& in, const FramePlanes& out, int n, const Geo
 	p.states = d_streams; p.woffs = d_woffs; p.stream_rows = g.R; p.stream_row0 = 0;
 	finish_tasks(p);
 	// every component goes to the cheapest kernel that can serve it (plan_launches)
-	plan_launches(p, g_bi, g_kernel_mode, in_place, g_ctx.max_smem_optin - 1024, g_ctx.fast_pad, lp);
+	plan_launches(p, *s.bi, g_kernel_mode, in_place, g_ctx.max_smem_optin - 1024, g_ctx.fast_pad, lp);
 }
 
 // Streams + grain kernels for `n` frames whose epoch-relative index starts at frame0.
-int run_frames_device(const FramePlanes& in, const FramePlanes& out, int n, const Geometry& g, bool in_place,
+int run_frames_device(const StateRef& s, const FramePlanes& in, const FramePlanes& out, int n, const Geometry& g, bool in_place,
                       uint32_t epoch, uint64_t frame0, uint32_t* d_streams, cudaStream_t stream,
                       cudaStream_t table_stream = nullptr, cudaEvent_t table_ready = nullptr)
 {
 	FgsParams p;
 	LaunchPlan lp;
 	uint16_t* d_woffs = nullptr;
-	plan_frames(in, out, n, g, in_place, d_streams, p, lp, d_woffs);
+	plan_frames(s, in, out, n, g, in_place, d_streams, p, lp, d_woffs);
 	g_ctx.last_launch[4] = 0;
 	// the register table feeds the general kernel, the window-offset table the fast and gather kernels
 	if (int rc = launch_streams(epoch, lp.any_general ? d_streams : nullptr, (lp.any_fast || lp.any_gather || lp.any_edge) ? d_woffs : nullptr,
@@ -521,7 +546,7 @@ int run_frames_device(const FramePlanes& in, const FramePlanes& out, int n, cons
 		CUDA_TRY(cudaEventRecord(table_ready, table_stream));
 		CUDA_TRY(cudaStreamWaitEvent(stream, table_ready, 0));
 	}
-	if (int rc = images_before(stream)) return rc;
+	if (int rc = images_before(s, stream)) return rc;
 	if (lp.any_fast)
 		if (int rc = launch_apply(lp.fast, stream, kFast)) return rc;
 	if (lp.any_edge)
@@ -531,7 +556,7 @@ int run_frames_device(const FramePlanes& in, const FramePlanes& out, int n, cons
 	if (lp.any_general)
 		if (int rc = launch_apply(lp.general, stream, kGeneral)) return rc;
 	if (lp.any_fast && in.semi && lp.fast.fwide[1]) g_ctx.last_launch[4] |= 16; // the interleaved U/V lane ran
-	return images_after(stream);
+	return images_after(s, stream);
 }
 
 // How the output planes lie relative to the input planes: 0 disjoint, 1 in place (every overlapping plane pair is
@@ -539,56 +564,68 @@ int run_frames_device(const FramePlanes& in, const FramePlanes& out, int n, cons
 // Planes of consecutive frames interleave in memory (Y0 U0 V0 Y1 ...), so plane pairs are compared frame by frame in
 // closed form: with a common frame stride S, frame f1 of one plane meets frame f2 of the other iff their byte
 // extents overlap for some k = f1 - f2 within the batch. A semi-planar side has two planes (Y, interleaved UV).
-int aliasing(const FramePlanes& in, const FramePlanes& out, int n, const Geometry& g)
+// One side of an overlap test: planes, frame count, geometry and bytes per sample.
+struct Side {
+	const FramePlanes& f;
+	int n;
+	const Geometry& g;
+	size_t sample;
+};
+int64_t plane_extent(const Side& s, int c) // bytes one frame's plane spans
 {
-	auto extent = [&](const FramePlanes& pl, int c, size_t sample) { // bytes one frame's plane spans
-		const int64_t lines = plane_lines(pl, c, g), row = plane_row_bytes(pl, c, g, sample);
-		if (lines < 1 || row < 1) return (int64_t)0;
-		return (lines - 1) * pl.stride[c] + row;
-	};
-	// bounding ranges of the two calls' buffers
-	const uint8_t *ilo = nullptr, *ihi = nullptr, *olo = nullptr, *ohi = nullptr;
+	const int64_t lines = plane_lines(s.f, c, s.g), row = plane_row_bytes(s.f, c, s.g, s.sample);
+	if (lines < 1 || row < 1) return 0;
+	return (lines - 1) * s.f.stride[c] + row;
+}
+// Bounding byte range [lo, hi) of a side's buffers (lo null: no bytes).
+void side_span(const Side& s, const uint8_t*& lo, const uint8_t*& hi)
+{
+	lo = hi = nullptr;
 	for (int c = 0; c < 3; c++) {
-		const int64_t ei = extent(in, c, g.in_sample), eo = extent(out, c, g.out_sample);
-		if (ei > 0) {
-			const uint8_t* e = in.plane[c] + (int64_t)(n - 1) * in.frame_stride + ei;
-			if (!ilo || in.plane[c] < ilo) ilo = in.plane[c];
-			if (!ihi || e > ihi) ihi = e;
-		}
-		if (eo > 0) {
-			const uint8_t* e = out.plane[c] + (int64_t)(n - 1) * out.frame_stride + eo;
-			if (!olo || out.plane[c] < olo) olo = out.plane[c];
-			if (!ohi || e > ohi) ohi = e;
-		}
+		const int64_t e = plane_extent(s, c);
+		if (e <= 0) continue;
+		const uint8_t* end = s.f.plane[c] + (int64_t)(s.n - 1) * s.f.frame_stride + e;
+		if (!lo || s.f.plane[c] < lo) lo = s.f.plane[c];
+		if (!hi || end > hi) hi = end;
 	}
-	if (!ilo || !olo || ihi <= olo || ohi <= ilo) return 0;
-	if (n > 1 && in.frame_stride != out.frame_stride) return -1; // overlapping buffers walked with different strides
-	const int64_t S = in.frame_stride;
+}
+int overlap(const Side& a, const Side& b)
+{
+	const uint8_t *alo, *ahi, *blo, *bhi;
+	side_span(a, alo, ahi);
+	side_span(b, blo, bhi);
+	if (!alo || !blo || ahi <= blo || bhi <= alo) return 0;
+	if (a.n > 1 && b.n > 1 && a.f.frame_stride != b.f.frame_stride) return -1; // overlapping buffers walked with different strides
+	const int64_t S = a.n > 1 ? a.f.frame_stride : b.f.frame_stride;
 	int result = 0;
 	for (int i = 0; i < 3; i++)
 		for (int j = 0; j < 3; j++) {
-			const int64_t ei = extent(in, i, g.in_sample), ej = extent(out, j, g.out_sample);
+			const int64_t ei = plane_extent(a, i), ej = plane_extent(b, j);
 			if (ei <= 0 || ej <= 0) continue;
-			const bool same = i == j && in.plane[i] == out.plane[j] && in.stride[i] == out.stride[j] &&
-			                  plane_row_bytes(in, i, g, g.in_sample) == plane_row_bytes(out, j, g, g.out_sample) && in.msb == out.msb;
+			const bool same = i == j && a.f.plane[i] == b.f.plane[j] && a.f.stride[i] == b.f.stride[j] &&
+			                  plane_row_bytes(a.f, i, a.g, a.sample) == plane_row_bytes(b.f, j, b.g, b.sample) && a.f.msb == b.f.msb;
 			bool hit;
-			if (n > 1 && S > 0) {
-				// frame f1 of the input plane against frame f2 of the output plane: [f1 S, f1 S + ei) meets [D + f2 S, D + f2 S + ej)
-				// iff D - ei < k S < D + ej for k = f1 - f2, |k| <= n - 1
-				const int64_t D = (int64_t)(out.plane[j] - in.plane[i]);
-				auto floor_div = [](int64_t a, int64_t b) { int64_t q = a / b; return (a % b != 0 && ((a < 0) != (b < 0))) ? q - 1 : q; };
+			if ((a.n > 1 || b.n > 1) && S > 0) {
+				// frame f1 of plane i against frame f2 of plane j: [f1 S, f1 S + ei) meets [D + f2 S, D + f2 S + ej)
+				// iff D - ei < k S < D + ej for k = f1 - f2, -(b.n - 1) <= k <= a.n - 1
+				const int64_t D = (int64_t)(b.f.plane[j] - a.f.plane[i]);
+				auto floor_div = [](int64_t x, int64_t y) { int64_t q = x / y; return (x % y != 0 && ((x < 0) != (y < 0))) ? q - 1 : q; };
 				int64_t k_lo = floor_div(D - ei, S) + 1, k_hi = -floor_div(-(D + ej), S) - 1;
-				if (k_lo < -(int64_t)(n - 1)) k_lo = -(int64_t)(n - 1);
-				if (k_hi > (int64_t)(n - 1)) k_hi = (int64_t)(n - 1);
+				if (k_lo < -(int64_t)(b.n - 1)) k_lo = -(int64_t)(b.n - 1);
+				if (k_hi > (int64_t)(a.n - 1)) k_hi = (int64_t)(a.n - 1);
 				hit = k_lo <= k_hi;
 			} else {
-				hit = !(in.plane[i] + ei <= out.plane[j] || out.plane[j] + ej <= in.plane[i]);
+				hit = !(a.f.plane[i] + ei <= b.f.plane[j] || b.f.plane[j] + ej <= a.f.plane[i]);
 			}
 			if (!hit) continue;
 			if (!same) return -1;
 			result = 1;
 		}
 	return result;
+}
+int aliasing(const FramePlanes& in, const FramePlanes& out, int n, const Geometry& g)
+{
+	return overlap({in, n, g, g.in_sample}, {out, n, g, g.out_sample});
 }
 
 void packed_planes(vfgs_b200_planes& pl, const void* base, const Geometry& g, size_t sample, size_t frame_bytes)
@@ -599,33 +636,76 @@ void packed_planes(vfgs_b200_planes& pl, const void* base, const Geometry& g, si
 	pl.frame_stride = (int64_t)frame_bytes;
 }
 
+// Argument checks of a semi-planar call on state h, before any device work, and its geometry.
+int semiplanar_geometry(Geometry& g, const HwState& h, const vfgs_b200_semiplanar& in, const vfgs_b200_semiplanar& out, int width, int height)
+{
+	if (!in.y || !in.uv || !out.y || !out.uv) return set_err(VFGS_B200_ERR_ARG, "null plane pointer");
+	const int depth = 8 + h.bs;
+	if (in.format != (depth == 10 ? VFGS_B200_P010 : VFGS_B200_NV12))
+		return set_err(VFGS_B200_ERR_ARG, "input format %d does not match the configured depth %d (NV12 = 8, P010 = 10)", in.format, depth);
+	if (out.format != in.format && !(out.format == VFGS_B200_NV12 && in.format == VFGS_B200_P010))
+		return set_err(VFGS_B200_ERR_ARG, "output format %d from input format %d (same format, or NV12 from P010)", out.format, in.format);
+	if (h.csubx != 2)
+		return set_err(VFGS_B200_ERR_ARG, "semi-planar frames are 4:2:0 or 4:2:2 (4:4:4 frames are planar)");
+	if (int rc = make_geometry(g, h, width, height, out.format == in.format ? 0 : 8)) return rc;
+	for (int side = 0; side < 2; side++) {
+		const vfgs_b200_semiplanar& f = side ? out : in;
+		const int64_t sample = (int64_t)(side ? g.out_sample : g.in_sample);
+		if (f.stride_y < (int64_t)g.width * sample || f.stride_uv < 2 * (int64_t)g.cw * sample)
+			return set_err(VFGS_B200_ERR_ARG, "%s line stride shorter than a row", side ? "output" : "input");
+		if (sample == 2 && (((uintptr_t)f.y | (uintptr_t)f.uv | (uint64_t)f.stride_y | (uint64_t)f.stride_uv | (uint64_t)f.frame_stride) & 1))
+			return set_err(VFGS_B200_ERR_ARG, "%s P010 planes and strides must be 2-byte aligned", side ? "output" : "input");
+	}
+	return VFGS_B200_OK;
+}
+
+// Mirror of a hardware state in the layout of the reference's statics (see oracle/ref_harness.c refh_state):
+// pattern[2][9][64][64], sLUT[3][256], pLUT[3][256], 4 LFSR registers, then scale_shift, bs, Y_min, Y_max, C_min, C_max,
+// csubx, csuby as ints (vfgs_b200_get_state, vfgs_b200_session_get_state).
+size_t state_dump(const HwState& h, void* dst, size_t cap)
+{
+	const size_t need = sizeof(h.pattern) + sizeof(h.slut) + sizeof(h.plut) + 4 * sizeof(uint32_t) + 8 * sizeof(int);
+	if (!dst || cap < need) return need;
+	uint8_t* p = (uint8_t*)dst;
+	memcpy(p, h.pattern, sizeof(h.pattern)); p += sizeof(h.pattern);
+	memcpy(p, h.slut, sizeof(h.slut)); p += sizeof(h.slut);
+	memcpy(p, h.plut, sizeof(h.plut)); p += sizeof(h.plut);
+	const uint32_t regs[4] = {h.rnd, h.rnd_up, h.line_rnd, h.line_rnd_up};
+	memcpy(p, regs, sizeof(regs)); p += sizeof(regs);
+	const int sc[8] = {h.scale_shift, h.bs, h.y_min, h.y_max, h.c_min, h.c_max, h.csubx, h.csuby};
+	memcpy(p, sc, sizeof(sc));
+	return need;
+}
+
 int prepare(int device)
 {
 	if (int rc = ensure_ctx(device)) return rc;
 	return upload_blob();
 }
 
-// Body of the device frame entry points, after their own argument checks: overlap check (before any device work),
-// then the grain launches, through a scratch output buffer where in place would not be safe.
-int run_call(const FramePlanes& in, const FramePlanes& out, int nframes, const Geometry& g, cudaStream_t st)
+// An in-place call whose plan puts a sample-adaptive component on the general kernel (in_place_needs_scratch).
+bool needs_scratch(const StateRef& s, const FramePlanes& in, const FramePlanes& out, int nframes, const Geometry& g)
 {
-	const int alias = nframes ? aliasing(in, out, nframes, g) : 0; // argument check first: needs no device
-	if (alias < 0)
-		return set_err(VFGS_B200_ERR_ARG, g.in_depth != g.out_depth ? "in-place needs equal depths"
-		               : "input and output planes overlap without being identical (same planes, strides and depth)");
-	if (int rc = prepare(-1)) return rc;
-	if (nframes == 0) return VFGS_B200_OK;
-	const bool in_place = alias == 1;
+	FgsParams pp; LaunchPlan lpp; uint16_t* w = nullptr; // cheap host-side planning pass: which kernels would serve the components
+	plan_frames(s, in, out, nframes, g, true, nullptr, pp, lpp, w);
+	return in_place_needs_scratch(lpp, *s.bi);
+}
+
+int stream_switch(cudaStream_t st)
+{
 	Context& c = g_ctx;
 	if (c.used_stream && c.last_stream != st) CUDA_TRY(cudaStreamSynchronize(c.last_stream)); // d_streams is shared
 	c.last_stream = st; c.used_stream = true;
-	bool scratch = false;
-	if (in_place) { // cheap host-side planning pass: which kernels would serve the components
-		FgsParams pp; LaunchPlan lpp; uint16_t* w = nullptr;
-		plan_frames(in, out, nframes, g, true, nullptr, pp, lpp, w);
-		scratch = in_place_needs_scratch(lpp, g_bi);
-	}
-	if (scratch) {
+	return VFGS_B200_OK;
+}
+
+// Grain launches of one whole-frame call on state `s` (its registers advance), through a scratch output buffer where
+// in place would not be safe. alias: what aliasing() found (0 or 1).
+int run_job(const StateRef& s, const FramePlanes& in, const FramePlanes& out, int nframes, const Geometry& g, int alias, cudaStream_t st)
+{
+	const bool in_place = alias == 1;
+	Context& c = g_ctx;
+	if (in_place && needs_scratch(s, in, out, nframes, g)) {
 		// In place with sample-adaptive pattern selection on a kernel that reads the neighbouring block's INPUT
 		// sample (see in_place_needs_scratch), which another warp may already have overwritten. The frames go
 		// through a scratch output buffer (packed, in the caller's layout) in sub-batches and are copied back (two
@@ -637,7 +717,7 @@ int run_call(const FramePlanes& in, const FramePlanes& out, int nframes, const G
 		if (per > nframes) per = nframes;
 		if (int rc = grow(c.d_scratch, c.scratch_cap, (size_t)per * fb)) return rc;
 		if (int rc = grow(c.d_streams, c.streams_cap, (size_t)per * g.R * g.spitch * kBlockTableBytes + 16)) return rc;
-		const uint32_t epoch = hw().line_rnd;
+		const uint32_t epoch = s.h->line_rnd;
 		const int nplanes = in.semi ? 2 : 3;
 		FramePlanes po = out;
 		size_t soff[3] = {0, 0, 0};
@@ -653,7 +733,7 @@ int run_call(const FramePlanes& in, const FramePlanes& out, int nframes, const G
 				pi.plane[k] = in.plane[k] + (size_t)f0 * in.frame_stride;
 				po.plane[k] = c.d_scratch + soff[k];
 			}
-			if (int rc = run_frames_device(pi, po, n, g, false, epoch, (uint64_t)f0, c.d_streams, st)) return rc;
+			if (int rc = run_frames_device(s, pi, po, n, g, false, epoch, (uint64_t)f0, c.d_streams, st)) return rc;
 			for (int f = 0; f < n; f++) // rows of the caller's planes may be padded: 2-D copies, plane by plane
 				for (int k = 0; k < nplanes; k++) {
 					const size_t row = (size_t)po.stride[k];
@@ -662,16 +742,393 @@ int run_call(const FramePlanes& in, const FramePlanes& out, int nframes, const G
 					                           cudaMemcpyDeviceToDevice, st));
 				}
 		}
-		advance_registers(g, (uint64_t)nframes);
+		advance_registers(*s.h, g, (uint64_t)nframes);
 		return VFGS_B200_OK;
 	}
 	const int t = (int)(c.tab_next++ & 1u);
 	if (int rc = grow(c.d_tab[t], c.tab_cap[t], (size_t)nframes * g.R * g.spitch * kBlockTableBytes + 16)) return rc;
 	if (c.tab_used[t]) CUDA_TRY(cudaStreamWaitEvent(c.s_tab, c.tab_free[t], 0)); // the grain kernels of two calls ago read this buffer
-	if (int rc = run_frames_device(in, out, nframes, g, in_place, hw().line_rnd, 0, c.d_tab[t], st, c.s_tab, c.tab_ready[t])) return rc;
+	if (int rc = run_frames_device(s, in, out, nframes, g, in_place, s.h->line_rnd, 0, c.d_tab[t], st, c.s_tab, c.tab_ready[t])) return rc;
 	CUDA_TRY(cudaEventRecord(c.tab_free[t], st));
 	c.tab_used[t] = true;
-	advance_registers(g, (uint64_t)nframes);
+	advance_registers(*s.h, g, (uint64_t)nframes);
+	return VFGS_B200_OK;
+}
+
+// Body of the device frame entry points, after their own argument checks: overlap check (before any device work),
+// then the grain launches on the global state.
+int run_call(const FramePlanes& in, const FramePlanes& out, int nframes, const Geometry& g, cudaStream_t st)
+{
+	const int alias = nframes ? aliasing(in, out, nframes, g) : 0; // argument check first: needs no device
+	if (alias < 0)
+		return set_err(VFGS_B200_ERR_ARG, g.in_depth != g.out_depth ? "in-place needs equal depths"
+		               : "input and output planes overlap without being identical (same planes, strides and depth)");
+	if (int rc = prepare(-1)) return rc;
+	if (nframes == 0) return VFGS_B200_OK;
+	if (int rc = stream_switch(st)) return rc;
+	return run_job(global_state(), in, out, nframes, g, alias, st);
+}
+
+} // namespace
+
+// A session: a snapshot of one complete hardware state with its own table images in device memory (built once, never
+// rewritten, so no ring and no reuse wait). last_batch: the event after the last batched launch that read it; the
+// image set's last_use covers the single-job route.
+struct vfgs_b200_session {
+	HwState hw;
+	TableInfo bi;
+	ImageSet img;
+	bool uploaded = false; // the upload is known to be complete: launches need not wait for it
+	std::shared_ptr<CUevent_st> last_batch;
+};
+
+namespace {
+
+StateRef session_state(vfgs_b200_session* s) { return {&s->hw, &s->bi, &s->img}; }
+
+// One job of a batched call after its argument checks.
+struct JobPlan {
+	vfgs_b200_session* s;
+	FramePlanes in, out;
+	Geometry g;
+	int n, alias;
+	bool batched;       // served by the MULTI launches (else by the single-job route)
+	LaunchPlan lp;
+	uint32_t epoch;     // the session's line_rnd at enqueue
+	size_t tab_off;     // bytes into d_tab of its window-offset table
+};
+
+typedef void (*MultiKernel)(const MultiParams);
+
+template <bool FOLD, bool SHIFT>
+MultiKernel gather_multi_kernel(bool in16, bool out8, bool msb)
+{
+	if (msb) return out8 ? fgs_apply_gather_multi_kernel<true, true, FOLD, SHIFT, true> : fgs_apply_gather_multi_kernel<true, false, FOLD, SHIFT, true>;
+	return !in16 ? fgs_apply_gather_multi_kernel<false, false, FOLD, SHIFT>
+	     : out8 ? fgs_apply_gather_multi_kernel<true, true, FOLD, SHIFT> : fgs_apply_gather_multi_kernel<true, false, FOLD, SHIFT>;
+}
+
+// The MULTI instantiation of a group key (group_key; kinds numbered as LaunchPlan::kind: 0 fast, 1 gather, 3 EDGE) and
+// its CTA size: the same choice launch_apply makes for one job.
+MultiKernel multi_kernel(int key, int& threads)
+{
+	const int kind = key & 3;
+	const bool in16 = key & 4, out8 = key & 8, allwide = key & 16, semi = key & 32;
+	if (kind == 1) {
+		threads = kGatherThreads;
+		const bool fold = key & 64, shift = key & 128, msb = key & 256;
+		return fold ? (shift ? gather_multi_kernel<true, true>(in16, out8, msb) : gather_multi_kernel<true, false>(in16, out8, msb))
+		            : (shift ? gather_multi_kernel<false, true>(in16, out8, msb) : gather_multi_kernel<false, false>(in16, out8, msb));
+	}
+	threads = fast_threads(in16, in16 && out8, kind == 3, allwide);
+	if (kind == 3)
+		return !in16 ? fgs_apply_fast_multi_kernel<false, false, true> : out8 ? fgs_apply_fast_multi_kernel<true, true, true> : fgs_apply_fast_multi_kernel<true, false, true>;
+	if (semi)
+		return allwide ? fgs_apply_fast_multi_kernel<true, false, false, true, true>
+		     : !in16 ? fgs_apply_fast_multi_kernel<false, false, false, false, true>
+		     : out8 ? fgs_apply_fast_multi_kernel<true, true, false, false, true> : fgs_apply_fast_multi_kernel<true, false, false, false, true>;
+	if (allwide) return fgs_apply_fast_multi_kernel<true, false, false, true>;
+	return !in16 ? fgs_apply_fast_multi_kernel<false, false> : out8 ? fgs_apply_fast_multi_kernel<true, true> : fgs_apply_fast_multi_kernel<true, false>;
+}
+
+// Argument checks of one job against its session's state (what the single-job entry points refuse), and its geometry.
+int check_job(const vfgs_b200_job& j, int k, JobPlan& jp)
+{
+	if (!j.session) return set_err(VFGS_B200_ERR_ARG, "job %d: null session", k);
+	const bool planar = j.in || j.out, semi = j.sp_in || j.sp_out;
+	if (planar == semi) return set_err(VFGS_B200_ERR_ARG, "job %d: set exactly one of the planar and the semi-planar pairs", k);
+	if (planar ? !(j.in && j.out) : !(j.sp_in && j.sp_out)) return set_err(VFGS_B200_ERR_ARG, "job %d: null planes", k);
+	if (j.nframes < 0) return set_err(VFGS_B200_ERR_ARG, "job %d: negative frame count", k);
+	jp.s = j.session;
+	jp.n = j.nframes;
+	if (planar) {
+		if (int rc = make_geometry(jp.g, j.session->hw, j.width, j.height, j.out_depth)) return rc;
+		jp.in = frame_planes(*j.in); jp.out = frame_planes(*j.out);
+	} else {
+		if (j.out_depth) return set_err(VFGS_B200_ERR_ARG, "job %d: out_depth is 0 for semi-planar jobs (the output format selects it)", k);
+		if (int rc = semiplanar_geometry(jp.g, j.session->hw, *j.sp_in, *j.sp_out, j.width, j.height)) return rc;
+		jp.in = frame_planes(*j.sp_in); jp.out = frame_planes(*j.sp_out);
+	}
+	jp.alias = jp.n ? aliasing(jp.in, jp.out, jp.n, jp.g) : 0;
+	if (jp.alias < 0)
+		return set_err(VFGS_B200_ERR_ARG, jp.g.in_depth != jp.g.out_depth ? "job %d: in-place needs equal depths"
+		               : "job %d: input and output planes overlap without being identical (same planes, strides and depth)", k);
+	return VFGS_B200_OK;
+}
+
+// Refuses a call in which the buffers of two jobs overlap (in place within one job stays allowed): jobs sorted by the
+// start of their bounding byte range, each tested against the following ones whose range starts before its own ends.
+int check_disjoint(const std::vector<JobPlan>& jp)
+{
+	struct Span { const uint8_t *lo, *hi; int k; };
+	std::vector<Span> sp;
+	for (int k = 0; k < (int)jp.size(); k++) {
+		const JobPlan& j = jp[k];
+		if (!j.n) continue;
+		const uint8_t *ilo, *ihi, *olo, *ohi;
+		side_span({j.in, j.n, j.g, j.g.in_sample}, ilo, ihi);
+		side_span({j.out, j.n, j.g, j.g.out_sample}, olo, ohi);
+		if (!ilo && !olo) continue;
+		sp.push_back({!ilo ? olo : !olo ? ilo : std::min(ilo, olo), std::max(ihi, ohi), k});
+	}
+	std::sort(sp.begin(), sp.end(), [](const Span& a, const Span& b) { return a.lo < b.lo; });
+	for (size_t x = 0; x < sp.size(); x++)
+		for (size_t y = x + 1; y < sp.size() && sp[y].lo < sp[x].hi; y++) {
+			const JobPlan &a = jp[sp[x].k], &b = jp[sp[y].k];
+			const Side as[2] = {{a.in, a.n, a.g, a.g.in_sample}, {a.out, a.n, a.g, a.g.out_sample}};
+			const Side bs[2] = {{b.in, b.n, b.g, b.g.in_sample}, {b.out, b.n, b.g, b.g.out_sample}};
+			for (int u = 0; u < 2; u++)
+				for (int v = 0; v < 2; v++)
+					if (overlap(as[u], bs[v]))
+						return set_err(VFGS_B200_ERR_ARG, "the buffers of jobs %d and %d overlap", std::min(sp[x].k, sp[y].k), std::max(sp[x].k, sp[y].k));
+		}
+	return VFGS_B200_OK;
+}
+
+template <typename T>
+int grow_host(T*& p, size_t& cap, size_t need)
+{
+	if (need <= cap) return VFGS_B200_OK;
+	if (p) CUDA_TRY(cudaFreeHost(p));
+	p = nullptr; cap = 0;
+	need = (need + 4095) & ~(size_t)4095;
+	CUDA_TRY(cudaHostAlloc((void**)&p, need, cudaHostAllocDefault));
+	cap = need;
+	return VFGS_B200_OK;
+}
+
+size_t align16(size_t x) { return (x + 15) & ~(size_t)15; }
+
+// The jobs of a call that the MULTI launches serve: one stream-kernel launch for all their block tables, then one grain
+// launch per kernel instantiation (group_key).
+int run_batched(std::vector<JobPlan>& jp, cudaStream_t st, int& bits)
+{
+	Context& c = g_ctx;
+	size_t tab_bytes = 0;
+	int njobs = 0;
+	long long nwarps = 0;
+	for (JobPlan& j : jp) {
+		if (!j.batched) continue;
+		j.tab_off = tab_bytes;
+		tab_bytes += (align16((size_t)j.n * j.g.R * j.g.spitch * 4) + (size_t)j.n * j.g.R * j.g.spitch * 8 + 255) & ~(size_t)255;
+		njobs++;
+		nwarps += (long long)j.n * j.g.R;
+	}
+	if (!njobs) return VFGS_B200_OK;
+	const int t = (int)(c.tab_next++ & 1u);
+	if (int rc = grow(c.d_tab[t], c.tab_cap[t], tab_bytes)) return rc;
+	uint8_t* tab = (uint8_t*)c.d_tab[t];
+	std::vector<const LaunchPlan*> plans;
+	for (JobPlan& j : jp) {
+		if (!j.batched) continue;
+		uint16_t* woffs = (uint16_t*)(tab + j.tab_off + align16((size_t)j.n * j.g.R * j.g.spitch * 4));
+		for (FgsParams* q : {&j.lp.fast, &j.lp.edge, &j.lp.gather}) { q->states = nullptr; q->woffs = woffs; }
+		plans.push_back(&j.lp);
+		if (j.lp.any_fast && j.in.semi && j.lp.fast.fwide[1]) bits |= 16; // the interleaved U/V lane runs
+	}
+	std::vector<LaunchGroup> groups;
+	group_launches(plans, groups);
+	// descriptors: StreamJob[njobs], then per group FgsParams[m] and long long task0[m + 1]
+	size_t bytes = align16(sizeof(StreamJob) * njobs);
+	std::vector<size_t> goff(groups.size());
+	for (size_t k = 0; k < groups.size(); k++) {
+		goff[k] = bytes;
+		bytes += align16(sizeof(FgsParams) * groups[k].p.size()) + align16(sizeof(long long) * (groups[k].p.size() + 1));
+	}
+	if (c.desc_used[t]) CUDA_TRY(cudaEventSynchronize(c.desc_copied[t])); // the staging buffer's previous copy has left it
+	if (c.tab_used[t]) CUDA_TRY(cudaStreamWaitEvent(c.s_tab, c.tab_free[t], 0)); // the grain kernels of two calls ago read these buffers
+	if (bytes > c.desc_cap[t]) { // the device copy may still be read: wait for the table stream before it is freed
+		if (c.d_desc[t]) CUDA_TRY(cudaStreamSynchronize(c.s_tab));
+		if (int rc = grow(c.d_desc[t], c.desc_cap[t], bytes)) return rc;
+	}
+	if (int rc = grow_host(c.h_desc[t], c.hdesc_cap[t], bytes)) return rc; // its last copy is done (desc_copied)
+	uint8_t* h = c.h_desc[t];
+	uint8_t* d = c.d_desc[t];
+	StreamJob* sj = (StreamJob*)h;
+	long long w0 = 0;
+	int k = 0;
+	for (const JobPlan& j : jp) {
+		if (!j.batched) continue;
+		StreamJob& s = sj[k++];
+		s.warp0 = w0; s.epoch = j.epoch; s.R = j.g.R; s.nb = j.g.nb; s.spitch = j.g.spitch;
+		s.states = nullptr; s.woffs = (uint16_t*)j.lp.fast.woffs;
+		s.wp = make_woff_params(j.lp.fast, j.lp.kind);
+		w0 += (long long)j.n * j.g.R;
+	}
+	for (size_t g = 0; g < groups.size(); g++) {
+		FgsParams* fp = (FgsParams*)(h + goff[g]);
+		long long* t0 = (long long*)(h + goff[g] + align16(sizeof(FgsParams) * groups[g].p.size()));
+		t0[0] = 0;
+		for (size_t m = 0; m < groups[g].p.size(); m++) {
+			fp[m] = *groups[g].p[m];
+			t0[m + 1] = t0[m] + fp[m].total_tasks;
+		}
+	}
+	CUDA_TRY(cudaMemcpyAsync(d, h, bytes, cudaMemcpyHostToDevice, c.s_tab));
+	CUDA_TRY(cudaEventRecord(c.desc_copied[t], c.s_tab));
+	c.desc_used[t] = true;
+	{ // block tables of every job: one launch on the table stream
+		const int grid = (int)((nwarps * 32 + kLfsrThreads - 1) / kLfsrThreads);
+		lfsr_states_jobs_kernel<<<grid, kLfsrThreads, 0, c.s_tab>>>(c.d_pow2, (const StreamJob*)d, njobs, nwarps);
+		CUDA_TRY(cudaGetLastError());
+		g_launches++;
+	}
+	CUDA_TRY(cudaEventRecord(c.tab_ready[t], c.s_tab));
+	CUDA_TRY(cudaStreamWaitEvent(st, c.tab_ready[t], 0));
+	for (const JobPlan& j : jp) // images of sessions whose upload is not known to be complete
+		if (j.batched && !j.s->uploaded) {
+			if (cudaEventQuery(j.s->img.uploaded) == cudaSuccess) j.s->uploaded = true;
+			else CUDA_TRY(cudaStreamWaitEvent(st, j.s->img.uploaded, 0));
+		}
+	for (size_t g = 0; g < groups.size(); g++) {
+		const LaunchGroup& part = groups[g];
+		MultiParams mp;
+		memset(&mp, 0, sizeof(mp));
+		mp.jobs = (const FgsParams*)(d + goff[g]);
+		mp.task0 = (const long long*)(d + goff[g] + align16(sizeof(FgsParams) * part.p.size()));
+		mp.njobs = (int)part.p.size();
+		long long total = 0;
+		for (const FgsParams* q : part.p) total += q->total_tasks;
+		const int kind = part.key & 3, smem = part.smem;
+		if (total <= 0) continue;
+		int threads = 0;
+		MultiKernel kern = multi_kernel(part.key, threads);
+		if (smem > c.multi_smem_attr[part.key]) {
+			CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+			c.multi_smem_attr[part.key] = smem;
+		}
+		int& per_sm = c.multi_per_sm[part.key]; // resident CTAs per SM, asked once per key and shared-memory size
+		if (c.multi_occ_smem[part.key] != smem) {
+			CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, threads, (size_t)smem));
+			c.multi_occ_smem[part.key] = smem;
+		}
+		if (per_sm < 1) return set_err(VFGS_B200_ERR_CUDA, "grain kernel does not fit on an SM (smem %d)", smem);
+		const int wpc = threads / 32;
+		const long long want = (total + wpc - 1) / wpc, cap = (long long)c.sm_count * per_sm;
+		const int grid = (int)(want < cap ? want : cap);
+		cudaEvent_t e0 = nullptr, e1 = nullptr;
+		if (c.timing) {
+			if (c.ev_used == c.ev_begin.size()) {
+				cudaEvent_t a, b;
+				CUDA_TRY(cudaEventCreate(&a));
+				CUDA_TRY(cudaEventCreate(&b));
+				c.ev_begin.push_back(a); c.ev_end.push_back(b);
+			}
+			e0 = c.ev_begin[c.ev_used]; e1 = c.ev_end[c.ev_used]; c.ev_used++;
+			CUDA_TRY(cudaEventRecord(e0, st));
+		}
+		kern<<<grid, threads, (size_t)smem, st>>>(mp);
+		CUDA_TRY(cudaGetLastError());
+		if (c.timing) CUDA_TRY(cudaEventRecord(e1, st));
+		g_launches++;
+		c.last_launch[0] = grid; c.last_launch[1] = threads; c.last_launch[2] = smem; c.last_launch[3] = c.sm_count;
+		bits |= kind == 0 ? 1 : kind == 1 ? 4 : 8;
+	}
+	CUDA_TRY(cudaEventRecord(c.tab_free[t], st));
+	c.tab_used[t] = true;
+	// the call's end, which its sessions keep: an event of the pool that no session holds any more, else a new one
+	std::shared_ptr<CUevent_st> done;
+	for (const std::shared_ptr<CUevent_st>& e : c.call_events)
+		if (e.use_count() == 1) { done = e; break; }
+	if (!done) {
+		cudaEvent_t ev;
+		CUDA_TRY(cudaEventCreateWithFlags(&ev, cudaEventDisableTiming));
+		done.reset(ev, [](cudaEvent_t e) { cudaEventDestroy(e); });
+		c.call_events.push_back(done);
+	}
+	CUDA_TRY(cudaEventRecord(done.get(), st));
+	for (JobPlan& j : jp)
+		if (j.batched) j.s->last_batch = done;
+	return VFGS_B200_OK;
+}
+
+int run_jobs(const vfgs_b200_job* jobs, int njobs, cudaStream_t st)
+{
+	if (njobs < 0) return set_err(VFGS_B200_ERR_ARG, "negative job count");
+	if (njobs && !jobs) return set_err(VFGS_B200_ERR_ARG, "null job list");
+	std::vector<JobPlan> jp((size_t)njobs);
+	for (int k = 0; k < njobs; k++) // argument checks first: they need no device
+		if (int rc = check_job(jobs[k], k, jp[k])) return rc;
+	if (int rc = check_disjoint(jp)) return rc;
+	for (JobPlan& j : jp) { // plans; a launch the kernels cannot take is refused before any device work
+		if (!j.n) continue;
+		uint16_t* w = nullptr;
+		FgsParams p;
+		plan_frames(session_state(j.s), j.in, j.out, j.n, j.g, j.alias == 1, nullptr, p, j.lp, w);
+		// the general kernel and the in-place scratch detour take the single-job route
+		const bool scratch = j.alias == 1 && in_place_needs_scratch(j.lp, j.s->bi);
+		j.batched = !j.lp.any_general && !scratch;
+		if (!scratch) // (the scratch detour cuts a job into sub-batches of 256 MB, far below the limit)
+			for (const FgsParams* q : {&j.lp.fast, &j.lp.edge, &j.lp.gather, &j.lp.general})
+				if (q->total_tasks >= (1ll << 31))
+					return set_err(VFGS_B200_ERR_ARG, "batch too large for one launch (%lld warp-tasks): split the job", q->total_tasks);
+	}
+	if (!njobs) return VFGS_B200_OK;
+	if (int rc = ensure_ctx(-1)) return rc;
+	if (int rc = stream_switch(st)) return rc;
+	int bits = 0;
+	for (JobPlan& j : jp) { // registers advance in list order; single-job-route jobs launch here
+		if (!j.n) continue;
+		if (j.batched) {
+			j.epoch = j.s->hw.line_rnd;
+			advance_registers(j.s->hw, j.g, (uint64_t)j.n);
+		} else {
+			if (int rc = run_job(session_state(j.s), j.in, j.out, j.n, j.g, j.alias, st)) return rc;
+			bits |= g_ctx.last_launch[4];
+		}
+	}
+	const int rc = run_batched(jp, st, bits);
+	g_ctx.last_launch[4] = bits;
+	return rc;
+}
+
+int create_session(vfgs_b200_session** out)
+{
+	if (!out) return set_err(VFGS_B200_ERR_ARG, "null session pointer");
+	*out = nullptr;
+	const HwState& h = hw();
+	// the geometry-independent conditions of make_geometry
+	if (h.scale_shift + h.bs < 8 || h.scale_shift + h.bs > 13)
+		return set_err(VFGS_B200_ERR_STATE, "scale_shift %d + bs %d outside 8..13 (vfgs_hw.c:170)", h.scale_shift, h.bs);
+	for (int c = 0; c < 3; c++)
+		for (int i = 0; i < 256; i++)
+			if ((h.plut[c][i] >> 4) >= kSlots)
+				return set_err(VFGS_B200_ERR_STATE, "pattern LUT %d entry %d selects slot %d: the hardware has slots 0..8 (vfgs_hw.c:49,218)", c, i, h.plut[c][i] >> 4);
+	if (int rc = ensure_ctx(-1)) return rc;
+	Context& c = g_ctx;
+	std::unique_ptr<vfgs_b200_session> s(new vfgs_b200_session());
+	s->hw = h;
+	std::vector<uint8_t> blob, fblob;
+	build_tables(s->hw, s->bi, blob, fblob);
+	if (s->bi.bytes > c.max_smem_optin - 1024)
+		return set_err(VFGS_B200_ERR_STATE, "table image of %d bytes exceeds shared memory", s->bi.bytes);
+	ImageSet& m = s->img;
+	auto fail = [&](int rc) {
+		if (m.d_blob) cudaFree(m.d_blob);
+		if (m.d_fblob) cudaFree(m.d_fblob);
+		if (m.h_stage) cudaFreeHost(m.h_stage);
+		if (m.uploaded) cudaEventDestroy(m.uploaded);
+		if (m.last_use) cudaEventDestroy(m.last_use);
+		return rc;
+	};
+	const size_t gb = (size_t)s->bi.gbytes, fb = (size_t)s->bi.fbytes;
+#define SESSION_TRY(expr) do { cudaError_t e_ = (expr); if (e_ != cudaSuccess) return fail(set_err(VFGS_B200_ERR_CUDA, "%s -> %s", #expr, cudaGetErrorString(e_))); } while (0)
+	SESSION_TRY(cudaMalloc((void**)&m.d_blob, gb));
+	SESSION_TRY(cudaMalloc((void**)&m.d_fblob, fb));
+	SESSION_TRY(cudaHostAlloc((void**)&m.h_stage, gb + fb, cudaHostAllocDefault));
+	SESSION_TRY(cudaEventCreateWithFlags(&m.uploaded, cudaEventDisableTiming));
+	SESSION_TRY(cudaEventCreateWithFlags(&m.last_use, cudaEventDisableTiming));
+	memcpy(m.h_stage, blob.data(), gb);
+	memcpy(m.h_stage + gb, fblob.data(), fb);
+	SESSION_TRY(cudaMemcpyAsync(m.d_blob, m.h_stage, gb, cudaMemcpyHostToDevice, c.s_tab));
+	SESSION_TRY(cudaMemcpyAsync(m.d_fblob, m.h_stage + gb, fb, cudaMemcpyHostToDevice, c.s_tab));
+	SESSION_TRY(cudaEventRecord(m.uploaded, c.s_tab));
+	if (s->bi.bytes > c.smem_attr) { // the general kernel of the single-job route
+		SESSION_TRY(cudaFuncSetAttribute(fgs_apply_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, s->bi.bytes));
+		c.smem_attr = s->bi.bytes;
+	}
+#undef SESSION_TRY
+	*out = s.release();
 	return VFGS_B200_OK;
 }
 
@@ -804,7 +1261,7 @@ void vfgs_add_grain_line(void* Y, void* U, void* V, int y, int width)
 		chk(cudaMemcpyAsync(c.d_line + lpad + cpad, V, cbytes, cudaMemcpyHostToDevice, st), "V H2D");
 	}
 	FgsParams p;
-	fill_common(p, g);
+	fill_common(p, g, global_state());
 	p.nframes = 1;
 	p.y_begin = y; p.y_end = y + 1;
 	p.row_begin = y >> 4; p.rows = 1;
@@ -817,7 +1274,7 @@ void vfgs_add_grain_line(void* Y, void* U, void* V, int y, int width)
 	}
 	p.states = c.d_streams; p.stream_rows = 2; p.stream_row0 = (y >> 4) - 1;
 	finish_tasks(p);
-	if (images_before(st) || launch_apply(p, st) || images_after(st)) fatal("vfgs_add_grain_line");
+	if (images_before(global_state(), st) || launch_apply(p, st) || images_after(global_state(), st)) fatal("vfgs_add_grain_line");
 	chk(cudaMemcpyAsync(Y, c.d_line + region, lbytes, cudaMemcpyDeviceToHost, st), "Y D2H");
 	if (chroma) {
 		chk(cudaMemcpyAsync(U, c.d_line + region + lpad, cbytes, cudaMemcpyDeviceToHost, st), "U D2H");
@@ -862,25 +1319,8 @@ int vfgs_b200_add_grain_semiplanar_device(const vfgs_b200_semiplanar* in, const 
                                           int width, int height, void* stream)
 {
 	if (!in || !out || nframes < 0) return set_err(VFGS_B200_ERR_ARG, "null planes or negative frame count");
-	if (!in->y || !in->uv || !out->y || !out->uv) return set_err(VFGS_B200_ERR_ARG, "null plane pointer");
-	const HwState& h = hw();
-	const int depth = 8 + h.bs;
-	if (in->format != (depth == 10 ? VFGS_B200_P010 : VFGS_B200_NV12))
-		return set_err(VFGS_B200_ERR_ARG, "input format %d does not match the configured depth %d (NV12 = 8, P010 = 10)", in->format, depth);
-	if (out->format != in->format && !(out->format == VFGS_B200_NV12 && in->format == VFGS_B200_P010))
-		return set_err(VFGS_B200_ERR_ARG, "output format %d from input format %d (same format, or NV12 from P010)", out->format, in->format);
-	if (h.csubx != 2)
-		return set_err(VFGS_B200_ERR_ARG, "semi-planar frames are 4:2:0 or 4:2:2 (4:4:4 frames are planar)");
 	Geometry g;
-	if (int rc = make_geometry(g, width, height, out->format == in->format ? 0 : 8)) return rc;
-	for (int side = 0; side < 2; side++) {
-		const vfgs_b200_semiplanar& f = side ? *out : *in;
-		const int64_t sample = (int64_t)(side ? g.out_sample : g.in_sample);
-		if (f.stride_y < (int64_t)g.width * sample || f.stride_uv < 2 * (int64_t)g.cw * sample)
-			return set_err(VFGS_B200_ERR_ARG, "%s line stride shorter than a row", side ? "output" : "input");
-		if (sample == 2 && (((uintptr_t)f.y | (uintptr_t)f.uv | (uint64_t)f.stride_y | (uint64_t)f.stride_uv | (uint64_t)f.frame_stride) & 1))
-			return set_err(VFGS_B200_ERR_ARG, "%s P010 planes and strides must be 2-byte aligned", side ? "output" : "input");
-	}
+	if (int rc = semiplanar_geometry(g, hw(), *in, *out, width, height)) return rc;
 	return run_call(frame_planes(*in), frame_planes(*out), nframes, g, (cudaStream_t)stream);
 }
 
@@ -936,7 +1376,7 @@ int vfgs_b200_add_grain_frames_host(const void* in, void* out, int nframes, int 
 		vfgs_b200_planes pi, po;
 		packed_planes(pi, s.d_in, g, g.in_sample, g.in_frame_bytes);
 		packed_planes(po, s.d_out, g, g.out_sample, g.out_frame_bytes);
-		if (int rc = run_frames_device(frame_planes(pi), frame_planes(po), n, g, false, epoch, (uint64_t)f0, s.d_streams, c.s_k)) return rc;
+		if (int rc = run_frames_device(global_state(), frame_planes(pi), frame_planes(po), n, g, false, epoch, (uint64_t)f0, s.d_streams, c.s_k)) return rc;
 		CUDA_TRY(cudaEventRecord(s.k_done, c.s_k));
 		CUDA_TRY(cudaStreamWaitEvent(c.s_d2h, s.k_done, 0));
 		CUDA_TRY(cudaMemcpyAsync(hout + (size_t)f0 * g.out_frame_bytes, s.d_out, (size_t)n * g.out_frame_bytes, cudaMemcpyDeviceToHost, c.s_d2h));
@@ -945,7 +1385,7 @@ int vfgs_b200_add_grain_frames_host(const void* in, void* out, int nframes, int 
 	CUDA_TRY(cudaStreamSynchronize(c.s_d2h));
 	CUDA_TRY(cudaStreamSynchronize(c.s_k));
 	CUDA_TRY(cudaStreamSynchronize(c.s_h2d));
-	advance_registers(g, (uint64_t)nframes);
+	advance_registers(hw(), g, (uint64_t)nframes);
 	return VFGS_B200_OK;
 }
 
@@ -954,7 +1394,7 @@ int vfgs_b200_skip_frames(int64_t nframes, int width, int height)
 	if (nframes < 0) return set_err(VFGS_B200_ERR_ARG, "negative frame count");
 	Geometry g;
 	if (int rc = make_geometry(g, width, height, 0)) return rc;
-	advance_registers(g, (uint64_t)nframes);
+	advance_registers(hw(), g, (uint64_t)nframes);
 	return VFGS_B200_OK;
 }
 
@@ -973,21 +1413,7 @@ void vfgs_b200_set_lfsr(const uint32_t regs[4])
 // Mirror of the hardware state in the layout of the reference's statics (see oracle/ref_harness.c
 // refh_state): pattern[2][9][64][64], sLUT[3][256], pLUT[3][256], 4 LFSR registers, then
 // scale_shift, bs, Y_min, Y_max, C_min, C_max, csubx, csuby as ints.
-size_t vfgs_b200_get_state(void* dst, size_t cap)
-{
-	const HwState& h = hw();
-	const size_t need = sizeof(h.pattern) + sizeof(h.slut) + sizeof(h.plut) + 4 * sizeof(uint32_t) + 8 * sizeof(int);
-	if (!dst || cap < need) return need;
-	uint8_t* p = (uint8_t*)dst;
-	memcpy(p, h.pattern, sizeof(h.pattern)); p += sizeof(h.pattern);
-	memcpy(p, h.slut, sizeof(h.slut)); p += sizeof(h.slut);
-	memcpy(p, h.plut, sizeof(h.plut)); p += sizeof(h.plut);
-	const uint32_t regs[4] = {h.rnd, h.rnd_up, h.line_rnd, h.line_rnd_up};
-	memcpy(p, regs, sizeof(regs)); p += sizeof(regs);
-	const int sc[8] = {h.scale_shift, h.bs, h.y_min, h.y_max, h.c_min, h.c_max, h.csubx, h.csuby};
-	memcpy(p, sc, sizeof(sc));
-	return need;
-}
+size_t vfgs_b200_get_state(void* dst, size_t cap) { return state_dump(hw(), dst, cap); }
 
 void* vfgs_b200_host_alloc(size_t bytes)
 {
@@ -1038,6 +1464,47 @@ void vfgs_b200_last_launch(int out[5])
 {
 	for (int i = 0; i < 5; i++) out[i] = g_ctx.last_launch[i];
 }
+
+int vfgs_b200_session_create(vfgs_b200_session** out) { return create_session(out); }
+
+void vfgs_b200_session_destroy(vfgs_b200_session* s)
+{
+	if (!s) return;
+	if (s->img.in_use) cudaEventSynchronize(s->img.last_use);
+	if (s->last_batch) cudaEventSynchronize(s->last_batch.get());
+	cudaFree(s->img.d_blob);
+	cudaFree(s->img.d_fblob);
+	cudaFreeHost(s->img.h_stage);
+	cudaEventDestroy(s->img.uploaded);
+	cudaEventDestroy(s->img.last_use);
+	delete s;
+}
+
+void vfgs_b200_session_get_lfsr(const vfgs_b200_session* s, uint32_t regs[4])
+{
+	const HwState& h = s->hw;
+	regs[0] = h.rnd; regs[1] = h.rnd_up; regs[2] = h.line_rnd; regs[3] = h.line_rnd_up;
+}
+
+void vfgs_b200_session_set_lfsr(vfgs_b200_session* s, const uint32_t regs[4])
+{
+	HwState& h = s->hw;
+	h.rnd = regs[0]; h.rnd_up = regs[1]; h.line_rnd = regs[2]; h.line_rnd_up = regs[3];
+}
+
+int vfgs_b200_session_skip_frames(vfgs_b200_session* s, int64_t nframes, int width, int height)
+{
+	if (!s) return set_err(VFGS_B200_ERR_ARG, "null session");
+	if (nframes < 0) return set_err(VFGS_B200_ERR_ARG, "negative frame count");
+	Geometry g;
+	if (int rc = make_geometry(g, s->hw, width, height, 0)) return rc;
+	advance_registers(s->hw, g, (uint64_t)nframes);
+	return VFGS_B200_OK;
+}
+
+size_t vfgs_b200_session_get_state(const vfgs_b200_session* s, void* dst, size_t cap) { return state_dump(s->hw, dst, cap); }
+
+int vfgs_b200_add_grain_jobs_device(const vfgs_b200_job* jobs, int njobs, void* stream) { return run_jobs(jobs, njobs, (cudaStream_t)stream); }
 
 } // extern "C"
 

@@ -62,14 +62,10 @@ __device__ __forceinline__ void bulk_copy_g2s(void* dst_smem, const void* src_gm
 // uint32[64][32]; lane i owns output bit i, a ballot assembles the word), then walk the row 32 steps
 // at a time: consecutive blocks are consecutive 32-bit windows of one bit-stream, so lane l takes
 // window l of every {word k, word k+1} pair and the 32 registers go out as one coalesced store.
-__global__ void __launch_bounds__(kLfsrThreads)
-lfsr_states_kernel(uint32_t epoch_state, const uint32_t* __restrict__ pow2, uint32_t* __restrict__ states,
-                   uint16_t* __restrict__ woffs, const WoffParams wp,
-                   int nframes, int R, int nb, int spitch, unsigned long long frame0)
+__device__ __forceinline__ void lfsr_row_tables(uint32_t epoch_state, const uint32_t* __restrict__ pow2, uint32_t* __restrict__ states,
+                                                uint16_t* __restrict__ woffs, const WoffParams& wp, int warp, int R, int nb,
+                                                int spitch, unsigned long long frame0, int lane)
 {
-	const int warp = (int)((blockIdx.x * (unsigned)blockDim.x + threadIdx.x) >> 5);
-	const int lane = threadIdx.x & 31;
-	if (warp >= nframes * R) return; // warp-uniform
 	const int f = warp / R, r = warp - f * R;
 	unsigned long long t = ((frame0 + (unsigned long long)f) * (unsigned long long)(R - 1) + (unsigned long long)r) *
 	                       (unsigned long long)nb;
@@ -101,6 +97,30 @@ lfsr_states_kernel(uint32_t epoch_state, const uint32_t* __restrict__ pow2, uint
 		}
 		s = next;
 	}
+}
+
+__global__ void __launch_bounds__(kLfsrThreads)
+lfsr_states_kernel(uint32_t epoch_state, const uint32_t* __restrict__ pow2, uint32_t* __restrict__ states,
+                   uint16_t* __restrict__ woffs, const WoffParams wp,
+                   int nframes, int R, int nb, int spitch, unsigned long long frame0)
+{
+	const int warp = (int)((blockIdx.x * (unsigned)blockDim.x + threadIdx.x) >> 5);
+	const int lane = threadIdx.x & 31;
+	if (warp >= nframes * R) return; // warp-uniform
+	lfsr_row_tables(epoch_state, pow2, states, woffs, wp, warp, R, nb, spitch, frame0, lane);
+}
+
+// Job-table form (vfgs_b200_add_grain_jobs_device): the block tables of every job of a call in one launch. One warp per
+// (job, frame, block-row); the job is found by binary search over the prefix of nframes * R (StreamJob::warp0). Frame 0
+// of a job is its session's register position at enqueue (StreamJob::epoch).
+__global__ void __launch_bounds__(kLfsrThreads)
+lfsr_states_jobs_kernel(const uint32_t* __restrict__ pow2, const StreamJob* __restrict__ jobs, int njobs, long long nwarps)
+{
+	const long long warp = (long long)((blockIdx.x * (unsigned long long)blockDim.x + threadIdx.x) >> 5);
+	const int lane = threadIdx.x & 31;
+	if (warp >= nwarps) return; // warp-uniform
+	const StreamJob& J = jobs[stream_job_of(jobs, njobs, warp)];
+	lfsr_row_tables(J.epoch, pow2, J.states, J.woffs, J.wp, (int)(warp - J.warp0), J.R, J.nb, J.spitch, 0ull, lane);
 }
 
 // ---- grain synthesis -----------------------------------------------------------------------
@@ -204,6 +224,61 @@ fgs_apply_fast_kernel(const __grid_constant__ FgsParams p)
 		process_task_fast<IN16, OUT8, EDGE, ALLWIDE, SEMI>(p, lut, (uint32_t)task, lane);
 }
 
+// Before a CTA overwrites tables the previous job's tasks read: every warp is done with them, and the generic-proxy
+// reads are ordered before the bulk copy's async-proxy writes.
+__device__ __forceinline__ void multi_switch_barrier()
+{
+	__syncthreads();
+	if (threadIdx.x == 0) asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+}
+
+// MULTI form (vfgs_b200_add_grain_jobs_device): the warp-tasks of several jobs of one instantiation, concatenated in job
+// order, in one launch. CTA b takes the contiguous range multi_cta_range(b); inside each job's part of it its warps take
+// tasks base + k * warps + w. Where the range enters the next job, the CTA waits for its warps, brings in that job's
+// images (next mbarrier phase) and re-expands the LUTs with that job's scale shift. The job's FgsParams are read from
+// global memory (uniform, L1-resident): no static shared memory is added, so the probe measures the same pad.
+template <bool IN16, bool OUT8, bool EDGE = false, bool ALLWIDE = false, bool SEMI = false>
+__global__ void __launch_bounds__(FastCta<IN16, OUT8, EDGE, ALLWIDE>::threads, 1)
+fgs_apply_fast_multi_kernel(const __grid_constant__ MultiParams m)
+{
+	constexpr int kFastThreads = FastCta<IN16, OUT8, EDGE, ALLWIDE>::threads, kFastWarps = kFastThreads / 32;
+	extern __shared__ __align__(128) uint8_t smem[];
+	__shared__ __align__(8) uint64_t bar;
+
+	const uint32_t pad = (0u - smem_u32(smem)) & (uint32_t)(kLutAlign - 1);
+	if (m.probe) {
+		if (threadIdx.x == 0) *m.probe = pad;
+		return;
+	}
+	uint8_t* lut_ptr = smem + pad;
+	if (threadIdx.x == 0) mbar_init(&bar, 1);
+	__syncthreads();
+
+	const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+	const smem_addr_t lut = smem_addr(lut_ptr);
+	MultiCursor cur;
+	multi_begin(m.task0, m.njobs, (int)gridDim.x, (int)blockIdx.x, cur);
+	uint32_t phase = 0;
+	int j;
+	long long lo, end;
+	while (multi_next(m.task0, cur, j, lo, end)) {
+		const long long t0 = m.task0[j];
+		const FgsParams& p = m.jobs[j];
+		if (phase) multi_switch_barrier();
+		if (threadIdx.x == 0) {
+			mbar_arrive_expect_tx(&bar, (uint32_t)(p.fimg_bytes[0] + p.fimg_bytes[1] + p.fimg_bytes[2]));
+			for (int c = 0; c < 3; c++)
+				if (p.fimg_bytes[c]) bulk_copy_g2s(lut_ptr + p.fimg_off[c], p.fblob + p.fimg_src[c], (uint32_t)p.fimg_bytes[c], &bar);
+		}
+		expand_fast_luts((uint32_t*)lut_ptr, (const uint32_t*)p.fblob, (uint32_t)p.pow16, threadIdx.x, kFastThreads);
+		mbar_wait(&bar, phase & 1);
+		phase++;
+		__syncthreads();
+		for (long long task = lo + warp; task < end; task += kFastWarps)
+			process_task_fast<IN16, OUT8, EDGE, ALLWIDE, SEMI>(p, lut, (uint32_t)(task - t0), lane);
+	}
+}
+
 // Gather path: components with sample-adaptive pattern selection (fgs_gather.h). Shared memory: one
 // per-lane replicated LUT (32 KB, entry layouts: gather_lut_entry) per gather component, each on a
 // 32 KB boundary, then the general table image (compact LUTs + pattern slots; FOLD: + the negated slots)
@@ -250,6 +325,51 @@ fgs_apply_gather_kernel(const __grid_constant__ FgsParams p)
 	const long long stride = (long long)gridDim.x * kGatherWarps;
 	for (long long task = (long long)blockIdx.x * kGatherWarps + (threadIdx.x >> 5); task < p.total_tasks; task += stride)
 		process_task_gather<IN16, OUT8, FOLD, SHIFT, MSB>(p, luts, img, (uint32_t)task, lane);
+}
+
+// MULTI form of the gather kernel: the schedule and the job switch of fgs_apply_fast_multi_kernel; a switch brings in the
+// next job's general image and rebuilds its per-lane LUTs.
+template <bool IN16, bool OUT8, bool FOLD, bool SHIFT, bool MSB = false>
+__global__ void __launch_bounds__(kGatherThreads, VFGS_GATHER_CTAS)
+fgs_apply_gather_multi_kernel(const __grid_constant__ MultiParams m)
+{
+	extern __shared__ __align__(128) uint8_t smem[];
+	__shared__ __align__(8) uint64_t bar;
+
+	uint8_t* lut_ptr = smem + ((0u - smem_u32(smem)) & (uint32_t)(kLutAlign - 1));
+	if (threadIdx.x == 0) mbar_init(&bar, 1);
+	__syncthreads();
+
+	const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+	const smem_addr_t luts = smem_addr(lut_ptr);
+	MultiCursor cur;
+	multi_begin(m.task0, m.njobs, (int)gridDim.x, (int)blockIdx.x, cur);
+	uint32_t phase = 0;
+	int j;
+	long long lo, end;
+	while (multi_next(m.task0, cur, j, lo, end)) {
+		const long long t0 = m.task0[j];
+		const FgsParams& p = m.jobs[j];
+		uint8_t* img_ptr = lut_ptr + p.ngather * kLutBytes;
+		if (phase) multi_switch_barrier();
+		if (threadIdx.x == 0) {
+			mbar_arrive_expect_tx(&bar, (uint32_t)p.blob_bytes);
+			bulk_copy_g2s(img_ptr, p.blob, (uint32_t)p.blob_bytes, &bar);
+		}
+		mbar_wait(&bar, phase & 1);
+		phase++;
+		for (int c = 0; c < 3; c++) {
+			if (p.glut_index[c] < 0) continue;
+			const uint16_t* compact = (const uint16_t*)(img_ptr + p.lut_off) + c * 256;
+			uint32_t* lut = (uint32_t*)(lut_ptr + p.glut_index[c] * kLutBytes);
+			const uint32_t slot_bytes = (uint32_t)p.pat_size[c ? 1 : 0];
+			for (int i = threadIdx.x; i < 256 * 32; i += kGatherThreads) lut[i] = gather_lut_entry<IN16>(compact[i >> 5], slot_bytes);
+		}
+		__syncthreads();
+		const smem_addr_t img = smem_addr(img_ptr);
+		for (long long task = lo + warp; task < end; task += kGatherWarps)
+			process_task_gather<IN16, OUT8, FOLD, SHIFT, MSB>(p, luts, img, (uint32_t)(task - t0), lane);
+	}
 }
 
 // ---- firmware layer: one pattern job (fw_device.h) -----------------------------------------------

@@ -450,4 +450,130 @@ inline WoffParams make_woff_params(const FgsParams& p, const int kind[3])
 	return w;
 }
 
+// ---- batched calls (vfgs_b200_add_grain_jobs_device) ------------------------------------------------
+// One job of the job-table form of the LFSR stream kernel: its warps are [warp0, warp0 + nframes * R) of the launch.
+struct StreamJob {
+	long long warp0;
+	uint32_t epoch; // the session's line_rnd at enqueue: frame 0 of the job
+	int R, nb, spitch;
+	uint32_t* states; // register table (null: not needed), window-offset table
+	uint16_t* woffs;
+	WoffParams wp;
+};
+
+// Launch block of the MULTI grain kernels: the per-job launch parameters of one kernel instantiation and the prefix of
+// their task counts (task0[j] = first task of job j in the concatenation, task0[njobs] = total), in device memory.
+struct MultiParams {
+	const FgsParams* jobs;
+	const long long* task0;
+	int njobs;
+	uint32_t* probe; // not null: the fast kernel only reports its shared-memory pad here (as FgsParams::probe)
+};
+
+// Static schedule of a MULTI launch: CTA b of `grid` takes the concatenated tasks [lo, hi), contiguous and in job order.
+VFGS_HD void multi_cta_range(long long total, int grid, int b, long long& lo, long long& hi)
+{
+	lo = total * b / grid;
+	hi = total * (b + 1) / grid;
+}
+// The job holding concatenated task t: the first j with task0[j + 1] > t (jobs without tasks are passed over).
+VFGS_HD int multi_first_job(const long long* task0, int njobs, long long t)
+{
+	int lo = 0, hi = njobs - 1;
+	while (lo < hi) {
+		const int mid = (lo + hi) >> 1;
+		if (task0[mid + 1] > t) hi = mid; else lo = mid + 1;
+	}
+	return lo;
+}
+// A CTA's walk over its range, one job at a time (the loop of the MULTI kernels and of the host replay in tests/emu):
+// multi_next gives the next job j the range enters and the part [lo, end) of the range inside it; the CTA loads job j's
+// tables, then its warps take tasks lo + k * warps + w below end (job-local index: task - task0[j]).
+struct MultiCursor {
+	long long lo, hi;
+	int j;
+};
+VFGS_HD void multi_begin(const long long* task0, int njobs, int grid, int b, MultiCursor& c)
+{
+	multi_cta_range(task0[njobs], grid, b, c.lo, c.hi);
+	c.j = multi_first_job(task0, njobs, c.lo);
+}
+VFGS_HD bool multi_next(const long long* task0, MultiCursor& c, int& j, long long& lo, long long& end)
+{
+	while (c.lo < c.hi) {
+		const int k = c.j++;
+		const long long e = task0[k + 1] < c.hi ? task0[k + 1] : c.hi;
+		if (e <= c.lo) continue; // a job without tasks
+		j = k; lo = c.lo; end = e;
+		c.lo = e;
+		return true;
+	}
+	return false;
+}
+// The job of warp `warp` of the job-table stream kernel: the last job whose first warp is <= warp (jobs without frames
+// share warp0 with the next one).
+VFGS_HD int stream_job_of(const StreamJob* jobs, int njobs, long long warp)
+{
+	int lo = 0, hi = njobs - 1;
+	while (lo < hi) {
+		const int mid = (lo + hi + 1) >> 1;
+		if (jobs[mid].warp0 <= warp) lo = mid; else hi = mid - 1;
+	}
+	return lo;
+}
+
+// Which kernel instantiation serves a planned launch: the launches of the jobs of one call are grouped by this key.
+// kind: 0 fast, 1 gather, 3 the fast kernel's EDGE variant (the general kernel is never batched).
+//   fast  IN16 | OUT8 | ALLWIDE | SEMI   (the template flags of fgs_apply_fast_kernel)
+//   gather IN16 | OUT8 | FOLD | SHIFT | MSB
+inline int group_key(const FgsParams& p, int kind, bool fold, bool shift)
+{
+	const bool in16 = p.in_bytes == 2, out8 = p.out_bytes == 1;
+	int k = kind | (in16 ? 4 : 0) | (out8 ? 8 : 0);
+	if (kind == 0) k |= (in16 && !out8 && p.fallwide ? 16 : 0) | (p.ilv[1] ? 32 : 0);
+	if (kind == 1) k |= (fold ? 64 : 0) | (shift ? 128 : 0) | (p.msb_in ? 256 : 0);
+	return k;
+}
+
+// Registers after nframes whole frames of R block-rows of nb blocks (vfgs_hw.c:291-298,309-310 in closed form).
+inline void advance_frames(HwState& h, int R, int nb, uint64_t nframes, const JumpTable& jt)
+{
+	if (!nframes) return;
+	const uint32_t s0 = h.line_rnd;
+	const uint64_t adv = nframes * (uint64_t)(R - 1) * (uint64_t)nb;
+	if (R >= 2) {
+		h.line_rnd_up = jt.jump(s0, adv - (uint64_t)nb);
+		h.line_rnd = jt.jump(s0, adv);
+	}
+	h.rnd = jt.jump(h.line_rnd, (uint64_t)nb);
+	h.rnd_up = jt.jump(h.line_rnd_up, (uint64_t)nb);
+}
+
+// The launches of a batched call: the planned launches of its jobs, grouped by group_key in order of first appearance,
+// each group's jobs in list order, with the largest dynamic shared memory of its jobs' launches.
+struct LaunchGroup {
+	int key;
+	std::vector<const FgsParams*> p;
+	int smem;
+};
+inline void group_launches(const std::vector<const LaunchPlan*>& plans, std::vector<LaunchGroup>& groups)
+{
+	groups.clear();
+	auto add = [&](const FgsParams& q, int kind, bool fold, bool shift, int smem) {
+		const int key = group_key(q, kind, fold, shift);
+		for (LaunchGroup& g : groups)
+			if (g.key == key) {
+				g.p.push_back(&q);
+				if (smem > g.smem) g.smem = smem;
+				return;
+			}
+		groups.push_back({key, {&q}, smem});
+	};
+	for (const LaunchPlan* lp : plans) {
+		if (lp->any_fast) add(lp->fast, 0, false, false, lp->fast.fsmem);
+		if (lp->any_edge) add(lp->edge, 3, false, false, lp->edge.fsmem);
+		if (lp->any_gather) add(lp->gather, 1, lp->gather_fold, lp->gather_shift, lp->gather_smem);
+	}
+}
+
 } // namespace vfgs
