@@ -173,6 +173,9 @@ void vfgs_b200_session_get_lfsr(const vfgs_b200_session* s, uint32_t regs[4]);
 void vfgs_b200_session_set_lfsr(vfgs_b200_session* s, const uint32_t regs[4]);
 /* vfgs_b200_skip_frames on the session's registers. */
 int  vfgs_b200_session_skip_frames(vfgs_b200_session* s, int64_t nframes, int width, int height);
+/* vfgs_set_seed on the session's registers: seed << 1 into all four (src/vfgs_hw.c:339-344). SEI metadata never seeds
+ * (the reference's CLI seeds separately, src/vfgs_main.c:759-760). */
+int  vfgs_b200_session_set_seed(vfgs_b200_session* s, uint32_t seed);
 /* The session's state in the layout of vfgs_b200_get_state. */
 size_t vfgs_b200_session_get_state(const vfgs_b200_session* s, void* dst, size_t cap);
 

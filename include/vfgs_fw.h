@@ -23,6 +23,8 @@
 
 #include <stdint.h>
 
+#include "vfgs_b200.h"
+
 #ifdef __cplusplus
 extern "C" {
 #endif
@@ -76,6 +78,37 @@ typedef struct fgs_afgs1_s {
  * the reference (src/vfgs_main.c:750-757). */
 int vfgs_b200_init_sei(const fgs_sei* cfg);
 int vfgs_b200_init_afgs1(const fgs_afgs1* cfg);
+
+/* ---- Metadata of grain sessions (vfgs_b200.h): many sessions re-programmed in one asynchronous device call ----------
+ *
+ * Film grain metadata can change with every picture. One entry gives one session new metadata; one call takes a whole
+ * list, e.g. every stream of a round, and costs one kernel launch, one copy of the entries to the device and one copy
+ * of the new patterns back. The global state, its table images and the global firmware's working memory are not
+ * touched. */
+typedef struct vfgs_b200_session_metadata {
+	vfgs_b200_session* session;
+	const fgs_sei*     sei;    /* exactly one of the two is set */
+	const fgs_afgs1*   afgs1;
+} vfgs_b200_session_metadata;
+
+/* n entries, asynchronous on `stream` (a cudaStream_t, NULL = default stream).
+ *   State: each entry leaves its session in exactly the state vfgs_b200_init_sei / _afgs1 would leave the global state
+ *   in, were the session's state the global one: patterns, LUTs, scale shift, clip range and registers (AFGS1 reseeds
+ *   and sets the clip range; SEI leaves the registers alone: vfgs_b200_session_set_seed). Each session has its own copy
+ *   of the firmware's working memory, taken from the global one when the session was created, so a session behaves like
+ *   its own copy of the reference's process from that point on (with 4:2:2 / 4:4:4, the chroma patterns of an SEI
+ *   message read what earlier patterns left in that memory).
+ *   Ordering: jobs enqueued after the call, on any stream, use the new metadata; jobs enqueued before keep the old
+ *   tables, even while they still run (the call's device work waits on the device for them). The call never waits on
+ *   the host for device work, except to reuse its own page-locked staging two calls later, or when that staging grows.
+ *   vfgs_b200_session_get_state waits for the new patterns to arrive on the host.
+ *   Refused with VFGS_B200_ERR_ARG / _ERR_STATE before any device work or any change to any session: n < 0, a null
+ *   list or session, both or neither metadata pointers set, the same session twice, non-increasing AFGS1 scaling points,
+ *   ar_coeff_lag outside 1..3, more patterns than the hardware holds, a scale shift outside 2..7 (scale_shift + bs
+ *   outside 8..13), table images that do not fit shared memory. A refused call leaves every session as it was. (This is
+ *   stricter than vfgs_b200_init_sei / _afgs1, which, like the reference, have already set the LUTs when they refuse a
+ *   scale shift.) */
+int vfgs_b200_session_init_metadata(const vfgs_b200_session_metadata* list, int n, void* stream);
 
 #ifdef __cplusplus
 }

@@ -31,7 +31,8 @@ B200_SYMBOLS = (
     "vfgs_b200_force_general_kernel", "vfgs_b200_pipeline_stats", "vfgs_b200_init_sei", "vfgs_b200_init_afgs1",
     "vfgs_b200_add_grain_semiplanar_device", "vfgs_b200_session_create", "vfgs_b200_session_destroy",
     "vfgs_b200_session_get_lfsr", "vfgs_b200_session_set_lfsr", "vfgs_b200_session_skip_frames",
-    "vfgs_b200_session_get_state", "vfgs_b200_add_grain_jobs_device",
+    "vfgs_b200_session_get_state", "vfgs_b200_add_grain_jobs_device", "vfgs_b200_session_set_seed",
+    "vfgs_b200_session_init_metadata",
 )
 NV12, P010 = 1, 2  # VFGS_B200_NV12 / VFGS_B200_P010
 
@@ -62,6 +63,11 @@ def surface_planes(t, height: int, fmt: int) -> SemiPlanes:
     pitch = t.shape[2] * t.element_size()
     base = t.data_ptr()
     return SemiPlanes(base, base + height * pitch, pitch, pitch, t.shape[1] * pitch, fmt)
+
+
+class _CMetadata(C.Structure):
+    """vfgs_b200_session_metadata (include/vfgs_fw.h)."""
+    _fields_ = [("session", C.c_void_p), ("sei", C.c_void_p), ("afgs1", C.c_void_p)]
 
 
 class _CJob(C.Structure):
@@ -148,6 +154,8 @@ def load_library(global_symbols: bool = False) -> C.CDLL:
     L.vfgs_b200_session_get_state.argtypes = [vp, vp, C.c_size_t]
     L.vfgs_b200_session_get_state.restype = C.c_size_t
     L.vfgs_b200_add_grain_jobs_device.argtypes = [C.POINTER(_CJob), ci, vp]
+    L.vfgs_b200_session_set_seed.argtypes = [vp, C.c_uint32]
+    L.vfgs_b200_session_init_metadata.argtypes = [C.POINTER(_CMetadata), ci, vp]
     _lib = L
     return L
 
@@ -299,6 +307,24 @@ class VfgsHw:
             c.nframes, c.width, c.height, c.out_depth = j.nframes, j.width, j.height, j.out_depth
         self._chk(self.L.vfgs_b200_add_grain_jobs_device(arr, len(jobs), C.c_void_p(stream.cuda_stream)))
 
+    def init_sessions(self, entries, stream=None):
+        """entries: a list of ``(session, kind, raw)`` with kind ``"sei"`` or ``"afgs1"`` and raw the bytes of an fgs_sei /
+        fgs_afgs1 struct. Re-programs every session from its metadata in one asynchronous device call on ``stream`` (a
+        torch.cuda.Stream; default: torch's current stream), see vfgs_b200_session_init_metadata."""
+        import torch
+        if stream is None:
+            stream = torch.cuda.current_stream()
+        arr = (_CMetadata * max(len(entries), 1))()
+        keep = []
+        for k, (session, kind, raw) in enumerate(entries):
+            if kind not in ("sei", "afgs1"):
+                raise VfgsError(f"metadata kind {kind!r}: 'sei' or 'afgs1'")
+            buf = (C.c_uint8 * len(raw)).from_buffer_copy(raw)
+            keep.append(buf)
+            arr[k].session = session.handle if session is not None else None
+            setattr(arr[k], kind, C.cast(buf, C.c_void_p))
+        self._chk(self.L.vfgs_b200_session_init_metadata(arr, len(entries), C.c_void_p(stream.cuda_stream)))
+
 
 class Session:
     """One video stream's grain state (vfgs_b200_session): patterns, LUTs, scalars and LFSR registers, independent of
@@ -338,6 +364,18 @@ class Session:
 
     def skip_frames(self, n, width, height):
         self.hw._chk(self.L.vfgs_b200_session_skip_frames(C.c_void_p(self.handle), n, width, height))
+
+    def set_seed(self, seed):
+        """vfgs_set_seed on the session's registers."""
+        self.hw._chk(self.L.vfgs_b200_session_set_seed(C.c_void_p(self.handle), seed & 0xFFFFFFFF))
+
+    def init_sei(self, raw: bytes, stream=None):
+        """This session's FGC SEI metadata (the bytes of an fgs_sei struct): VfgsHw.init_sessions with one entry."""
+        self.hw.init_sessions([(self, "sei", raw)], stream)
+
+    def init_afgs1(self, raw: bytes, stream=None):
+        """This session's AFGS1 metadata (the bytes of an fgs_afgs1 struct): VfgsHw.init_sessions with one entry."""
+        self.hw.init_sessions([(self, "afgs1", raw)], stream)
 
     def get_state(self) -> dict:
         n = self.L.vfgs_b200_session_get_state(C.c_void_p(self.handle), None, 0)

@@ -44,6 +44,8 @@ inline void make_fw_tables(FwTables& t)
 
 enum FwKind { kFwFF64 = 0, kFwFF32 = 1, kFwAR = 2 };
 
+constexpr int kFwMaxPatterns = 8; // VFGS_MAX_PATTERNS, vfgs_hw.h:49
+
 struct FwJob {
 	int kind;
 	int bank, slot;       // destination pattern[bank][slot] (bank 0: vfgs_set_luma_pattern, 1: vfgs_set_chroma_pattern)
@@ -119,7 +121,7 @@ VFGS_HD void fw_ff_phase3(const FwJob& j, const FwTables& t, FwScratch& s, int t
 }
 
 // ---- auto-regressive pattern ------------------------------------------------------------------
-// phase 0 (one thread): the causal filter in raster order, vfgs_fw.c:465-495
+// phase 0 (one thread): the causal filter in raster order, vfgs_fw.c:465-495 (the host reference of the wavefront below)
 // buf: the field being generated (82 x 73 or 44 x 38 bytes; shared memory on the device), buf0: the luma field,
 // gauss: the Gaussian table
 VFGS_HD void fw_ar_phase0(const FwJob& j, const int8_t* gauss, int8_t* buf, const int8_t* buf0)
@@ -148,6 +150,70 @@ VFGS_HD void fw_ar_phase0(const FwJob& j, const int8_t* gauss, int8_t* buf, cons
 			buf[width * y + x] = (int8_t)(g > 127 ? 127 : g < -127 ? -127 : g);
 		}
 }
+// The same filter as data-parallel phases (the device form, fw_pattern_kernel and fw_sessions_kernel).
+// Noise: the Gaussian term of sample (x, y) is read at the LFSR after y * width + x steps from the seed. Thread tid of
+// nthreads takes one contiguous run of samples: one jump-ahead to its start (pow2: JumpTable as uint32[64][32]), then a
+// walk. noise: width * height bytes.
+VFGS_HD int fw_parity(uint32_t x)
+{
+#if defined(__CUDA_ARCH__)
+	return __popc(x) & 1;
+#else
+	return __builtin_popcount(x) & 1;
+#endif
+}
+VFGS_HD uint32_t fw_lfsr_jump(const uint32_t* pow2, uint32_t x, uint32_t n)
+{
+	for (int k = 0; n; k++, n >>= 1)
+		if (n & 1u) {
+			uint32_t y = 0;
+			for (int i = 0; i < 32; i++) y |= (uint32_t)fw_parity(pow2[k * 32 + i] & x) << i;
+			x = y;
+		}
+	return x;
+}
+VFGS_HD void fw_ar_noise(const FwJob& j, const int8_t* gauss, const uint32_t* pow2, int8_t* noise, int tid, int nthreads)
+{
+	const int sub = j.size == 32 ? 2 : 1;
+	const int n = sub > 1 ? 44 * 38 : 82 * 73;
+	const int chunk = (n + nthreads - 1) / nthreads, i0 = tid * chunk, i1 = i0 + chunk < n ? i0 + chunk : n;
+	if (i0 >= i1) return;
+	uint32_t rnd = fw_lfsr_jump(pow2, j.seed, (uint32_t)i0);
+	for (int i = i0; i < i1; i++) {
+		noise[i] = (int8_t)fw_round((int)gauss[rnd & 2047], j.shift);
+		rnd = lfsr_step(rnd);
+	}
+}
+// Wavefront: sample (x, y) reads (x-3..x-1, y) and (x-3..x+3, y-3..y-1), all of smaller t = x + 4y, so the samples of
+// one t are independent: step t computes them, one per lane (at most ceil(82 / 4) = 21 of them), and a warp barrier
+// separates the steps. The tap sum is integer, so the order does not change it: the result is fw_ar_phase0's, byte for
+// byte. buf0 (the luma field) must not overlap buf.
+VFGS_HD int fw_ar_wave_steps(const FwJob& j) { return j.size == 32 ? 44 + 4 * 37 : 82 + 4 * 72; }
+VFGS_HD void fw_ar_wave_step(const FwJob& j, const int8_t* noise, int8_t* buf, const int8_t* buf0, int t, int lane)
+{
+	const int sub = j.size == 32 ? 2 : 1;
+	const int width = sub > 1 ? 44 : 82, height = sub > 1 ? 38 : 73;
+	const int y = (t >= width ? (t - width + 4) >> 2 : 0) + lane; // smallest y with x = t - 4y < width, + lane
+	const int x = t - 4 * y;
+	if (x < 0 || y >= height) return;
+	int g = 0;
+	if (y >= 3 && x >= 3 && x < width - 3) {
+		for (int jj = -3; jj <= 0; jj++)
+			for (int i = -3; i <= 3 && (i < 0 || jj < 0); i++)
+				g += (int)j.coef[3 + jj][3 + i] * buf[width * (y + jj) + x + i];
+		if (j.cx && j.use_luma) { // luma injection, indexed as in fw_ar_phase0
+			const int i = (x - 3) * sub + 3, jj = (y - 3) * sub + 3;
+			int Z = buf0[width * sub * jj + i];
+			if (sub > 1) Z += buf0[width * sub * jj + i + 1];
+			if (sub > 1) Z += buf0[width * sub * (jj + 1) + i] + buf0[width * sub * (jj + 1) + i + 1];
+			g += j.cx * fw_round(Z, 2 * sub - 2);
+		}
+		g = fw_round(g, j.scale);
+	}
+	g += noise[width * y + x];
+	buf[width * y + x] = (int8_t)(g > 127 ? 127 : g < -127 ? -127 : g);
+}
+
 // phase 1: cropped area to P (vfgs_fw.c:497-501)
 VFGS_HD void fw_ar_phase1(const FwJob& j, FwScratch& s, int tid, int nthreads)
 {

@@ -9,10 +9,9 @@
 
 #include "../../include/vfgs_fw.h"
 #include "fw_device.h"
+#include "vfgs_tables.h"
 
 namespace vfgs {
-
-constexpr int kFwMaxPatterns = 8; // VFGS_MAX_PATTERNS, vfgs_hw.h:49
 
 struct FwPlan {
 	std::vector<FwJob> jobs;    // in the firmware's order (they share one pattern buffer, fw_device.h)
@@ -184,6 +183,22 @@ inline void fw_plan_afgs1(const fgs_afgs1& cfg, int csubx, int csuby, FwPlan& pl
 	memset(plan.plut[2], 1, 256); // >> 4 in the hardware: Cr reads chroma slot 0 as well (vfgs_hw.c:212)
 	plan.scale_shift = cfg.grain_scaling - 6;
 	plan.set_legal = true; plan.legal = cfg.clip_to_restricted_range;
+}
+
+// The host half of a firmware update (vfgs_fw.c:592-643, :697-707 through the setters): seed, LUTs, scale shift and clip
+// range into h, in the firmware's order. Returns false where the reference asserts on the scale shift (vfgs_hw.c:348);
+// the seed and the LUTs are then already set, as in the reference.
+inline bool fw_apply_host(HwState& h, const FwPlan& plan)
+{
+	if (plan.set_seed) hw_set_seed(h, plan.seed);
+	for (int cc = 0; cc < 3; cc++) {
+		hw_set_scale_lut(h, cc, plan.slut[cc]);
+		hw_set_pattern_lut(h, cc, plan.plut[cc]);
+	}
+	if (plan.scale_shift < 2 || plan.scale_shift >= 8) return false;
+	hw_set_scale_shift(h, plan.scale_shift);
+	if (plan.set_legal) hw_set_legal_range(h, plan.legal);
+	return true;
 }
 
 } // namespace vfgs

@@ -45,6 +45,17 @@ struct ImageSet {
 	bool in_use = false;
 };
 constexpr size_t kBlockTableBytes = sizeof(uint32_t) + 4 * sizeof(uint16_t); // per block: LFSR register + window offsets
+// Page-locked destination of the pattern copy back of a metadata call; done: the copy has arrived.
+struct PinBlock {
+	uint8_t* h = nullptr;
+	size_t cap = 0;
+	cudaEvent_t done = nullptr;
+	~PinBlock()
+	{
+		if (h) cudaFreeHost(h);
+		if (done) cudaEventDestroy(done);
+	}
+};
 
 struct Context {
 	bool ready = false;
@@ -88,6 +99,17 @@ struct Context {
 	int multi_smem_attr[512] = {}; // per group key (group_key): the MULTI kernel's dynamic shared memory attribute
 	int multi_occ_smem[512] = {}, multi_per_sm[512] = {}; // per group key: occupancy asked for that shared-memory size
 	std::vector<std::shared_ptr<CUevent_st>> call_events; // end-of-call events of batched calls, reused once no session holds one
+	// metadata calls on sessions (vfgs_b200_session_init_metadata): entry descriptors staged and copied like h_desc /
+	// d_desc, the new patterns written to d_meta_out and copied back into page-locked blocks that the sessions hold until
+	// they merge them (meta_pool, reused once no session holds a block and its copy is done)
+	uint8_t* h_meta[2] = {nullptr, nullptr};
+	uint8_t* d_meta[2] = {nullptr, nullptr};
+	int8_t* d_meta_out[2] = {nullptr, nullptr};
+	size_t hmeta_cap[2] = {0, 0}, meta_cap[2] = {0, 0}, meta_out_cap[2] = {0, 0};
+	cudaEvent_t meta_copied[2] = {nullptr, nullptr}, meta_free[2] = {nullptr, nullptr};
+	bool meta_used[2] = {false, false};
+	unsigned meta_next = 0;
+	std::vector<std::shared_ptr<PinBlock>> meta_pool;
 	Slot slot[kPipeSlots];
 	uint8_t* d_line = nullptr; // compat line path staging
 	size_t line_cap = 0;
@@ -227,6 +249,8 @@ int ensure_ctx(int device)
 		CUDA_TRY(cudaEventCreateWithFlags(&c.tab_ready[t], cudaEventDisableTiming));
 		CUDA_TRY(cudaEventCreateWithFlags(&c.tab_free[t], cudaEventDisableTiming));
 		CUDA_TRY(cudaEventCreateWithFlags(&c.desc_copied[t], cudaEventDisableTiming));
+		CUDA_TRY(cudaEventCreateWithFlags(&c.meta_copied[t], cudaEventDisableTiming));
+		CUDA_TRY(cudaEventCreateWithFlags(&c.meta_free[t], cudaEventDisableTiming));
 	}
 	for (ImageSet& m : c.img) { // fixed-size allocations: nothing is (re)allocated, hence nothing synchronises, on a configuration change
 		CUDA_TRY(cudaMalloc((void**)&m.d_blob, kImageBlobCap));
@@ -780,6 +804,21 @@ struct vfgs_b200_session {
 	ImageSet img;
 	bool uploaded = false; // the upload is known to be complete: launches need not wait for it
 	std::shared_ptr<CUevent_st> last_batch;
+	// metadata (vfgs_b200_session_init_metadata): the firmware's working memory (forked from the global one at create);
+	// from the first call on, a device pattern store, images of the maximum size (img.d_blob / d_fblob then point there;
+	// the snapshot-sized ones stay until destroy, since kernels queued before may read them) and pattern copies on their
+	// way back to hw.pattern (merged by vfgs_b200_session_get_state)
+	FwScratch* d_fw_scratch = nullptr;
+	int8_t* d_pattern = nullptr;
+	int8_t* h_pattern = nullptr; // page-locked staging of the first upload of the pattern store
+	uint8_t *d_blob0 = nullptr, *d_fblob0 = nullptr;
+	Minus128 m128;
+	struct Pending {
+		std::shared_ptr<PinBlock> blk;
+		size_t off;
+		std::vector<FwJob> jobs; // bank, slot of each 4096-byte copy
+	};
+	std::vector<Pending> pending;
 };
 
 namespace {
@@ -1082,6 +1121,18 @@ int run_jobs(const vfgs_b200_job* jobs, int njobs, cudaStream_t st)
 	return rc;
 }
 
+// The firmware's constant tables on the device (global firmware calls and metadata calls on sessions).
+int ensure_fw_tables()
+{
+	Context& c = g_ctx;
+	if (c.d_fw_tables) return VFGS_B200_OK;
+	static FwTables tables;
+	make_fw_tables(tables);
+	CUDA_TRY(cudaMalloc((void**)&c.d_fw_tables, sizeof(FwTables)));
+	CUDA_TRY(cudaMemcpy(c.d_fw_tables, &tables, sizeof(FwTables), cudaMemcpyHostToDevice));
+	return VFGS_B200_OK;
+}
+
 int create_session(vfgs_b200_session** out)
 {
 	if (!out) return set_err(VFGS_B200_ERR_ARG, "null session pointer");
@@ -1109,6 +1160,7 @@ int create_session(vfgs_b200_session** out)
 		if (m.h_stage) cudaFreeHost(m.h_stage);
 		if (m.uploaded) cudaEventDestroy(m.uploaded);
 		if (m.last_use) cudaEventDestroy(m.last_use);
+		if (s->d_fw_scratch) cudaFree(s->d_fw_scratch);
 		return rc;
 	};
 	const size_t gb = (size_t)s->bi.gbytes, fb = (size_t)s->bi.fbytes;
@@ -1122,13 +1174,185 @@ int create_session(vfgs_b200_session** out)
 	memcpy(m.h_stage + gb, fblob.data(), fb);
 	SESSION_TRY(cudaMemcpyAsync(m.d_blob, m.h_stage, gb, cudaMemcpyHostToDevice, c.s_tab));
 	SESSION_TRY(cudaMemcpyAsync(m.d_fblob, m.h_stage + gb, fb, cudaMemcpyHostToDevice, c.s_tab));
+	// the firmware's working memory forks here: a copy of the global one (whose pattern jobs run on the table stream too),
+	// or zeros where the global firmware never ran
+	SESSION_TRY(cudaMalloc((void**)&s->d_fw_scratch, sizeof(FwScratch)));
+	if (c.d_fw_scratch) SESSION_TRY(cudaMemcpyAsync(s->d_fw_scratch, c.d_fw_scratch, sizeof(FwScratch), cudaMemcpyDeviceToDevice, c.s_tab));
+	else SESSION_TRY(cudaMemsetAsync(s->d_fw_scratch, 0, sizeof(FwScratch), c.s_tab));
 	SESSION_TRY(cudaEventRecord(m.uploaded, c.s_tab));
+	scan_minus128(s->hw, s->m128);
 	if (s->bi.bytes > c.smem_attr) { // the general kernel of the single-job route
 		SESSION_TRY(cudaFuncSetAttribute(fgs_apply_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, s->bi.bytes));
 		c.smem_attr = s->bi.bytes;
 	}
 #undef SESSION_TRY
 	*out = s.release();
+	return VFGS_B200_OK;
+}
+
+// Pattern copies of earlier metadata calls into the session's mirror, in call order, with the setters' copy rules
+// (vfgs_hw.c:314-325). wait: wait for copies still in flight; else stop at the first one that has not arrived.
+void merge_patterns(vfgs_b200_session* s, bool wait)
+{
+	size_t k = 0;
+	for (; k < s->pending.size(); k++) {
+		const vfgs_b200_session::Pending& p = s->pending[k];
+		if (wait) cudaEventSynchronize(p.blk->done);
+		else if (cudaEventQuery(p.blk->done) != cudaSuccess) break;
+		HwState& h = s->hw;
+		for (size_t i = 0; i < p.jobs.size(); i++) {
+			const FwJob& j = p.jobs[i];
+			const int8_t* src = (const int8_t*)p.blk->h + p.off + i * 4096;
+			if (j.bank == 0) memcpy(h.pattern[0][j.slot], src, 4096);
+			else
+				for (int r = 0; r < 64 / h.csuby; r++) memcpy(h.pattern[1][j.slot][r], src + 64 * r, (size_t)(64 / h.csubx));
+		}
+	}
+	s->pending.erase(s->pending.begin(), s->pending.begin() + (ptrdiff_t)k);
+}
+
+// vfgs_b200_session_init_metadata: every check on the host first, then one descriptor upload, one fw_sessions_kernel
+// launch and one pattern copy back on `st`, and the host half of every update applied to its session's mirror.
+int init_metadata(const vfgs_b200_session_metadata* list, int n, cudaStream_t st)
+{
+	if (n < 0) return set_err(VFGS_B200_ERR_ARG, "negative entry count");
+	if (n && !list) return set_err(VFGS_B200_ERR_ARG, "null metadata list");
+	if (!n) return VFGS_B200_OK;
+	struct Entry {
+		vfgs_b200_session* s;
+		FwPlan plan;
+		TableInfo bi;
+		Minus128 m128;
+		size_t out; // index of its first pattern copy
+	};
+	std::vector<Entry> ent((size_t)n);
+	std::vector<vfgs_b200_session*> seen((size_t)n);
+	for (int k = 0; k < n; k++) {
+		const vfgs_b200_session_metadata& e = list[k];
+		if (!e.session) return set_err(VFGS_B200_ERR_ARG, "entry %d: null session", k);
+		if (!e.sei == !e.afgs1) return set_err(VFGS_B200_ERR_ARG, "entry %d: set exactly one of sei and afgs1", k);
+		seen[(size_t)k] = e.session;
+	}
+	std::sort(seen.begin(), seen.end());
+	if (std::adjacent_find(seen.begin(), seen.end()) != seen.end()) return set_err(VFGS_B200_ERR_ARG, "a session appears twice in one list");
+	if (int rc = ensure_ctx(-1)) return rc;
+	Context& c = g_ctx;
+	size_t ncopies = 0;
+	for (int k = 0; k < n; k++) { // plans and the checks of the state they lead to; nothing is changed yet
+		Entry& E = ent[(size_t)k];
+		E.s = list[k].session;
+		const HwState& h = E.s->hw;
+		if (list[k].sei) fw_plan_sei(*list[k].sei, h.csubx, h.csuby, E.plan);
+		else fw_plan_afgs1(*list[k].afgs1, h.csubx, h.csuby, E.plan);
+		if (E.plan.error) return set_err(VFGS_B200_ERR_STATE, "entry %d: %s", k, E.plan.error);
+		if ((int)E.plan.jobs.size() > 2 * kFwMaxPatterns) return set_err(VFGS_B200_ERR_STATE, "entry %d: too many patterns", k);
+		if (E.plan.scale_shift < 2 || E.plan.scale_shift >= 8)
+			return set_err(VFGS_B200_ERR_STATE, "entry %d: scale shift %d outside 2..7 (the reference asserts, vfgs_hw.c:348)", k, E.plan.scale_shift);
+		const int ss = E.plan.scale_shift + 6 - h.bs; // vfgs_set_scale_shift
+		if (ss + h.bs < 8 || ss + h.bs > 13)
+			return set_err(VFGS_B200_ERR_STATE, "entry %d: scale_shift %d + bs %d outside 8..13 (vfgs_hw.c:170)", k, ss, h.bs);
+		for (int cc = 0; cc < 3; cc++)
+			for (int i = 0; i < 256; i++)
+				if ((E.plan.plut[cc][i] >> 4) >= kSlots) return set_err(VFGS_B200_ERR_STATE, "entry %d: pattern LUT selects slot %d", k, E.plan.plut[cc][i] >> 4);
+		// firmware output is clipped to +-127 (fw_device.h): the slots it writes hold no -128 where the images read
+		E.m128 = E.s->m128;
+		for (const FwJob& j : E.plan.jobs) E.m128.used[j.bank][j.slot] = false;
+		layout_tables(E.plan.plut, h.csubx, h.csuby, E.m128, E.bi);
+		if (E.bi.bytes > c.max_smem_optin - 1024)
+			return set_err(VFGS_B200_ERR_STATE, "entry %d: table image of %d bytes exceeds shared memory", k, E.bi.bytes);
+		if ((size_t)E.bi.gbytes > kImageBlobCap || (size_t)E.bi.fbytes > kImageFblobCap)
+			return set_err(VFGS_B200_ERR_STATE, "entry %d: table images of %d + %d bytes exceed their buffers", k, E.bi.gbytes, E.bi.fbytes);
+		E.out = ncopies;
+		ncopies += E.plan.jobs.size();
+	}
+	if (int rc = ensure_fw_tables()) return rc;
+	const int t = (int)(c.meta_next++ & 1u);
+	const size_t dbytes = sizeof(MetaEntry) * (size_t)n, obytes = (ncopies ? ncopies : 1) * 4096;
+	// the staging buffer's previous copy has left it (two calls ago); d_meta / d_meta_out are free once that call's
+	// copy back is done (a wait on the device, except when a buffer has to grow)
+	if (c.meta_used[t]) CUDA_TRY(cudaEventSynchronize(c.meta_copied[t]));
+	if (c.meta_used[t] && (dbytes > c.meta_cap[t] || obytes > c.meta_out_cap[t])) CUDA_TRY(cudaEventSynchronize(c.meta_free[t]));
+	if (int rc = grow(c.d_meta[t], c.meta_cap[t], dbytes)) return rc;
+	if (int rc = grow(c.d_meta_out[t], c.meta_out_cap[t], obytes)) return rc;
+	if (int rc = grow_host(c.h_meta[t], c.hmeta_cap[t], dbytes)) return rc;
+	if (c.meta_used[t]) CUDA_TRY(cudaStreamWaitEvent(st, c.meta_free[t], 0));
+	// the page-locked block the patterns come back to: one no session holds any more whose copy is done, else a new one
+	std::shared_ptr<PinBlock> blk;
+	for (const std::shared_ptr<PinBlock>& b : c.meta_pool)
+		if (b.use_count() == 1 && b->cap >= obytes && cudaEventQuery(b->done) == cudaSuccess) { blk = b; break; }
+	if (!blk) {
+		blk = std::make_shared<PinBlock>();
+		CUDA_TRY(cudaEventCreateWithFlags(&blk->done, cudaEventDisableTiming));
+		const size_t cap = std::max(obytes, (size_t)64 << 10);
+		CUDA_TRY(cudaHostAlloc((void**)&blk->h, cap, cudaHostAllocDefault));
+		blk->cap = cap;
+		c.meta_pool.push_back(blk);
+	}
+	// first call on a session: its pattern store (the snapshot's patterns) and images of the maximum size
+	for (Entry& E : ent) {
+		vfgs_b200_session* s = E.s;
+		if (s->d_pattern) continue;
+		uint8_t *b = nullptr, *f = nullptr;
+		CUDA_TRY(cudaMalloc((void**)&s->d_pattern, sizeof(s->hw.pattern)));
+		CUDA_TRY(cudaHostAlloc((void**)&s->h_pattern, sizeof(s->hw.pattern), cudaHostAllocDefault));
+		CUDA_TRY(cudaMalloc((void**)&b, kImageBlobCap));
+		if (cudaMalloc((void**)&f, kImageFblobCap) != cudaSuccess) { cudaFree(b); return set_err(VFGS_B200_ERR_CUDA, "cudaMalloc of session images"); }
+		memcpy(s->h_pattern, s->hw.pattern, sizeof(s->hw.pattern));
+		CUDA_TRY(cudaMemcpyAsync(s->d_pattern, s->h_pattern, sizeof(s->hw.pattern), cudaMemcpyHostToDevice, st));
+		s->d_blob0 = s->img.d_blob; s->d_fblob0 = s->img.d_fblob;
+		s->img.d_blob = b; s->img.d_fblob = f;
+	}
+	// descriptors
+	MetaEntry* md = (MetaEntry*)c.h_meta[t];
+	for (int k = 0; k < n; k++) {
+		const Entry& E = ent[(size_t)k];
+		MetaEntry& m = md[k];
+		memset(&m, 0, sizeof(m));
+		for (size_t i = 0; i < E.plan.jobs.size(); i++) m.jobs[i] = E.plan.jobs[i];
+		m.njobs = (int)E.plan.jobs.size();
+		m.csubx = E.s->hw.csubx; m.csuby = E.s->hw.csuby;
+		memcpy(m.slut, E.plan.slut, sizeof(m.slut));
+		memcpy(m.plut, E.plan.plut, sizeof(m.plut));
+		m.bi = E.bi;
+		m.scratch = E.s->d_fw_scratch;
+		m.pattern = E.s->d_pattern;
+		m.blob = E.s->img.d_blob; m.fblob = E.s->img.d_fblob;
+		m.out = c.d_meta_out[t] + E.out * 4096;
+	}
+	CUDA_TRY(cudaMemcpyAsync(c.d_meta[t], c.h_meta[t], dbytes, cudaMemcpyHostToDevice, st));
+	CUDA_TRY(cudaEventRecord(c.meta_copied[t], st));
+	c.meta_used[t] = true;
+	// the kernel rewrites what earlier jobs of these sessions read (images) and what their creation wrote (working
+	// memory, first images): it waits on the device for those
+	for (Entry& E : ent) {
+		vfgs_b200_session* s = E.s;
+		CUDA_TRY(cudaStreamWaitEvent(st, s->img.uploaded, 0));
+		if (s->img.in_use) CUDA_TRY(cudaStreamWaitEvent(st, s->img.last_use, 0));
+		if (s->last_batch) CUDA_TRY(cudaStreamWaitEvent(st, s->last_batch.get(), 0));
+	}
+	fw_sessions_kernel<<<n, kFwThreads, 0, st>>>((const MetaEntry*)c.d_meta[t], c.d_fw_tables, c.d_pow2);
+	CUDA_TRY(cudaGetLastError());
+	g_launches++;
+	for (Entry& E : ent) { // later jobs of the session wait for its new images
+		CUDA_TRY(cudaEventRecord(E.s->img.uploaded, st));
+		E.s->uploaded = false;
+	}
+	if (ncopies) CUDA_TRY(cudaMemcpyAsync(blk->h, c.d_meta_out[t], ncopies * 4096, cudaMemcpyDeviceToHost, st));
+	CUDA_TRY(cudaEventRecord(blk->done, st));
+	CUDA_TRY(cudaEventRecord(c.meta_free[t], st));
+	// the host half: LUTs, scalars, registers and layout, so that jobs enqueued next plan against the new state
+	for (Entry& E : ent) {
+		vfgs_b200_session* s = E.s;
+		merge_patterns(s, false); // copies of earlier calls that have arrived
+		fw_apply_host(s->hw, E.plan);
+		s->bi = E.bi;
+		s->m128 = E.m128;
+		if (!E.plan.jobs.empty()) s->pending.push_back({blk, E.out * 4096, E.plan.jobs});
+		if (E.bi.bytes > c.smem_attr) { // the general kernel of the single-job route
+			CUDA_TRY(cudaFuncSetAttribute(fgs_apply_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, E.bi.bytes));
+			c.smem_attr = E.bi.bytes;
+		}
+	}
 	return VFGS_B200_OK;
 }
 
@@ -1159,7 +1383,7 @@ void vfgs_set_scale_lut(int c, uint8_t lut[]) // vfgs_hw.c:327-331
 {
 	pipe_before_state_change();
 	REQUIRE(c >= 0 && c < 3);
-	memcpy(hw().slut[c], lut, 256);
+	hw_set_scale_lut(hw(), c, lut);
 	g_dirty = true;
 }
 
@@ -1170,23 +1394,21 @@ void vfgs_set_pattern_lut(int c, uint8_t lut[]) // vfgs_hw.c:333-337
 	// Any table is accepted, like the reference does (vfgs_hw.c:333-337). lut[i] >> 4 indexes pattern[..][9] in
 	// vfgs_hw.c:218: an entry above slot 8 makes the reference read out of bounds if a sample ever hits it; here
 	// such a table is refused when grain is requested (make_geometry: VFGS_B200_ERR_STATE), not in the setter.
-	memcpy(hw().plut[c], lut, 256);
+	hw_set_pattern_lut(hw(), c, lut);
 	g_dirty = true;
 }
 
 void vfgs_set_seed(uint32_t seed) // vfgs_hw.c:339-344
 {
 	pipe_before_state_change();
-	HwState& h = hw();
-	h.rnd = h.rnd_up = h.line_rnd = h.line_rnd_up = seed << 1;
+	hw_set_seed(hw(), seed);
 }
 
 void vfgs_set_scale_shift(int shift) // vfgs_hw.c:346-350
 {
 	pipe_before_state_change();
 	REQUIRE(shift >= 2 && shift < 8);
-	HwState& h = hw();
-	h.scale_shift = shift + 6 - h.bs;
+	hw_set_scale_shift(hw(), shift);
 }
 
 void vfgs_set_depth(int depth) // vfgs_hw.c:352-362
@@ -1203,10 +1425,7 @@ void vfgs_set_depth(int depth) // vfgs_hw.c:352-362
 void vfgs_set_legal_range(int legal) // vfgs_hw.c:364-380
 {
 	pipe_before_state_change();
-	HwState& h = hw();
-	h.y_min = h.c_min = legal ? 16 : 0;
-	h.y_max = legal ? 235 : 255;
-	h.c_max = legal ? 240 : 255;
+	hw_set_legal_range(hw(), legal);
 }
 
 void vfgs_set_chroma_subsampling(int subx, int suby) // vfgs_hw.c:382-388
@@ -1472,8 +1691,14 @@ void vfgs_b200_session_destroy(vfgs_b200_session* s)
 	if (!s) return;
 	if (s->img.in_use) cudaEventSynchronize(s->img.last_use);
 	if (s->last_batch) cudaEventSynchronize(s->last_batch.get());
+	cudaEventSynchronize(s->img.uploaded); // creation uploads, or the last metadata kernel
 	cudaFree(s->img.d_blob);
 	cudaFree(s->img.d_fblob);
+	if (s->d_blob0) cudaFree(s->d_blob0);
+	if (s->d_fblob0) cudaFree(s->d_fblob0);
+	if (s->d_pattern) cudaFree(s->d_pattern);
+	if (s->h_pattern) cudaFreeHost(s->h_pattern);
+	cudaFree(s->d_fw_scratch);
 	cudaFreeHost(s->img.h_stage);
 	cudaEventDestroy(s->img.uploaded);
 	cudaEventDestroy(s->img.last_use);
@@ -1502,7 +1727,20 @@ int vfgs_b200_session_skip_frames(vfgs_b200_session* s, int64_t nframes, int wid
 	return VFGS_B200_OK;
 }
 
-size_t vfgs_b200_session_get_state(const vfgs_b200_session* s, void* dst, size_t cap) { return state_dump(s->hw, dst, cap); }
+size_t vfgs_b200_session_get_state(const vfgs_b200_session* s, void* dst, size_t cap)
+{
+	// patterns of metadata calls come back asynchronously: wait for them and merge them into the mirror first (the
+	// session is the caller's, not a constant object; the const of the signature is about its observable state)
+	if (dst && !s->pending.empty()) merge_patterns(const_cast<vfgs_b200_session*>(s), true);
+	return state_dump(s->hw, dst, cap);
+}
+
+int vfgs_b200_session_set_seed(vfgs_b200_session* s, uint32_t seed)
+{
+	if (!s) return set_err(VFGS_B200_ERR_ARG, "null session");
+	hw_set_seed(s->hw, seed);
+	return VFGS_B200_OK;
+}
 
 int vfgs_b200_add_grain_jobs_device(const vfgs_b200_job* jobs, int njobs, void* stream) { return run_jobs(jobs, njobs, (cudaStream_t)stream); }
 
@@ -1514,11 +1752,8 @@ namespace {
 int ensure_fw()
 {
 	Context& c = g_ctx;
-	if (c.d_fw_tables) return VFGS_B200_OK;
-	static FwTables tables;
-	make_fw_tables(tables);
-	CUDA_TRY(cudaMalloc((void**)&c.d_fw_tables, sizeof(FwTables)));
-	CUDA_TRY(cudaMemcpy(c.d_fw_tables, &tables, sizeof(FwTables), cudaMemcpyHostToDevice));
+	if (int rc = ensure_fw_tables()) return rc;
+	if (c.d_fw_scratch) return VFGS_B200_OK;
 	CUDA_TRY(cudaMalloc((void**)&c.d_fw_scratch, sizeof(FwScratch)));
 	CUDA_TRY(cudaMemset(c.d_fw_scratch, 0, sizeof(FwScratch)));
 	CUDA_TRY(cudaMalloc((void**)&c.d_fw_pattern, 2 * kSlots * 4096));
@@ -1528,8 +1763,8 @@ int ensure_fw()
 }
 
 // Pattern jobs on the table stream, results into the host mirror through the setters' copy rules, then LUTs and
-// scalars through the setters themselves. The host waits for the job kernels only (tens of microseconds each; the
-// auto-regressive filter is serial: ~0.2 ms): grain kernels queued on other streams keep running.
+// scalars with the setters' arithmetic (fw_apply_host). The host waits for the table stream, on which the job kernels
+// run (tens of microseconds each); grain kernels queued on other streams keep running.
 int fw_apply(FwPlan& plan)
 {
 	if (plan.error) return set_err(VFGS_B200_ERR_STATE, "%s", plan.error);
@@ -1541,7 +1776,7 @@ int fw_apply(FwPlan& plan)
 	HwState& h = hw();
 	for (size_t i = 0; i < plan.jobs.size(); i++) {
 		const FwJob& j = plan.jobs[i];
-		fw_pattern_kernel<<<1, kFwThreads, 0, c.s_tab>>>(j, c.d_fw_tables, c.d_fw_scratch, c.d_fw_pattern);
+		fw_pattern_kernel<<<1, kFwThreads, 0, c.s_tab>>>(j, c.d_fw_tables, c.d_pow2, c.d_fw_scratch, c.d_fw_pattern);
 		CUDA_TRY(cudaGetLastError());
 		g_launches++;
 		CUDA_TRY(cudaMemcpyAsync(c.h_fw_stage + i * 4096, c.d_fw_pattern + ((size_t)j.bank * kSlots + j.slot) * 4096, 4096,
@@ -1556,15 +1791,8 @@ int fw_apply(FwPlan& plan)
 			for (int r = 0; r < 64 / h.csuby; r++) memcpy(h.pattern[1][j.slot][r], src + 64 * r, (size_t)(64 / h.csubx));
 	}
 	g_dirty = true;
-	if (plan.set_seed) vfgs_set_seed(plan.seed);
-	for (int cc = 0; cc < 3; cc++) {
-		vfgs_set_scale_lut(cc, plan.slut[cc]);
-		vfgs_set_pattern_lut(cc, plan.plut[cc]);
-	}
-	if (plan.scale_shift < 2 || plan.scale_shift >= 8)
+	if (!fw_apply_host(h, plan))
 		return set_err(VFGS_B200_ERR_STATE, "scale shift %d outside 2..7 (the reference asserts, vfgs_hw.c:348)", plan.scale_shift);
-	vfgs_set_scale_shift(plan.scale_shift);
-	if (plan.set_legal) vfgs_set_legal_range(plan.legal);
 	return VFGS_B200_OK;
 }
 
@@ -1578,6 +1806,11 @@ int vfgs_b200_init_sei(const fgs_sei* cfg) // vfgs_fw.c:517-644
 	FwPlan plan;
 	fw_plan_sei(*cfg, hw().csubx, hw().csuby, plan);
 	return fw_apply(plan);
+}
+
+int vfgs_b200_session_init_metadata(const vfgs_b200_session_metadata* list, int n, void* stream)
+{
+	return init_metadata(list, n, (cudaStream_t)stream);
 }
 
 int vfgs_b200_init_afgs1(const fgs_afgs1* cfg) // vfgs_fw.c:663-708

@@ -372,22 +372,30 @@ fgs_apply_gather_multi_kernel(const __grid_constant__ MultiParams m)
 	}
 }
 
-// ---- firmware layer: one pattern job (fw_device.h) -----------------------------------------------
+// ---- firmware layer: pattern jobs (fw_device.h) -------------------------------------------------
 // One CTA per job, jobs of a configuration one after the other on the table stream (they share the firmware's pattern
 // buffer, fw_device.h). The frequency-filtering job is two 64 x 64 x 64 integer matrix passes spread over the CTA; the
-// auto-regressive filter is causal in raster order: one thread walks it in shared memory (6,000 samples x <= 24 taps).
+// auto-regressive filter takes the CTA for its noise term (lane-chunked LFSR walks from a jump-ahead each) and one warp
+// for the causal filter itself, which runs as a wavefront over anti-diagonals (fw_ar_wave_step: 370 steps for the
+// 82 x 73 luma field instead of a 5,986-sample serial walk).
 constexpr int kFwThreads = 256;
-__global__ void __launch_bounds__(kFwThreads)
-fw_pattern_kernel(const FwJob job, const FwTables* __restrict__ tables, FwScratch* scratch, int8_t* pattern)
+
+// The job's pattern into scratch->P. gauss: the Gaussian table in shared memory (AR jobs); noise, field: shared buffers
+// of 82 x 73 bytes.
+__device__ __forceinline__ void fw_make_pattern(const FwJob& job, const FwTables* __restrict__ tables, const uint32_t* __restrict__ pow2,
+                                                FwScratch* scratch, const int8_t* gauss, int8_t* noise, int8_t* field, int tid)
 {
-	__shared__ int8_t field[73 * 82];
-	__shared__ int8_t gauss[2048];
-	const int tid = threadIdx.x;
 	if (job.kind == kFwAR) {
 		const int sub = job.size == 32 ? 2 : 1, bytes = sub > 1 ? 44 * 38 : 82 * 73;
-		for (int i = tid; i < 2048; i += kFwThreads) gauss[i] = tables->gauss[i];
+		fw_ar_noise(job, gauss, pow2, noise, tid, kFwThreads);
 		__syncthreads();
-		if (tid == 0) fw_ar_phase0(job, gauss, field, scratch->Lbuf);
+		if (tid < 32) {
+			const int steps = fw_ar_wave_steps(job);
+			for (int t = 0; t < steps; t++) {
+				fw_ar_wave_step(job, noise, field, scratch->Lbuf, t, tid);
+				__syncwarp();
+			}
+		}
 		__syncthreads();
 		int8_t* keep = sub > 1 ? scratch->Cbuf : scratch->Lbuf; // the luma field stays for the chroma jobs (luma injection)
 		for (int i = tid; i < bytes; i += kFwThreads) keep[i] = field[i];
@@ -403,7 +411,61 @@ fw_pattern_kernel(const FwJob job, const FwTables* __restrict__ tables, FwScratc
 		fw_ff_phase3(job, *tables, *scratch, tid, kFwThreads);
 	}
 	__syncthreads();
+}
+
+__global__ void __launch_bounds__(kFwThreads)
+fw_pattern_kernel(const FwJob job, const FwTables* __restrict__ tables, const uint32_t* __restrict__ pow2, FwScratch* scratch, int8_t* pattern)
+{
+	__shared__ int8_t field[73 * 82];
+	__shared__ int8_t noise[73 * 82];
+	__shared__ int8_t gauss[2048];
+	const int tid = threadIdx.x;
+	if (job.kind == kFwAR) {
+		for (int i = tid; i < 2048; i += kFwThreads) gauss[i] = tables->gauss[i];
+		__syncthreads();
+	}
+	fw_make_pattern(job, tables, pow2, scratch, gauss, noise, field, tid);
 	fw_store_phase(job, *scratch, pattern, tid, kFwThreads);
+}
+
+// ---- firmware layer for sessions (vfgs_b200_session_init_metadata) ------------------------------------
+// One entry of a metadata call: a session's pattern jobs in firmware order, its new LUTs and image layout (host-made),
+// and where its firmware working memory, pattern store and table images live.
+struct MetaEntry {
+	FwJob jobs[2 * kFwMaxPatterns];
+	int njobs;
+	int csubx, csuby;
+	uint8_t slut[3][256], plut[3][256];
+	TableInfo bi;
+	FwScratch* scratch;
+	int8_t* pattern;       // int8 [2][9][64][64], the session's device pattern store
+	uint8_t *blob, *fblob; // the session's general and fast images (kImageBlobCap / kImageFblobCap bytes)
+	int8_t* out;           // njobs x 4096: each job's slot after its store, for the copy back to the host
+};
+
+// One CTA per entry: the entry's jobs one after the other against its session's working memory and pattern store, then
+// both table images from the pattern store and the new LUTs (fill_tables, the code build_tables runs on the host).
+__global__ void __launch_bounds__(kFwThreads)
+fw_sessions_kernel(const MetaEntry* __restrict__ entries, const FwTables* __restrict__ tables, const uint32_t* __restrict__ pow2)
+{
+	__shared__ int8_t field[73 * 82];
+	__shared__ int8_t noise[73 * 82];
+	__shared__ int8_t gauss[2048];
+	const MetaEntry& e = entries[blockIdx.x];
+	const int tid = threadIdx.x;
+	for (int i = tid; i < 2048; i += kFwThreads) gauss[i] = tables->gauss[i];
+	__syncthreads();
+	for (int k = 0; k < e.njobs; k++) {
+		const FwJob& job = e.jobs[k];
+		fw_make_pattern(job, tables, pow2, e.scratch, gauss, noise, field, tid);
+		fw_store_phase(job, *e.scratch, e.pattern, tid, kFwThreads);
+		__syncthreads();
+		const int8_t* slot = e.pattern + ((size_t)job.bank * kSlots + job.slot) * 4096;
+		for (int i = tid; i < 4096; i += kFwThreads) e.out[(size_t)k * 4096 + i] = slot[i];
+	}
+	__syncthreads();
+	const TableSrc src = {e.pattern, &e.slut[0][0], &e.plut[0][0], e.csubx, e.csuby};
+	fill_tables(src, e.bi, e.blob, e.fblob, tid, kFwThreads);
 }
 
 } // namespace vfgs

@@ -61,22 +61,59 @@ struct TableInfo {
 	int fpat_off[3][2], fpat_stride[3], fpat_copy[3], fbytes; // fpat_off: relative to the component image; fpat_copy: bytes from one column-shifted copy to the next
 };
 
+// The setters' arithmetic (vfgs_hw.c:327-380) on a given state: the global setters apply it to the global state, a
+// session's metadata update to the session's state.
+inline void hw_set_scale_lut(HwState& h, int c, const uint8_t* lut) { memcpy(h.slut[c], lut, 256); }
+inline void hw_set_pattern_lut(HwState& h, int c, const uint8_t* lut) { memcpy(h.plut[c], lut, 256); }
+inline void hw_set_seed(HwState& h, uint32_t seed) { h.rnd = h.rnd_up = h.line_rnd = h.line_rnd_up = seed << 1; }
+inline void hw_set_scale_shift(HwState& h, int shift) { h.scale_shift = shift + 6 - h.bs; }
+inline void hw_set_legal_range(HwState& h, int legal)
+{
+	h.y_min = h.c_min = legal ? 16 : 0;
+	h.y_max = legal ? 235 : 255;
+	h.c_max = legal ? 240 : 255;
+}
+
+// Which pattern slots may hold a -128 byte: the one property of the pattern bytes the image layout depends on (the
+// negated copies of sign folding and the fast image's -pattern must fit int8). used: the bytes the images read (64 x 64
+// for luma, (64/csuby) x (64/csubx) for chroma); rest: the other bytes of a chroma slot, which the sign-folding test
+// scans as well.
+struct Minus128 {
+	bool used[2][kSlots], rest[2][kSlots];
+};
+inline void scan_minus128(const HwState& h, Minus128& m)
+{
+	const int crows = 64 / h.csuby, ccols = 64 / h.csubx;
+	for (int b = 0; b < 2; b++)
+		for (int s = 0; s < kSlots; s++) {
+			m.used[b][s] = m.rest[b][s] = false;
+			for (int r = 0; r < 64; r++)
+				for (int x = 0; x < 64; x++)
+					if (h.pattern[b][s][r][x] == -128) {
+						if (b == 0 || (r < crows && x < ccols)) m.used[b][s] = true;
+						else m.rest[b][s] = true;
+					}
+		}
+}
+
 // General image layout (all offsets multiples of 16): LUT uint16[3][256] = scale | slot << 8, then the
 // luma slots in use (64 rows), then the chroma slots in use packed to (64/csuby) rows x (64/csubx) bytes;
-// rows cols + VFGS_PAT_ROW_SKEW bytes apart.
-inline void build_tables(const HwState& h, TableInfo& g_bi, std::vector<uint8_t>& g_blob, std::vector<uint8_t>& g_fblob)
+// rows cols + VFGS_PAT_ROW_SKEW bytes apart. Negated slot copies behind it, and the fast image, follow below.
+// The layout needs the pattern LUTs, the subsampling and the -128 flags only, so it is a host computation even where
+// the patterns themselves live on the device (sessions programmed from metadata).
+inline void layout_tables(const uint8_t plut[3][256], int csubx, int csuby, const Minus128& m, TableInfo& g_bi)
 {
 	int nslot[2] = {1, 1};
 	for (int c = 0; c < 3; c++) {
-		int first = h.plut[c][0] >> 4, uni = first;
+		int first = plut[c][0] >> 4, uni = first;
 		for (int i = 0; i < 256; i++) {
-			int s = h.plut[c][i] >> 4;
+			int s = plut[c][i] >> 4;
 			if (s != first) uni = -1;
 			if (s + 1 > nslot[c ? 1 : 0]) nslot[c ? 1 : 0] = s + 1;
 		}
 		g_bi.uniform_pi[c] = uni;
 	}
-	const int crows = 64 / h.csuby, ccols = 64 / h.csubx;
+	const int crows = 64 / csuby, ccols = 64 / csubx;
 	// pattern rows are stored cols + VFGS_PAT_ROW_SKEW bytes apart: the window rows are multiples of 4 (or 2), so
 	// with the natural power-of-two pitch the byte gathers of a line would fall into half of the banks
 	const int lpitch = 64 + VFGS_PAT_ROW_SKEW, cpitch = ccols + VFGS_PAT_ROW_SKEW;
@@ -90,32 +127,12 @@ inline void build_tables(const HwState& h, TableInfo& g_bi, std::vector<uint8_t>
 	for (int b = 0; b < 2; b++) { // negated copies of the banks' slots (gather kernel, sign folding)
 		g_bi.nslot[b] = nslot[b];
 		g_bi.neg_ok[b] = true;
-		for (int s = 0; s < nslot[b] && g_bi.neg_ok[b]; s++)
-			for (int r = 0; r < 64 && g_bi.neg_ok[b]; r++)
-				for (int x = 0; x < 64; x++)
-					if (h.pattern[b][s][r][x] == -128) { g_bi.neg_ok[b] = false; break; }
+		for (int s = 0; s < nslot[b]; s++)
+			if (m.used[b][s] || m.rest[b][s]) g_bi.neg_ok[b] = false;
 		g_bi.neg_off[b] = g_bi.gbytes - g_bi.pat_off[b]; // relative to the bank's plain slots
 		g_bi.gbytes += nslot[b] * g_bi.pat_size[b];
 	}
 	g_bi.gbytes = (g_bi.gbytes + 15) & ~15;
-	g_blob.assign((size_t)g_bi.gbytes, 0);
-	uint16_t* lut = (uint16_t*)g_blob.data();
-	for (int c = 0; c < 3; c++)
-		for (int i = 0; i < 256; i++) lut[c * 256 + i] = (uint16_t)(h.slut[c][i] | ((h.plut[c][i] >> 4) << 8));
-	for (int s = 0; s < nslot[0]; s++)
-		for (int r = 0; r < 64; r++)
-			memcpy(&g_blob[g_bi.pat_off[0] + s * g_bi.pat_size[0] + r * lpitch], h.pattern[0][s][r], 64);
-	for (int s = 0; s < nslot[1]; s++)
-		for (int r = 0; r < crows; r++)
-			memcpy(&g_blob[g_bi.pat_off[1] + s * g_bi.pat_size[1] + r * cpitch], h.pattern[1][s][r], (size_t)ccols);
-	for (int b = 0; b < 2; b++) {
-		if (!g_bi.neg_ok[b]) continue;
-		const int rows = b ? crows : 64, cols = b ? ccols : 64, pitch = g_bi.pat_stride[b];
-		for (int s = 0; s < nslot[b]; s++)
-			for (int r = 0; r < rows; r++)
-				for (int x = 0; x < cols; x++)
-					g_blob[g_bi.pat_off[b] + g_bi.neg_off[b] + s * g_bi.pat_size[b] + r * pitch + x] = (uint8_t)(int8_t)-h.pattern[b][s][r][x];
-	}
 
 	// fast-path image: compact scale LUT, then per component the single slot as +pattern and -pattern, each in
 	// fast_copies() column-shifted copies (copy k holds the pattern moved left by k * 8 / copies bytes), so that
@@ -124,12 +141,9 @@ inline void build_tables(const HwState& h, TableInfo& g_bi, std::vector<uint8_t>
 	g_bi.fshare_cbcr = false;
 	for (int c = 0; c < 3; c++) {
 		const int rows = c ? crows : 64, cols = c ? ccols : 64;
-		const int ncopy = fast_copies((c && h.csubx > 1) ? 8 : 16);
+		const int ncopy = fast_copies((c && csubx > 1) ? 8 : 16);
 		const int slot = g_bi.uniform_pi[c];
-		bool ok = slot >= 0;
-		for (int r = 0; ok && r < rows; r++)
-			for (int x = 0; x < cols; x++)
-				if (h.pattern[c ? 1 : 0][slot][r][x] == -128) { ok = false; break; }
+		const bool ok = slot >= 0 && !m.used[c ? 1 : 0][slot];
 		g_bi.fast_ok[c] = ok;
 		// row pitch = cols + VFGS_FAST_ROW_SKEW: the window rows oy are multiples of 4 (or 2), so with a power-of-two
 		// pitch every window of a line would start in the same few banks; the skew spreads them over all banks
@@ -148,24 +162,83 @@ inline void build_tables(const HwState& h, TableInfo& g_bi, std::vector<uint8_t>
 		}
 	}
 	g_bi.fbytes = (off + 15) & ~15;
-	g_fblob.assign((size_t)g_bi.fbytes, 0);
-	uint32_t* clut = (uint32_t*)g_fblob.data();
-	for (int i = 0; i < 256; i++) clut[i] = (uint32_t)h.slut[0][i] | ((uint32_t)h.slut[1][i] << 8) | ((uint32_t)h.slut[2][i] << 16);
-	for (int c = 0; c < 3; c++) {
-		if (!g_bi.fast_ok[c] || (c == 2 && g_bi.fshare_cbcr)) continue;
-		const int rows = c ? crows : 64, cols = c ? ccols : 64;
-		const int ncopy = fast_copies((c && h.csubx > 1) ? 8 : 16), shift = 8 / ncopy;
-		for (int k = 0; k < ncopy; k++) {
-			const int pitch = g_bi.fpat_stride[c];
-			int8_t* plus = (int8_t*)&g_fblob[g_bi.fimg_src[c] + g_bi.fpat_off[c][0] + k * g_bi.fpat_copy[c]];
-			int8_t* minus = (int8_t*)&g_fblob[g_bi.fimg_src[c] + g_bi.fpat_off[c][1] + k * g_bi.fpat_copy[c]];
-			for (int r = 0; r < rows; r++)
-				for (int x = 0; x + k * shift < cols; x++) {
-					const int8_t v = h.pattern[c ? 1 : 0][g_bi.uniform_pi[c]][r][x + k * shift];
-					plus[r * pitch + x] = v; minus[r * pitch + x] = (int8_t)-v;
-				}
-		}
+}
+
+// What the image bytes are made of: pattern int8 [2][9][64][64], sLUT and pLUT uint8 [3][256], the subsampling.
+struct TableSrc {
+	const int8_t* pattern;
+	const uint8_t* slut;
+	const uint8_t* plut;
+	int csubx, csuby;
+};
+VFGS_HD int8_t table_pattern(const TableSrc& s, int bank, int slot, int r, int x) { return s.pattern[((bank * kSlots + slot) * 64 + r) * 64 + x]; }
+
+// Byte o of the general image (layout_tables): every byte, padding included, so that a fill in any order and by any
+// number of threads gives the same image.
+VFGS_HD uint8_t general_image_byte(const TableSrc& s, const TableInfo& bi, int o)
+{
+	if (o < bi.pat_off[0]) { // LUT uint16[3][256], little-endian
+		const int e = o >> 1, c = e >> 8, i = e & 255;
+		const int v = s.slut[c * 256 + i] | ((s.plut[c * 256 + i] >> 4) << 8);
+		return (uint8_t)((o & 1) ? v >> 8 : v);
 	}
+	const int crows = 64 / s.csuby, ccols = 64 / s.csubx;
+	for (int neg = 0; neg < 2; neg++)
+		for (int b = 0; b < 2; b++) {
+			const int base = bi.pat_off[b] + (neg ? bi.neg_off[b] : 0);
+			if (o < base || o >= base + bi.nslot[b] * bi.pat_size[b]) continue;
+			if (neg && !bi.neg_ok[b]) return 0;
+			const int rel = o - base, slot = rel / bi.pat_size[b], in = rel - slot * bi.pat_size[b];
+			const int r = in / bi.pat_stride[b], x = in - r * bi.pat_stride[b];
+			if (r >= (b ? crows : 64) || x >= (b ? ccols : 64)) return 0;
+			const int8_t v = table_pattern(s, b, slot, r, x);
+			return (uint8_t)(neg ? (int8_t)-v : v);
+		}
+	return 0;
+}
+
+// Byte o of the fast image (layout_tables).
+VFGS_HD uint8_t fast_image_byte(const TableSrc& s, const TableInfo& bi, int o)
+{
+	if (o < 256 * 4) { // uint32 lut[256] = sLUT[Y] | sLUT[U] << 8 | sLUT[V] << 16
+		const int i = o >> 2, c = o & 3;
+		return c < 3 ? s.slut[c * 256 + i] : (uint8_t)0;
+	}
+	const int crows = 64 / s.csuby, ccols = 64 / s.csubx;
+	for (int c = 0; c < 3; c++) {
+		if (!bi.fast_ok[c] || (c == 2 && bi.fshare_cbcr)) continue;
+		if (o < bi.fimg_src[c] || o >= bi.fimg_src[c] + bi.fimg_bytes[c]) continue;
+		const int cols = c ? ccols : 64, rows = c ? crows : 64;
+		const int shift = 8 / fast_copies((c && s.csubx > 1) ? 8 : 16);
+		int rel = o - bi.fimg_src[c];
+		const bool minus = rel >= bi.fpat_off[c][1];
+		if (minus) rel -= bi.fpat_off[c][1];
+		const int k = rel / bi.fpat_copy[c], in = rel - k * bi.fpat_copy[c];
+		const int r = in / bi.fpat_stride[c], x = in - r * bi.fpat_stride[c];
+		if (r >= rows || x + k * shift >= cols) return 0;
+		const int8_t v = table_pattern(s, c ? 1 : 0, bi.uniform_pi[c], r, x + k * shift);
+		return (uint8_t)(minus ? (int8_t)-v : v);
+	}
+	return 0;
+}
+
+// Both images (bi.gbytes and bi.fbytes bytes), thread `tid` of `nthreads` doing its share: one thread in build_tables,
+// a CTA in fw_sessions_kernel.
+VFGS_HD void fill_tables(const TableSrc& s, const TableInfo& bi, uint8_t* blob, uint8_t* fblob, int tid, int nthreads)
+{
+	for (int o = tid; o < bi.gbytes; o += nthreads) blob[o] = general_image_byte(s, bi, o);
+	for (int o = tid; o < bi.fbytes; o += nthreads) fblob[o] = fast_image_byte(s, bi, o);
+}
+
+inline void build_tables(const HwState& h, TableInfo& g_bi, std::vector<uint8_t>& g_blob, std::vector<uint8_t>& g_fblob)
+{
+	Minus128 m;
+	scan_minus128(h, m);
+	layout_tables(h.plut, h.csubx, h.csuby, m, g_bi);
+	g_blob.assign((size_t)g_bi.gbytes, 0);
+	g_fblob.assign((size_t)g_bi.fbytes, 0);
+	const TableSrc s = {&h.pattern[0][0][0][0], &h.slut[0][0], &h.plut[0][0], h.csubx, h.csuby};
+	fill_tables(s, g_bi, g_blob.data(), g_fblob.data(), 0, 1);
 }
 
 
